@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the driver's measurement contract for colosseum_b200.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload step|vi|all]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload step|vi|all] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[1], "C2"): DeepSeaContinuous(size=30, p_rand=0.1) -- S=465, A=2 -- with
 65,536 parallel envs PER GPU advanced by the batched step kernel; metric = batched env-steps/sec over all GPUs.
@@ -39,6 +39,10 @@ def c2_workload(S, A, N):
     return (f"C2 DeepSeaContinuous(size=30,p_rand=0.1) S={S} A={A}, {N} envs per GPU, batched step by inverse-CDF over the "
             "dense CDF row, auto-reset, visitation counts on")
 L2_FLUSH_BYTES = 256 << 20
+# untimed steps enqueued right before the headline's timed replay (about 70 ms at the ~15 G env-steps/s this bench
+# measures for the headline on a B200 at 1,000 W): the GPU is busy and at its steady clocks when the timed steps start,
+# and the count is fixed, so the final env state depends on the arguments only
+LEAD_IN_STEPS = 16384
 
 
 def vi_sweep_bytes(S, A, store_q=True):
@@ -171,11 +175,16 @@ def max_over_ranks(x, world):
     return float(t.item())
 
 
-def _rotating_graph(torch, tb, N, rank, actions, n_steps_min, seed0, min_ms, world, track_visits=True):
+def _rotating_graph(torch, tb, N, rank, actions, n_steps, seed0, min_ms, world, track_visits=True, outputs=False):
     """`value` protocol: inputs larger than L2 instead of a flush.  NB independent env batches of N envs (each with its
-    own tables; together > 1.5 x the 126 MB L2) are stepped in rotation from ONE CUDA graph of max(n_steps_min, NB)
-    launches; the graph is replayed until the timed region is at least `min_ms`.  Returns ms per step (device time,
-    CUDA events on the launching stream, max over ranks), the number of timed steps and the region length."""
+    own tables; together > 1.5 x the 126 MB L2) are stepped in rotation (step i on batch i % NB) from ONE CUDA graph.
+    min_ms=None: the graph holds exactly `n_steps` launches and the timed region is one replay of it, enqueued right
+    behind at least LEAD_IN_STEPS untimed steps from a second graph that steps every batch once, in order, so that
+    whatever `n_steps` is, each timed step's batch was last stepped NB - 1 batches (more than L2) earlier.  Otherwise
+    the graph holds max(n_steps, NB) launches and is replayed until the timed region is at least `min_ms`.  Returns ms
+    per step (device time, CUDA events on the launching stream, max over ranks), the number of timed steps, the region
+    length and the bytes it touched; outputs=True adds what the last timed step left in its batch (the TimeStep
+    fields, env state and visitation counts) as host arrays."""
     from colosseum_b200.batched_mdp import BatchedMDP
 
     per_batch = 38 * N + 4 * tb.S * tb.A * (tb.ld + tb.ld // 4 + tb.ld // 32) + 2 * tb.S * tb.A * tb.ld
@@ -190,7 +199,7 @@ def _rotating_graph(torch, tb, N, rank, actions, n_steps_min, seed0, min_ms, wor
     for i in range(max(3, min(NB, 8))):  # untimed warm-up steps, same rotation
         batches[i % NB].step_async(actions[i % n_act], auto_reset=True)
     torch.cuda.synchronize()
-    per_graph = max(n_steps_min, NB)
+    per_graph = n_steps if min_ms is None else max(n_steps, NB)
     graph = torch.cuda.CUDAGraph()
     with torch.cuda.graph(graph):  # step i runs on env batch i % NB
         for i in range(per_graph):
@@ -198,12 +207,24 @@ def _rotating_graph(torch, tb, N, rank, actions, n_steps_min, seed0, min_ms, wor
     graph.replay()
     torch.cuda.synchronize()
     g0, g1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    g0.record()
-    graph.replay()
-    g1.record()
-    g1.synchronize()
-    reps = max(1, int(np.ceil(1.3 * min_ms / max(g0.elapsed_time(g1), 1e-3))))  # 30 % margin over the calibration replay
+    if min_ms is None:
+        reps, lead_in = 1, -(-LEAD_IN_STEPS // NB)
+        lead = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(lead):  # step j on env batch j: each pass ends on batch NB - 1, right before timed step 0
+            for j in range(NB):
+                batches[j].step_async(actions[j % n_act], auto_reset=True)
+        lead.replay()
+        torch.cuda.synchronize()
+    else:
+        g0.record()
+        graph.replay()
+        g1.record()
+        g1.synchronize()
+        reps = max(1, int(np.ceil(1.3 * min_ms / max(g0.elapsed_time(g1), 1e-3))))  # 30 % margin over the calibration replay
+        lead_in = 0
     barrier_sync(world)
+    for _ in range(lead_in):
+        lead.replay()
     g0.record()
     for _ in range(reps):
         graph.replay()
@@ -212,8 +233,17 @@ def _rotating_graph(torch, tb, N, rank, actions, n_steps_min, seed0, min_ms, wor
     ms = max_over_ranks(g0.elapsed_time(g1), world)
     assert all(int(b.status.item()) == 0 for b in batches)
     out = dict(ms_per_step=ms / (reps * per_graph), timed_steps=reps * per_graph, region_ms=ms, batches=NB,
-               bytes_touched=NB * per_batch, steps_per_graph=per_graph, replays=reps)
+               batch_bytes=per_batch, bytes_touched=NB * per_batch, timed_bytes=min(reps * per_graph, NB) * per_batch,
+               steps_per_graph=per_graph, replays=reps, lead_in_steps=lead_in * NB)
+    if outputs:
+        last = batches[(per_graph - 1) % NB]
+        ts = last._timestep()
+        out["outputs"] = {name: t.cpu().numpy() for name, t in (
+            ("step_type", ts.step_type), ("reward", ts.reward), ("discount", ts.discount), ("observation", ts.observation),
+            ("state", last.state), ("h", last.h), ("visits_s", last.visits_s), ("visits_sa", last.visits_sa))}
     del graph, batches
+    if min_ms is None:
+        del lead
     torch.cuda.empty_cache()
     return out
 
@@ -284,12 +314,13 @@ def bench_step_gpu(args, rank, world):
     del flush
 
     # ---- headline: back-to-back kernel throughput.  The per-step event pair above has a floor of ~10 us on B200
-    # (measured with a 32-env launch), i.e. most of it is launch + event latency, not the kernel.  Here the steps of
-    # NB independent env batches (each with its own tables; together larger than L2, so no flush is needed) are
-    # captured in one CUDA graph and replayed until the timed region is >= 50 ms: no CPU in the loop.
+    # (measured with a 32-env launch), i.e. most of it is launch + event latency, not the kernel.  Here the --steps
+    # steps of NB independent env batches (each with its own tables; together larger than L2, so no flush is needed)
+    # are captured in one CUDA graph and timed over one replay: no CPU in the loop.
     b2b = None
     try:
-        b2b = _rotating_graph(torch, tb, N, rank, actions, args.steps, 99, 50.0, world)
+        b2b = _rotating_graph(torch, tb, N, rank, actions, args.steps, 99, None, world,
+                              outputs=args.dump_outputs is not None)
     except Exception as e:  # reported, never fatal: the flushed number above does not depend on it
         b2b = dict(error=f"{type(e).__name__}: {e}")
 
@@ -1002,6 +1033,20 @@ def run_reference_arm(args):
 
 
 # ------------------------------------------------------------------------------------------------ main
+def dump_outputs(directory, b2b, rank):
+    """`--dump-outputs`: rank 0 writes the arrays of the last timed headline step as <directory>/<name>.npy, float32
+    fields as they are and integer fields as float64 (exact below 2**53).  Actions, seeds and step counts depend only on
+    the arguments, so two builds run with the same arguments can be compared output for output."""
+    if "outputs" not in b2b:
+        raise SystemExit(f"--dump-outputs: the headline step leg failed: {b2b.get('error')}")
+    outputs = b2b.pop("outputs")
+    if rank != 0:
+        return
+    os.makedirs(directory, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a if a.dtype == np.float32 else a.astype(np.float64))
+
+
 _RESULT_FD = None
 
 
@@ -1048,7 +1093,14 @@ def main():
     ap.add_argument("--c5-transport", default="fused", choices=["fused", "nccl"])
     ap.add_argument("--cpu-seconds", type=float, default=8.0)
     ap.add_argument("--no-sweep", action="store_true", help="skip the env-count sweep of the step leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed headline step left in its env batch (TimeStep fields, env state, "
+                         "visitation counts; rank 0) as DIR/<name>.npy, to compare builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "b200" or args.workload not in ("all", "step")):
+        ap.error("--dump-outputs needs the headline step leg (--impl b200, --workload all or step)")
     args.warmup = max(args.warmup, 3)
 
     if args.impl == "reference":
@@ -1090,6 +1142,8 @@ def main():
     if agents is not None:
         agents["model_based"] = bench_model_based_agents_gpu(args, rank, world)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs is not None:  # after the sampler's nvidia-smi child has been stopped: it may exit here
+        dump_outputs(args.dump_outputs, step["b2b"], rank)
     if world > 1:
         import torch.distributed as dist
 
@@ -1184,13 +1238,16 @@ def main():
         flushed_note = "L2 flushed between timed steps (256 MiB write), each step timed with its own CUDA-event pair"
         if "ms_per_step" in b2b:
             # headline protocol: inputs larger than L2 instead of a flush -- step i runs on env batch i % NB, every batch
-            # with its own tables, max(K, NB) steps captured in one CUDA graph, replayed until the region is >= 50 ms
+            # with its own tables, the K steps captured in one CUDA graph and timed over one replay
             sec = b2b["ms_per_step"] / 1e3
-            l2_note = (f"no flush: step i runs on env batch i % {b2b['batches']} ({b2b['batches']} independent batches of "
-                       f"{N} envs, each with its own tables; {b2b['bytes_touched'] / 2**20:.0f} MiB touched per rotation > "
-                       f"126 MB L2); {b2b['steps_per_graph']} steps per CUDA graph, replayed {b2b['replays']} times inside "
-                       f"ONE CUDA-event pair: {b2b['timed_steps']} timed steps, {b2b['region_ms']:.1f} ms timed region "
-                       "(--steps sets the minimum graph length; the region is never shorter than 50 ms)")
+            nb, mib = b2b["batches"], b2b["batch_bytes"] / 2**20
+            l2_note = (f"no flush: step i runs on env batch i % {nb} ({nb} independent batches of {N} envs, each with its "
+                       f"own tables, {mib:.1f} MiB each); the {b2b['timed_steps']} steps of --steps captured in one CUDA "
+                       f"graph and timed over one replay inside ONE CUDA-event pair, enqueued right behind "
+                       f"{b2b['lead_in_steps']} untimed steps that step the {nb} batches in order, so each timed step's "
+                       f"batch was last stepped {nb - 1} batches ({(nb - 1) * mib:.0f} MiB > 126 MB L2) earlier; the "
+                       f"timed steps touch {b2b['timed_bytes'] / 2**20:.0f} MiB in a {b2b['region_ms']:.3f} ms region "
+                       "(one replay: noisier than a long region, a larger --steps gives a steadier number)")
             launches, region_s = b2b["timed_steps"], b2b["region_ms"] / 1e3
         else:
             sec, l2_note, launches, region_s = sec_flushed, flushed_note, step["launches"], step["ms"] / 1e3

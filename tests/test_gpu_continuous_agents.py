@@ -107,13 +107,13 @@ def test_ucrl2_golden_trace_and_reference_tables():
 
 
 def test_ucrl2_device_loop_through_the_reference_class():
-    """where the reference package is staged (baseline/_ref on the GPU box): the device loops' trajectories through the
+    """where the reference package is staged (oracle/reference_import.py): the device loops' trajectories through the
     UNMODIFIED UCRL2Continuous -- its episode ends and model tables must be the device's, bit for bit, and its numba
     extended VI must land within the stopping tolerance of the device's Q."""
     from oracle.reference_import import reference_available
 
     if not reference_available():
-        pytest.skip("the reference package is not staged (baseline/_ref)")
+        pytest.skip("the unmodified Colosseum package is not staged (oracle/_ref or $COLOSSEUM_REFERENCE_ROOT)")
     import colosseum_b200.agent_loop as al
     from make_qlearning_golden import reference_models
     from make_ucrl2_golden import mdp_spec, replay_reference
@@ -364,7 +364,7 @@ def test_psrl_continuous_device_loop_through_the_reference_class():
     from oracle.reference_import import reference_available
 
     if not reference_available():
-        pytest.skip("the reference package is not staged (baseline/_ref)")
+        pytest.skip("the unmodified Colosseum package is not staged (oracle/_ref or $COLOSSEUM_REFERENCE_ROOT)")
     import colosseum_b200.agent_loop as al
     from make_qlearning_golden import reference_models
     from make_ucrl2_golden import mdp_spec

@@ -3,8 +3,8 @@ names (colosseum_b200/patch.py); the reference's own property layer (colosseum/m
 mdp/base_finite.py:167-208) then decides which DP runs on which tensor, and every number it returns is compared with
 the value the UNPATCHED reference produced for the same constructor arguments (tests/golden/inst_*.npz).
 
-The reference package is the unmodified one: /root/reference in the build container, its `pip install --target
-baseline/_ref` twin on the GPU box (oracle/reference_import.py).  Skipped when neither is present."""
+The reference package is the unmodified one, staged outside git (oracle/reference_import.py says where it is looked
+for).  Skipped when it is not staged."""
 import numpy as np
 import pytest
 
@@ -18,7 +18,7 @@ def ref():
     from oracle.reference_import import import_reference, reference_available
 
     if not reference_available():
-        pytest.skip("the reference package is not staged (baseline/_ref)")
+        pytest.skip("the unmodified Colosseum package is not staged (oracle/_ref or $COLOSSEUM_REFERENCE_ROOT)")
     import_reference()
     import colosseum.mdp  # noqa: F401
 

@@ -53,7 +53,7 @@ def test_from_mdp_matches_golden_recording():
     from oracle.reference_import import import_reference, reference_available
 
     if not reference_available():
-        pytest.skip("/root/reference not present")
+        pytest.skip("the unmodified Colosseum package is not staged (oracle/_ref or $COLOSSEUM_REFERENCE_ROOT)")
     import_reference()
     import colosseum.mdp  # noqa: F401
     from colosseum.mdp.simple_grid import SimpleGridContinuous
@@ -74,7 +74,7 @@ def test_patch_rebinds_reference_names():
     from oracle.reference_import import import_reference, reference_available
 
     if not reference_available():
-        pytest.skip("/root/reference not present")
+        pytest.skip("the unmodified Colosseum package is not staged (oracle/_ref or $COLOSSEUM_REFERENCE_ROOT)")
     import_reference()
     import colosseum.mdp  # noqa: F401
     import colosseum.hardness.measures.diameter as ref_diam
@@ -106,7 +106,7 @@ def test_patched_reference_fails_loudly_without_gpu():
     from oracle.reference_import import import_reference, reference_available
 
     if not reference_available():
-        pytest.skip("/root/reference not present")
+        pytest.skip("the unmodified Colosseum package is not staged (oracle/_ref or $COLOSSEUM_REFERENCE_ROOT)")
     if torch.cuda.is_available():
         pytest.skip("needs a box without a GPU")
     import_reference()
