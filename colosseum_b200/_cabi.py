@@ -12,6 +12,8 @@ LIB_PATH = os.environ.get("COLO_B200_LIB") or os.path.join(_PKG, "_lib", "libcol
 OK, OVERFLOW, MAX_ITER, NEEDS_RESET, SERVER_LAPSED, BAD_ACTION = 0, 1, 2, 3, 4, 5
 FOLD_MAX, FOLD_PI, FOLD_MIN = 0, 1, 2
 STEP_FIRST, STEP_MID, STEP_LAST = 0, 1, 2
+# step-kernel variants of colo_step_kernel_launches (include/colosseum_b200.h, COLO_STEP_KIND_*)
+STEP_KIND_LEAN, STEP_KIND_KARY, STEP_KIND_SHORT, STEP_KIND_LONG, STEP_KIND_SUCC = 0, 1, 2, 3, 4
 
 
 class ColosseumB200Error(RuntimeError):
@@ -191,6 +193,7 @@ PROTOTYPES = {
     "colo_launch_count": (_ULL, []),
     "colo_reset_launch_count": (None, []),
     "colo_backup_tma_sweeps": (_ULL, []),
+    "colo_step_kernel_launches": (_ULL, [_I]),
     "colo_stream_synchronize": (_I, [_P]),
     "colo_backup_f32": (_I, [C.POINTER(BackupArgs), _P]),
     "colo_backup_f64acc": (_I, [C.POINTER(BackupArgs), _P]),

@@ -17,6 +17,7 @@
 
 #include <cuda.h>
 
+#include <atomic>
 #include <thread>
 #include <vector>
 
@@ -25,6 +26,11 @@
 namespace colo {
 
 constexpr int kStepThreads = 64;  // small CTAs: 2048 warp-tiles at N=65,536 spread evenly over 148 SMs
+
+// step launches per kernel variant (colo_step_kernel_launches), counted on the host where the variant is chosen, so a
+// caller can tell which kernel served a call; a launch captured into a CUDA graph counts once, at capture
+static std::atomic<unsigned long long> g_step_launches[COLO_STEP_KINDS];
+static void count_step_launch(int kind) { g_step_launches[kind].fetch_add(1, std::memory_order_relaxed); }
 
 struct StepIO {
   long long N;
@@ -876,6 +882,7 @@ static int launch_dense(const colo_mdp_tables* tb, const StepIO& io, void* strea
         COLO_LEAN(8);
       }
 #undef COLO_LEAN
+      count_step_launch(COLO_STEP_KIND_LEAN);
       return check_launch("env_step_kary_lean_kernel");
     }
     COLO_ARG_CHECK(!io.io_compact, "io_compact is offered by the common call of the dense f32 step only (supplied actions, "
@@ -897,6 +904,7 @@ static int launch_dense(const colo_mdp_tables* tb, const StepIO& io, void* strea
         COLO_KARY(8);
       }
 #undef COLO_KARY
+      count_step_launch(COLO_STEP_KIND_KARY);
       return check_launch("env_step_dense_kary_kernel");
     }
     const int grid = grid_for(kStepThreads / 32, (io.N + tile - 1) / tile);
@@ -917,10 +925,12 @@ static int launch_dense(const colo_mdp_tables* tb, const StepIO& io, void* strea
       COLO_SHORT(8, 2);
     }
 #undef COLO_SHORT
+    count_step_launch(COLO_STEP_KIND_SHORT);
   } else {
     COLO_ARG_CHECK(!io.io_compact, "io_compact needs rows of at most 1024 states");
     const int grid = grid_for(kStepThreads / 32, (io.N + 31) / 32);
     launch_step(env_step_dense_kernel<TC, 8, SERVER>, grid, SERVER, share, tb, io, st);
+    count_step_launch(COLO_STEP_KIND_LONG);
   }
   return check_launch("env_step_dense_kernel");
 }
@@ -932,6 +942,7 @@ static int launch_succ(const colo_mdp_tables* tb, const StepIO& io, void* stream
   COLO_ARG_CHECK(!io.io_compact, "io_compact is offered by the dense f32 step only");
   if (io.N == 0) return COLO_OK;
   launch_step(env_step_succ_kernel<SERVER>, grid_for(kStepThreads, io.N), SERVER, share, tb, io, (cudaStream_t)stream);
+  count_step_launch(COLO_STEP_KIND_SUCC);
   return check_launch("env_step_succ_kernel");
 }
 
@@ -1438,6 +1449,10 @@ int colo_env_server_stop(const colo_env_server* srv, void* stream) {
     return COLO_ERR_CUDA;
   }
   return COLO_OK;
+}
+
+unsigned long long colo_step_kernel_launches(int kind) {
+  return kind >= 0 && kind < COLO_STEP_KINDS ? colo::g_step_launches[kind].load(std::memory_order_relaxed) : 0ULL;
 }
 
 int colo_emit_observations(const float* table, const int* state, const int* h, const unsigned char* step_type,

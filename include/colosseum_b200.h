@@ -58,6 +58,15 @@ int colo_stream_synchronize(void* stream);
 void colo_reset_launch_count(void);
 /* sweeps taken by the TMA-staged variant of the streaming backup kernel (COLO_BACKUP_TMA=1, DESIGN 4.1) since load */
 unsigned long long colo_backup_tma_sweeps(void);
+/* step launches since load that went to each step-kernel variant (`kind`: COLO_STEP_KIND_*; 0 for any other value).
+ * Counted on the host when the launch is enqueued: a launch captured into a CUDA graph counts once. */
+#define COLO_STEP_KIND_LEAN 0  /* env_step_kary_lean_kernel: the common dense f32 call                         */
+#define COLO_STEP_KIND_KARY 1  /* env_step_dense_kary_kernel: rows of <= 1024 states, every other dense call    */
+#define COLO_STEP_KIND_SHORT 2 /* env_step_dense_short_kernel: the warp-cooperative kernel (COLO_STEP_KERNEL=coop) */
+#define COLO_STEP_KIND_LONG 3  /* env_step_dense_kernel: rows of more than 1024 states (or ld % 128 != 0)      */
+#define COLO_STEP_KIND_SUCC 4  /* env_step_succ_kernel: successor-list tables                                  */
+#define COLO_STEP_KINDS 5
+unsigned long long colo_step_kernel_launches(int kind);
 
 /* ---------------------------------------------------------------- (B) Bellman backups ------------------- */
 /*
