@@ -4,6 +4,7 @@ the batched agent/MDP interaction step and the dynamic-programming Bellman backu
     colosseum_b200.dynamic_programming   twin of colosseum.dynamic_programming
     colosseum_b200.hardness              twin of colosseum.hardness.measures
     colosseum_b200.batched_mdp           BatchedMDP: N parallel BaseMDP.reset/step
+                                         MixedBatchedMDP: envs of many MDP instances in one batch, one launch per step
     colosseum_b200.tables                host-side table extraction from reference MDP objects
     colosseum_b200.patch                 install the GPU path behind the reference's own module attributes
 

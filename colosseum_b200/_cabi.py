@@ -14,6 +14,7 @@ FOLD_MAX, FOLD_PI, FOLD_MIN = 0, 1, 2
 STEP_FIRST, STEP_MID, STEP_LAST = 0, 1, 2
 # step-kernel variants of colo_step_kernel_launches (include/colosseum_b200.h, COLO_STEP_KIND_*)
 STEP_KIND_LEAN, STEP_KIND_KARY, STEP_KIND_SHORT, STEP_KIND_LONG, STEP_KIND_SUCC = 0, 1, 2, 3, 4
+STEP_KIND_MIXED_SUCC, STEP_KIND_MIXED_DENSE = 5, 6
 
 
 class ColosseumB200Error(RuntimeError):
@@ -234,6 +235,13 @@ PROTOTYPES = {
     "colo_env_step_dense_f64": (_I, [C.POINTER(MdpTables), C.POINTER(EnvBatch), _I, _P, _P, _ULL, _I, _P]),
     "colo_env_step_succ": (_I, [C.POINTER(MdpTables), C.POINTER(EnvBatch), _I, _P, _P, _ULL, _I, _P]),
     "colo_env_random_steps": (_I, [C.POINTER(MdpTables), C.POINTER(EnvBatch), _I, _I, _ULL, _I, _P]),
+    "colo_mixed_tables_create": (_I, [C.POINTER(MdpTables), _I, C.POINTER(C.c_longlong), C.POINTER(C.c_ulonglong), _I,
+                                      _P, C.POINTER(C.c_void_p)]),
+    "colo_mixed_tables_destroy": (None, [_P]),
+    "colo_mixed_visits_size": (_LL, [_P, _I]),
+    "colo_mixed_env_reset": (_I, [_P, C.POINTER(EnvBatch), _P, _ULL, _P]),
+    "colo_mixed_env_step": (_I, [_P, C.POINTER(EnvBatch), _I, _P, _P, _ULL, _I, _P]),
+    "colo_mixed_env_random_steps": (_I, [_P, C.POINTER(EnvBatch), _I, _ULL, _I, _P]),
     "colo_emit_noise_correlated": (_I, [_P, _P, _P, _LL, _I, _I, _P, _I, _D, _ULL, _ULL, _ULL, _P]),
     "colo_env_pipeline_run": (_I, [_P, _I, _P, _I, _ULL, _I, _P, _P]),
     "colo_env_pipeline_run_threads": (_I, [_P, _I, _P, _I, _ULL, _I, _P, _P]),

@@ -599,6 +599,237 @@ class BatchedMDP:
             self._visits_sa.zero_()
 
 
+class MixedBatchedMDP:
+    """One batch whose envs belong to different MDP instances, stepped by ONE launch per reset / step / fused random
+    steps whatever the number of instances (include/colosseum_b200.h, colo_mixed_tables).  Instance i owns the
+    contiguous envs `segment(i)`; there, with the instance's own tables, H, action range and seed `seed[i]`, the batch
+    is bit-identical to `BatchedMDP(tables[i], n_envs[i], mode, seed=seed[i])` driven by the same calls.
+
+        env = MixedBatchedMDP([inst.tables for inst in suite], 1024, mode="succ", seed=0)
+        env.reset()
+        env.random_steps_fused(1000)
+        env.get_visitation_counts(3)      # instance 3's state counts
+
+    `n_envs` and `seed` are an int for every instance or one value per instance.  Observations are state indices within
+    the env's own instance.  Host I/O, compact I/O, the pipelines, the step server and emission maps are single-MDP."""
+    VISIT_COPIES = BatchedMDP.VISIT_COPIES
+
+    def __init__(self, tables, n_envs, mode: str = "succ", seed=0, track_visits: bool = True):
+        import torch
+
+        assert mode in _MODES
+        self.torch = torch
+        self.tables = list(tables)
+        n = len(self.tables)
+        assert n >= 1, "a mixed batch needs at least one instance"
+        sizes = [int(n_envs)] * n if np.ndim(n_envs) == 0 else [int(x) for x in n_envs]
+        seeds = [int(seed)] * n if np.ndim(seed) == 0 else [int(x) for x in seed]
+        assert len(sizes) == n and len(seeds) == n, "n_envs and seed: one value, or one per instance"
+        assert all(x >= 1 for x in sizes), "every instance needs at least one env"
+        self.mode = mode
+        self.sizes = np.array(sizes, np.int64)
+        self.offsets = np.concatenate([[0], np.cumsum(self.sizes)[:-1]]).astype(np.int64)
+        self.seeds = np.array(seeds, np.uint64)
+        self.n_envs = int(self.sizes.sum())
+        self.n_states = np.array([tb.S for tb in self.tables], np.int64)
+        self.n_actions = np.array([tb.A for tb in self.tables], np.int64)
+        self.H = np.array([tb.H for tb in self.tables], np.int64)  # 0: continuous
+        self._s_off = np.concatenate([[0], np.cumsum(self.n_states)]).astype(np.int64)
+        self._sa_off = np.concatenate([[0], np.cumsum(self.n_states * self.n_actions)]).astype(np.int64)
+        # the single-MDP upload, reused as is: in the dense modes it also builds the short-row search index (cdf_mid,
+        # cdf_coarse, rew_cls_pad) for rows of <= 1024 states, which the mixed kernels do not read -- a few build
+        # launches per instance at construction and up to about half the bytes of an f32 dense CDF again
+        self.dev = []
+        for i, tb in enumerate(self.tables):
+            try:
+                self.dev.append(DeviceTables(tb, mode))
+            except AssertionError as e:
+                raise AssertionError(f"instance {i}: {e}") from None
+        self._c_tables = (_cabi.MdpTables * n)(*[d.c for d in self.dev])
+        self._handle = None
+        self._make_handle()
+        N = self.n_envs
+        # i32[N]: the instance of every env, for the caller.  It mirrors the env -> instance map the handle uploaded for
+        # the kernels (same sizes, same order; both fixed at construction) -- the kernels never read this copy.
+        self.instance = torch.repeat_interleave(torch.arange(n, dtype=torch.int32),
+                                                torch.from_numpy(self.sizes)).to("cuda")
+        self.state = torch.zeros(N, dtype=torch.int32, device="cuda")
+        self.h = torch.zeros(N, dtype=torch.int32, device="cuda")
+        # obs i32 | reward f32 | discount f32 | step_type u8, as BatchedMDP's device-resident block (one clone per TimeStep)
+        self._out = torch.zeros(13 * N, dtype=torch.uint8, device="cuda")
+        self.obs = self._out[: 4 * N].view(torch.int32)
+        self.reward = self._out[4 * N: 8 * N].view(torch.float32)
+        self.discount = self._out[8 * N: 12 * N].view(torch.float32)
+        self.step_type = self._out[12 * N:]
+        self.step_type.fill_(_cabi.STEP_LAST)  # stepping before reset() is flagged, as in BatchedMDP
+        self.action = torch.zeros(N, dtype=torch.int32, device="cuda")
+        self.status = torch.zeros(1, dtype=torch.int32, device="cuda")
+        vc = self.VISIT_COPIES
+        size = _cabi.lib().colo_mixed_visits_size
+        self._visits_s = torch.zeros((vc, size(self._handle, 0)), dtype=torch.int64, device="cuda") if track_visits else None
+        self._visits_sa = torch.zeros((vc, size(self._handle, 1)), dtype=torch.int64, device="cuda") if track_visits else None
+        self.t = 0
+        self._was_reset = False
+        self._udt = torch.float32 if mode == "dense_f32" else torch.float64
+        b = _cabi.EnvBatch()
+        b.N = N  # seed / env0 are not used by the mixed calls: every env takes them from its instance
+        b.state, b.h, b.step_type = _cabi.ptr(self.state), _cabi.ptr(self.h), _cabi.ptr(self.step_type)
+        b.action, b.reward, b.obs = _cabi.ptr(self.action), _cabi.ptr(self.reward), _cabi.ptr(self.obs)
+        b.visits_s, b.visits_sa, b.visits_copies = _cabi.ptr(self._visits_s), _cabi.ptr(self._visits_sa), vc
+        b.status = _cabi.ptr(self.status)
+        b.discount = _cabi.ptr(self.discount)
+        self._batch = b
+        self._batch_ref = C.byref(b)
+        self._own_action_ptr = b.action
+
+    # BatchedMDP's helpers read only these of its attributes
+    host_io = compact_io = scalar_api = False
+    _u = BatchedMDP._u
+    _timestep = BatchedMDP._timestep
+
+    def _make_handle(self):
+        n = len(self.tables)
+        out = C.c_void_p()
+        rc = _cabi.lib().colo_mixed_tables_create(self._c_tables, n, (C.c_longlong * n)(*self.sizes.tolist()),
+                                                  (C.c_ulonglong * n)(*self.seeds.tolist()), _MODES[self.mode],
+                                                  _cabi.current_stream(), C.byref(out))
+        _cabi.check(rc, "colo_mixed_tables_create")
+        if self._handle is not None:
+            _cabi.lib().colo_mixed_tables_destroy(self._handle)
+        self._handle = out.value
+
+    def __del__(self):
+        try:
+            if getattr(self, "_handle", None):
+                _cabi.lib().colo_mixed_tables_destroy(self._handle)
+                self._handle = None
+        except Exception:
+            pass
+
+    @property
+    def n_instances(self):
+        return len(self.tables)
+
+    def segment(self, i: int) -> slice:
+        """the envs of instance i"""
+        return slice(int(self.offsets[i]), int(self.offsets[i] + self.sizes[i]))
+
+    def action_spec(self, i: int):
+        return DiscreteArray(int(self.n_actions[i]), name="action")
+
+    def observation_spec(self, i: int):
+        return DiscreteArray(int(self.n_states[i]), name="observation")
+
+    def reset(self, u_next=None) -> BatchedTimeStep:
+        """BaseMDP.reset for every env, from its own instance's start distribution"""
+        u = self._u(u_next, self.torch.float64)
+        rc = _cabi.lib().colo_mixed_env_reset(self._handle, self._batch_ref, _cabi.ptr(u), self.t, _cabi.current_stream())
+        _cabi.check(rc, "colo_mixed_env_reset")
+        self.t += 1
+        self._was_reset = True
+        return self._timestep()
+
+    def step_async(self, action=None, auto_reset=False, u_next=None, u_reward=None, check=False):
+        """BatchedMDP.step_async over all envs: action=None plays uniformly random actions in [0, A_i) of every env's
+        instance and records them in self.action"""
+        torch = self.torch
+        random_actions = action is None
+        act_ptr = self._own_action_ptr
+        if not random_actions:
+            if isinstance(action, torch.Tensor) and action.is_cuda and action.dtype == torch.int32 and action.is_contiguous():
+                act_ptr = action.data_ptr()
+            elif isinstance(action, torch.Tensor):
+                self.action.copy_(action, non_blocking=True)
+            else:
+                a = np.array(np.broadcast_to(np.asarray(action, np.int32), (self.n_envs,)))
+                self.action.copy_(torch.from_numpy(a), non_blocking=True)
+        un = None if u_next is None else self._u(u_next, self._udt)
+        ur = None if u_reward is None else self._u(u_reward, torch.float32)
+        self._batch.action = act_ptr
+        rc = _cabi.lib().colo_mixed_env_step(self._handle, self._batch_ref, int(random_actions), _cabi.ptr(un),
+                                             _cabi.ptr(ur), self.t, int(bool(auto_reset)),
+                                             torch.cuda.current_stream().cuda_stream)
+        if rc != 0:
+            _cabi.check(rc, "colo_mixed_env_step")
+        self.t += 1
+        if check or not auto_reset:
+            st = int(self.status.item())
+            if st == _cabi.BAD_ACTION:
+                self.status.zero_()
+                raise ValueError("an action outside [0, A) of its env's instance was supplied (that env was not stepped)")
+            if st == _cabi.NEEDS_RESET:
+                self.status.zero_()
+                if not self._was_reset:
+                    raise AttributeError("step() called before reset() (reference: necessary_reset is unset)")
+                raise AssertionError("an episode has terminated: call reset() or step(..., auto_reset=True)")
+
+    def step(self, action, auto_reset=False, u_next=None, u_reward=None) -> BatchedTimeStep:
+        self.step_async(action, auto_reset, u_next, u_reward)
+        return self._timestep()
+
+    def random_step(self, auto_reset=False):
+        """BaseMDP.random_step for every env: returns (BatchedTimeStep, actions)"""
+        self.step_async(None, auto_reset)
+        return self._timestep(), self.action.clone()
+
+    def random_steps(self, n, auto_reset=False):
+        return [self.random_step(auto_reset) for _ in range(n)]
+
+    def random_steps_fused(self, n, auto_reset=True):
+        """n random-agent steps of every env in ONE launch -- bit-identical to n calls of random_step()"""
+        self._batch.action = self._own_action_ptr
+        rc = _cabi.lib().colo_mixed_env_random_steps(self._handle, self._batch_ref, int(n), self.t, int(bool(auto_reset)),
+                                                     _cabi.current_stream())
+        _cabi.check(rc, "colo_mixed_env_random_steps")
+        self.t += int(n)
+        if not auto_reset and int(self.status.item()) == _cabi.NEEDS_RESET:
+            self.status.zero_()
+            raise AssertionError("an episode has terminated: call reset() or use auto_reset=True")
+        return self._timestep()
+
+    def get_visitation_counts(self, i: int, state_only=True):
+        """instance i's counts (base.py:1357-1373): i64[S_i], or i64[S_i, A_i] counted on the NEXT node"""
+        if self._visits_s is None:
+            return None
+        if state_only:
+            return self._visits_s[:, int(self._s_off[i]): int(self._s_off[i + 1])].sum(0)
+        S, A = int(self.n_states[i]), int(self.n_actions[i])
+        return self._visits_sa[:, int(self._sa_off[i]): int(self._sa_off[i + 1])].sum(0).view(S, A)
+
+    def reset_visitation_counts(self):
+        if self._visits_s is not None:
+            self._visits_s.zero_()
+            self._visits_sa.zero_()
+
+    def state_dict(self):
+        """everything needed to continue the trajectories bit for bit"""
+        self.torch.cuda.current_stream().synchronize()
+        d = {"sizes": self.sizes.copy(), "seeds": self.seeds.copy(), "t": self.t, "mode": self.mode,
+             "was_reset": self._was_reset, "state": self.state.cpu(), "h": self.h.cpu(),
+             "step_type": self.step_type.cpu().clone(), "obs": self.obs.cpu().clone(),
+             "reward": self.reward.cpu().clone(), "discount": self.discount.cpu().clone()}
+        if self._visits_s is not None:
+            d["visits_s"], d["visits_sa"] = self._visits_s.sum(0).cpu(), self._visits_sa.sum(0).cpu()
+        return d
+
+    def load_state_dict(self, d):
+        assert np.array_equal(d["sizes"], self.sizes) and d["mode"] == self.mode, \
+            "checkpoint of another batch shape / sampler mode"
+        if not np.array_equal(d["seeds"], self.seeds):
+            self.seeds = np.array(d["seeds"], np.uint64)
+            self._make_handle()
+        self.t = int(d["t"])
+        self._was_reset = bool(d["was_reset"])
+        for name in ("state", "h", "step_type", "obs", "reward", "discount"):
+            getattr(self, name).copy_(d[name])
+        if self._visits_s is not None and "visits_s" in d:
+            self._visits_s.zero_()
+            self._visits_sa.zero_()
+            self._visits_s[0].copy_(d["visits_s"])
+            self._visits_sa[0].copy_(d["visits_sa"])
+        self.torch.cuda.current_stream().synchronize()
+
+
 def split_sizes(n: int, groups: int):
     """sizes and offsets of `groups` contiguous shards of n items, the first n % groups shards one item larger"""
     assert 1 <= groups <= n

@@ -207,9 +207,11 @@ struct EnvIn {
   float un32, ur;
 };
 
+// `seed` / `ctr`: the env's Philox key and counter -- (io.seed, io.env0 + e) in a single-MDP batch, (the instance's
+// seed, e - the instance's first env) in a mixed batch
 template <bool F32U>
 __device__ __forceinline__ EnvIn load_env(const StepIO& io, const colo_mdp_tables& tb, long long e,
-                                           unsigned long long t) {
+                                           unsigned long long t, unsigned long long seed, unsigned long long ctr) {
   EnvIn in;
   in.bad = 0;
   in.st = io.step_type[e];
@@ -217,7 +219,7 @@ __device__ __forceinline__ EnvIn load_env(const StepIO& io, const colo_mdp_table
   in.h = io.h[e];  // needed only by the epilogue: issued here so that its (cold) latency overlaps the search
   Philox4 w;
   const bool need_rng = io.u_next == nullptr || io.u_rew == nullptr || io.random_actions;
-  if (need_rng) w = philox4x32_10(io.seed, io.env0 + (uint64_t)e, t);
+  if (need_rng) w = philox4x32_10(seed, ctr, t);
   if (io.u_next) {
     if (F32U) {
       in.un32 = reinterpret_cast<const float*>(io.u_next)[e];
@@ -240,9 +242,17 @@ __device__ __forceinline__ EnvIn load_env(const StepIO& io, const colo_mdp_table
   return in;
 }
 
-// epilogue of a regular step for one env held by this thread
+template <bool F32U>
+__device__ __forceinline__ EnvIn load_env(const StepIO& io, const colo_mdp_tables& tb, long long e,
+                                           unsigned long long t) {
+  return load_env<F32U>(io, tb, e, t, io.seed, io.env0 + (uint64_t)e);
+}
+
+// epilogue of a regular step for one env held by this thread.  off_s / off_sa: where the env's MDP starts in the
+// counter rows (non-zero in a mixed batch, whose instances share one concatenated [copies][sum S] / [copies][sum S*A])
 __device__ __forceinline__ void finish_env(const StepIO& io, const colo_mdp_tables& tb, long long e, const EnvIn& in,
-                                           int nxt, int cls, bool stepping, bool resetting) {
+                                           int nxt, int cls, bool stepping, bool resetting, long long off_s = 0,
+                                           long long off_sa = 0) {
   if (resetting) {  // auto_reset path == BaseMDP.reset(): the action is ignored, reward is None (NaN here)
     nxt = sample_start(tb, in.un64);
     io.state[e] = nxt;
@@ -266,8 +276,15 @@ __device__ __forceinline__ void finish_env(const StepIO& io, const colo_mdp_tabl
     io.obs[e] = last ? -1 : nxt;
   }
   const long long copy = blockIdx.x & io.visits_mask;  // privatised counters: spread same-state atomics over L2
-  if (io.visits_s) aggregated_inc(io.visits_s + copy * io.n_s, nxt, stepping || resetting);
-  if (io.visits_sa) aggregated_inc(io.visits_sa + copy * io.n_sa, (long long)nxt * tb.A + in.a, stepping);
+  if (io.visits_s) aggregated_inc(io.visits_s + copy * io.n_s, off_s + nxt, stepping || resetting);
+  if (io.visits_sa) aggregated_inc(io.visits_sa + copy * io.n_sa, off_sa + (long long)nxt * tb.A + in.a, stepping);
+}
+
+// the dense reward class of a step s --a--> nxt
+__device__ __forceinline__ int dense_cls(const colo_mdp_tables& tb, const EnvIn& in, int nxt) {
+  if (tb.rew_cls_sas) return tb.rew_cls_sas[((size_t)in.s * tb.A + in.a) * tb.S + nxt];
+  if (tb.rew_cls_sa) return tb.rew_cls_sa[(size_t)in.s * tb.A + in.a];
+  return 0;
 }
 
 // Position of x in one monotone dense row, warp-cooperative.  The row is read as quads (4 consecutive entries per
@@ -304,6 +321,18 @@ __device__ __forceinline__ int row_count_below(const TC* __restrict__ row, int l
     }
   }
   return ld;
+}
+
+// next state of one env from its dense row, searched by the whole warp (row, S, ld, u warp-uniform):
+// first j with cdf[j] > u * total  ==  number of entries <= x
+template <typename TC, int NCH>
+__device__ __forceinline__ int warp_row_next(const TC* __restrict__ row, int S, int ld, TC u, int lane) {
+  const TC total = __ldg(row + S - 1);
+  const TC x = u * total;
+  int nxt = row_count_below<TC, NCH, false>(row, ld, x, lane);
+  if (nxt >= S)  // x >= total (rounding): bisect's hi = n-1 clamp == first index where the row reaches total
+    nxt = row_count_below<TC, NCH, true>(row, ld, total, lane);
+  return nxt;
 }
 
 constexpr int kEnvUnroll = 4;  // independent row searches in flight per warp
@@ -349,22 +378,11 @@ __global__ void __launch_bounds__(kStepThreads) env_step_dense_kernel(const colo
         const int a_i = __shfl_sync(FULL, a_l, i);
         const TC u_i = __shfl_sync(FULL, u_l, i);
         const TC* row = cdf + ((size_t)s_i * A + a_i) * ld;
-        const TC total = __ldg(row + S - 1);
-        const TC x = u_i * total;
-        // first j with cdf[j] > x  ==  number of entries <= x
-        int nxt = row_count_below<TC, NCH, false>(row, ld, x, lane);
-        if (nxt >= S)  // x >= total (rounding): bisect's hi = n-1 clamp == first index where the row reaches total
-          nxt = row_count_below<TC, NCH, true>(row, ld, total, lane);
+        const int nxt = warp_row_next<TC, NCH>(row, S, ld, u_i, lane);
         if (lane == i) my_next = nxt;
       }
     }
-    int cls = 0;
-    if (stepping) {
-      if (tb.rew_cls_sas)
-        cls = tb.rew_cls_sas[((size_t)in.s * A + in.a) * S + my_next];
-      else if (tb.rew_cls_sa)
-        cls = tb.rew_cls_sa[(size_t)in.s * A + in.a];
-    }
+    const int cls = stepping ? dense_cls(tb, in, my_next) : 0;
     finish_env(io, tb, valid ? e : 0, in, my_next, cls, stepping, resetting);
   }
   if (!SERVER) return;
@@ -685,6 +703,34 @@ __global__ void __launch_bounds__(kLeanThreads) env_step_kary_lean_kernel(const 
   aggregated_inc(io.visits_sa + (size_t)copy * io.n_sa, (long long)nxt * A + a, stepping);
 }
 
+// one step of one env from successor-list tables (every lane of the warp calls it: finish_env uses warp collectives);
+// seed / ctr / off_s / off_sa as in load_env and finish_env
+__device__ __forceinline__ void succ_env_step(const StepIO& io, const colo_mdp_tables& tb, long long e, bool valid,
+                                              unsigned long long t, unsigned long long seed, unsigned long long ctr,
+                                              long long off_s, long long off_sa) {
+  EnvIn in;
+  in.s = 0; in.a = 0; in.st = COLO_STEP_MID; in.h = 0; in.bad = 0; in.un64 = 0.0; in.un32 = 0.f; in.ur = 0.f;
+  if (valid) in = load_env<false>(io, tb, e, t, seed, ctr);
+  const bool is_last = valid && in.st == COLO_STEP_LAST;
+  const bool resetting = is_last && io.auto_reset;
+  const bool stepping = valid && !is_last && !in.bad;
+  if (is_last && !io.auto_reset && io.status) *io.status = COLO_NEEDS_RESET;
+  int nxt = 0, cls = 0;
+  if (stepping) {
+    const size_t sa = (size_t)in.s * tb.A + in.a;
+    const size_t base = sa * tb.Ksucc;
+    const int n = __ldg(tb.succ_len + sa);
+    int pos = 0;
+    if (n > 1) {
+      const double total = __ldg(tb.succ_cum + base + n - 1) + 0.0;
+      pos = bisect_count(tb.succ_cum + base, n, in.un64 * total);
+    }
+    nxt = __ldg(tb.succ_idx + base + pos);
+    cls = tb.rew_cls_succ ? __ldg(tb.rew_cls_succ + base + pos) : 0;
+  }
+  finish_env(io, tb, valid ? e : 0, in, nxt, cls, stepping, resetting, off_s, off_sa);
+}
+
 template <bool SERVER>
 __global__ void __launch_bounds__(kStepThreads) env_step_succ_kernel(const colo_mdp_tables tb, const StepIO io) {
   const long long n_thr = (long long)gridDim.x * kStepThreads;
@@ -697,64 +743,129 @@ __global__ void __launch_bounds__(kStepThreads) env_step_succ_kernel(const colo_
     t_pass += pass - io.srv_seq0 - 1;
   }
   for (long long e = (long long)blockIdx.x * kStepThreads + threadIdx.x; e < n_pad; e += n_thr)
-  for (int step = 0; step < io.n_steps; ++step) {  // an env is owned by the same thread for every step of the launch
-    const bool valid = e < io.N;
-    EnvIn in;
-    in.s = 0; in.a = 0; in.st = COLO_STEP_MID; in.h = 0; in.bad = 0; in.un64 = 0.0; in.un32 = 0.f; in.ur = 0.f;
-    if (valid) in = load_env<false>(io, tb, e, t_pass + step);
-    const bool is_last = valid && in.st == COLO_STEP_LAST;
-    const bool resetting = is_last && io.auto_reset;
-    const bool stepping = valid && !is_last && !in.bad;
-    if (is_last && !io.auto_reset && io.status) *io.status = COLO_NEEDS_RESET;
-    int nxt = 0, cls = 0;
-    if (stepping) {
-      const size_t sa = (size_t)in.s * tb.A + in.a;
-      const size_t base = sa * tb.Ksucc;
-      const int n = __ldg(tb.succ_len + sa);
-      int pos = 0;
-      if (n > 1) {
-        const double total = __ldg(tb.succ_cum + base + n - 1) + 0.0;
-        pos = bisect_count(tb.succ_cum + base, n, in.un64 * total);
-      }
-      nxt = __ldg(tb.succ_idx + base + pos);
-      cls = tb.rew_cls_succ ? __ldg(tb.rew_cls_succ + base + pos) : 0;
-    }
-    finish_env(io, tb, valid ? e : 0, in, nxt, cls, stepping, resetting);
-  }
+  for (int step = 0; step < io.n_steps; ++step)  // an env is owned by the same thread for every step of the launch
+    succ_env_step(io, tb, e, e < io.N, t_pass + step, io.seed, io.env0 + (uint64_t)e, 0, 0);
   if (!SERVER) return;
   server_done(io, pass);
   }
 }
 
+// BaseMDP.reset of one env (valid); returns its start state
+__device__ __forceinline__ int reset_env(const StepIO& io, const colo_mdp_tables& tb, long long e,
+                                         unsigned long long seed, unsigned long long ctr) {
+  const double* u_next = reinterpret_cast<const double*>(io.u_next);
+  double u;
+  if (u_next)
+    u = u_next[e];
+  else {
+    Philox4 w = philox4x32_10(seed, ctr, io.t);
+    u = u53(w.w[0], w.w[1]);
+  }
+  const int s0 = sample_start(tb, u);
+  io.state[e] = s0;
+  io.h[e] = 0;
+  io.step_type[e] = COLO_STEP_FIRST;
+  if (io.step_type_mirror) io.step_type_mirror[e] = COLO_STEP_FIRST;
+  if (io.discount) io.discount[e] = __int_as_float(0x7fc00000);
+  if (io.reward) io.reward[e] = __int_as_float(0x7fc00000);  // the reference's reward of a FIRST TimeStep is None
+  if (io.io_compact)
+    reinterpret_cast<short*>(io.obs)[e] = (short)s0;
+  else
+    io.obs[e] = s0;
+  return s0;
+}
+
 __global__ void __launch_bounds__(kStepThreads) env_reset_kernel(const colo_mdp_tables tb, const StepIO io) {
   const long long n_thr = (long long)gridDim.x * kStepThreads;
   const long long n_pad = (io.N + 31) & ~31LL;
-  const double* u_next = reinterpret_cast<const double*>(io.u_next);
   for (long long e = (long long)blockIdx.x * kStepThreads + threadIdx.x; e < n_pad; e += n_thr) {
     const bool valid = e < io.N;
-    int s0 = 0;
-    if (valid) {
-      double u;
-      if (u_next)
-        u = u_next[e];
-      else {
-        Philox4 w = philox4x32_10(io.seed, io.env0 + (uint64_t)e, io.t);
-        u = u53(w.w[0], w.w[1]);
-      }
-      s0 = sample_start(tb, u);
-      io.state[e] = s0;
-      io.h[e] = 0;
-      io.step_type[e] = COLO_STEP_FIRST;
-      if (io.step_type_mirror) io.step_type_mirror[e] = COLO_STEP_FIRST;
-      if (io.discount) io.discount[e] = __int_as_float(0x7fc00000);
-      if (io.reward) io.reward[e] = __int_as_float(0x7fc00000);  // the reference's reward of a FIRST TimeStep is None
-      if (io.io_compact)
-        reinterpret_cast<short*>(io.obs)[e] = (short)s0;
-      else
-        io.obs[e] = s0;
-    }
+    const int s0 = valid ? reset_env(io, tb, e, io.seed, io.env0 + (uint64_t)e) : 0;
     const long long copy = blockIdx.x & io.visits_mask;
     if (io.visits_s) aggregated_inc(io.visits_s + copy * io.n_s, s0, valid);
+  }
+}
+
+// ---- mixed batches (colo_mixed_tables): envs of different MDP instances in one launch ---------------------------------
+// Instance i owns the contiguous envs [start, start + n_i).  Env e looks up its instance in inst_of[e] and then runs the
+// per-env code above on that instance's tables, Philox key and counter (seed_i; e - start), and counter offsets.  Envs of
+// one instance are contiguous, so the lanes of a warp almost always read the same descriptor (one broadcast load).
+struct MixedInst {
+  colo_mdp_tables tb;
+  unsigned long long seed;
+  long long start;          // first env of the instance
+  long long off_s, off_sa;  // sum of S, of S*A over the instances before it: its columns in the counter rows
+};
+
+__device__ __forceinline__ int mixed_inst_of(const int* __restrict__ inst_of, long long e, bool valid) {
+  return valid ? __ldg(inst_of + e) : 0;  // lanes past the batch take part in the warp collectives as instance 0
+}
+
+__global__ void __launch_bounds__(kStepThreads) env_reset_mixed_kernel(const MixedInst* __restrict__ insts,
+                                                                      const int* __restrict__ inst_of, const StepIO io) {
+  const long long n_thr = (long long)gridDim.x * kStepThreads;
+  const long long n_pad = (io.N + 31) & ~31LL;
+  for (long long e = (long long)blockIdx.x * kStepThreads + threadIdx.x; e < n_pad; e += n_thr) {
+    const bool valid = e < io.N;
+    const MixedInst d = insts[mixed_inst_of(inst_of, e, valid)];
+    const int s0 = valid ? reset_env(io, d.tb, e, d.seed, (unsigned long long)(e - d.start)) : 0;
+    const long long copy = blockIdx.x & io.visits_mask;
+    if (io.visits_s) aggregated_inc(io.visits_s + copy * io.n_s, d.off_s + s0, valid);
+  }
+}
+
+__global__ void __launch_bounds__(kStepThreads) env_step_succ_mixed_kernel(const MixedInst* __restrict__ insts,
+                                                                          const int* __restrict__ inst_of, const StepIO io) {
+  const long long n_thr = (long long)gridDim.x * kStepThreads;
+  const long long n_pad = (io.N + 31) & ~31LL;
+  for (long long e = (long long)blockIdx.x * kStepThreads + threadIdx.x; e < n_pad; e += n_thr) {
+    const bool valid = e < io.N;
+    const MixedInst d = insts[mixed_inst_of(inst_of, e, valid)];
+    for (int step = 0; step < io.n_steps; ++step)
+      succ_env_step(io, d.tb, e, valid, io.t + step, d.seed, (unsigned long long)(e - d.start), d.off_s, d.off_sa);
+  }
+}
+
+// the warp-per-env dense search of env_step_dense_kernel, every env searching its own instance's row
+template <typename TC, int NCH>
+__global__ void __launch_bounds__(kStepThreads) env_step_dense_mixed_kernel(const MixedInst* __restrict__ insts,
+                                                                           const int* __restrict__ inst_of, const StepIO io) {
+  const int lane = threadIdx.x & 31;
+  const long long warp_global = ((long long)blockIdx.x * kStepThreads + threadIdx.x) >> 5;
+  const long long n_warps = ((long long)gridDim.x * kStepThreads) >> 5;
+  const long long n_tiles = (io.N + 31) >> 5;
+  constexpr bool F32U = sizeof(TC) == 4;
+  for (long long tile = warp_global; tile < n_tiles; tile += n_warps) {
+    const long long e = tile * 32 + lane;
+    const bool valid = e < io.N;
+    const MixedInst d = insts[mixed_inst_of(inst_of, e, valid)];
+    const TC* __restrict__ cdf = reinterpret_cast<const TC*>(d.tb.cdf);
+    for (int step = 0; step < io.n_steps; ++step) {
+      EnvIn in;
+      in.s = 0; in.a = 0; in.st = COLO_STEP_MID; in.h = 0; in.bad = 0; in.un64 = 0.0; in.un32 = 0.f; in.ur = 0.f;
+      if (valid) in = load_env<F32U>(io, d.tb, e, io.t + step, d.seed, (unsigned long long)(e - d.start));
+      const bool is_last = valid && in.st == COLO_STEP_LAST;
+      const bool resetting = is_last && io.auto_reset;
+      const bool stepping = valid && !is_last && !in.bad;
+      if (is_last && !io.auto_reset && io.status) *io.status = COLO_NEEDS_RESET;
+      // lanes that do not step search row 0 of their instance; every lane hands the warp its own row and shape
+      const TC* row_l = cdf + (stepping ? ((size_t)in.s * d.tb.A + in.a) * d.tb.ld : 0);
+      const TC u_l = F32U ? (TC)in.un32 : (TC)in.un64;
+      int my_next = 0;
+      for (int i0 = 0; i0 < 32; i0 += kEnvUnroll) {
+#pragma unroll
+        for (int k = 0; k < kEnvUnroll; ++k) {
+          const int i = i0 + k;
+          const TC* row = reinterpret_cast<const TC*>(__shfl_sync(FULL, (unsigned long long)row_l, i));
+          const int S_i = __shfl_sync(FULL, d.tb.S, i), ld_i = __shfl_sync(FULL, d.tb.ld, i);
+          const TC u_i = __shfl_sync(FULL, u_l, i);
+          const int nxt = warp_row_next<TC, NCH>(row, S_i, ld_i, u_i, lane);
+          if (lane == i) my_next = nxt;
+        }
+      }
+      const int cls = stepping ? dense_cls(d.tb, in, my_next) : 0;
+      finish_env(io, d.tb, valid ? e : 0, in, my_next, cls, stepping, resetting, d.off_s, d.off_sa);
+    }
   }
 }
 
@@ -1028,6 +1139,158 @@ int colo_env_random_steps(const colo_mdp_tables* tb, const colo_env_batch* batch
   if (mode == 0) return colo::launch_dense<float, false>(tb, io, stream);
   if (mode == 1) return colo::launch_dense<double, false>(tb, io, stream);
   return colo::launch_succ<false>(tb, io, stream);
+}
+
+// ---- mixed batches ------------------------------------------------------------------------------------------------------
+struct colo_mixed_tables {
+  int n_inst, mode;
+  long long N, sum_s, sum_sa;
+  colo::MixedInst* insts;  // device [n_inst]
+  int* inst_of;            // device [N]: instance of every env
+};
+
+static int mixed_check_instance(const colo_mdp_tables* tb, int mode) {
+  int r = colo::check_tables_common(tb);
+  if (r != COLO_OK) return r;
+  if (mode == 2) {
+    COLO_ARG_CHECK(tb->succ_cum && tb->succ_idx && tb->succ_len && tb->Ksucc > 0, "successor tables");
+  } else {
+    COLO_ARG_CHECK(tb->cdf && tb->ld >= tb->S && tb->ld % 4 == 0, "dense cdf with ld % 4 == 0 is required");
+    COLO_ARG_CHECK((uintptr_t)tb->cdf % 16 == 0, "cdf must be 16-byte aligned");
+  }
+  return COLO_OK;
+}
+
+void colo_mixed_tables_destroy(colo_mixed_tables* h) {
+  if (!h) return;
+  if (h->insts) cudaFree(h->insts);
+  if (h->inst_of) cudaFree(h->inst_of);
+  free(h);
+}
+
+int colo_mixed_tables_create(const colo_mdp_tables* host_tables, int n_inst, const long long* n_envs,
+                             const unsigned long long* seeds, int mode, void* stream, colo_mixed_tables** out) {
+  COLO_ARG_CHECK(out && host_tables && n_envs && seeds, "host_tables, n_envs, seeds, out");
+  COLO_ARG_CHECK(n_inst >= 1, "colo_mixed_tables_create: n_inst >= 1");
+  COLO_ARG_CHECK(mode >= 0 && mode <= 2, "mode in {0,1,2}");
+  // every instance is validated before anything touches the device
+  std::vector<colo::MixedInst> insts((size_t)n_inst);
+  long long N = 0, sum_s = 0, sum_sa = 0;
+  for (int i = 0; i < n_inst; ++i) {
+    if (mixed_check_instance(&host_tables[i], mode) != COLO_OK) {
+      char why[256];
+      snprintf(why, sizeof(why), "%s", colo_last_error());
+      colo::set_error("colo_mixed_tables_create: instance %d: %s", i, why);
+      return COLO_ERR_ARG;
+    }
+    if (n_envs[i] < 1) {
+      colo::set_error("colo_mixed_tables_create: instance %d: n_envs %lld < 1", i, n_envs[i]);
+      return COLO_ERR_ARG;
+    }
+    colo::MixedInst& d = insts[(size_t)i];
+    d.tb = host_tables[i];
+    d.seed = seeds[i];
+    d.start = N;
+    d.off_s = sum_s;
+    d.off_sa = sum_sa;
+    N += n_envs[i];
+    sum_s += host_tables[i].S;
+    sum_sa += (long long)host_tables[i].S * host_tables[i].A;
+  }
+  COLO_ARG_CHECK(N < (1LL << 31), "colo_mixed_tables_create: fewer than 2^31 envs in all");
+  std::vector<int> inst_of((size_t)N);
+  for (int i = 0; i < n_inst; ++i)
+    for (long long e = insts[(size_t)i].start; e < insts[(size_t)i].start + n_envs[i]; ++e) inst_of[(size_t)e] = i;
+  colo_mixed_tables* h = (colo_mixed_tables*)calloc(1, sizeof(colo_mixed_tables));
+  COLO_ARG_CHECK(h != nullptr, "out of host memory");
+  h->n_inst = n_inst;
+  h->mode = mode;
+  h->N = N;
+  h->sum_s = sum_s;
+  h->sum_sa = sum_sa;
+  cudaStream_t st = (cudaStream_t)stream;
+  cudaError_t e = cudaMalloc((void**)&h->insts, sizeof(colo::MixedInst) * (size_t)n_inst);
+  if (e == cudaSuccess) e = cudaMalloc((void**)&h->inst_of, sizeof(int) * (size_t)N);
+  if (e == cudaSuccess)
+    e = cudaMemcpyAsync(h->insts, insts.data(), sizeof(colo::MixedInst) * (size_t)n_inst, cudaMemcpyHostToDevice, st);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(h->inst_of, inst_of.data(), sizeof(int) * (size_t)N, cudaMemcpyHostToDevice, st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);  // the host staging vectors die with this call
+  if (e != cudaSuccess) {
+    colo::set_error("colo_mixed_tables_create: %s", cudaGetErrorString(e));
+    colo_mixed_tables_destroy(h);
+    return COLO_ERR_CUDA;
+  }
+  *out = h;
+  return COLO_OK;
+}
+
+long long colo_mixed_visits_size(const colo_mixed_tables* h, int pairs) {
+  return h == nullptr ? 0 : (pairs ? h->sum_sa : h->sum_s);
+}
+
+static int make_mixed_io(const colo_mixed_tables* h, const colo_env_batch* b, int random_actions, const void* u_next,
+                         const float* u_rew, unsigned long long t, int auto_reset, colo::StepIO* io) {
+  COLO_ARG_CHECK(h != nullptr && b != nullptr, "mixed tables, batch");
+  if (b->N != h->N) {
+    colo::set_error("bad argument: batch N = %lld, the mixed tables hold %lld envs", b->N, h->N);
+    return COLO_ERR_ARG;
+  }
+  COLO_ARG_CHECK(!b->io_compact, "mixed batches have no compact I/O");
+  colo_mdp_tables shape;
+  memset(&shape, 0, sizeof(shape));
+  shape.S = shape.A = 1;
+  const int r = make_io(&shape, b, random_actions, u_next, u_rew, t, auto_reset, io);
+  if (r != COLO_OK) return r;
+  io->n_s = h->sum_s;  // counter rows are the concatenation of the instances' rows
+  io->n_sa = h->sum_sa;
+  io->seed = io->env0 = 0;  // every env takes its key and counter from its instance
+  return COLO_OK;
+}
+
+int colo_mixed_env_reset(const colo_mixed_tables* h, const colo_env_batch* batch, const double* u_next,
+                         unsigned long long t, void* stream) {
+  colo::StepIO io;
+  const int r = make_mixed_io(h, batch, 0, u_next, nullptr, t, 0, &io);
+  if (r != COLO_OK) return r;
+  colo::env_reset_mixed_kernel<<<colo::grid_for(colo::kStepThreads, io.N), colo::kStepThreads, 0, (cudaStream_t)stream>>>(
+      h->insts, h->inst_of, io);
+  return colo::check_launch("env_reset_mixed_kernel");
+}
+
+static int launch_mixed(const colo_mixed_tables* h, const colo::StepIO& io, void* stream) {
+  COLO_ARG_CHECK(io.reward && io.action, "env buffers");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (h->mode == 2) {
+    colo::env_step_succ_mixed_kernel<<<colo::grid_for(colo::kStepThreads, io.N), colo::kStepThreads, 0, st>>>(
+        h->insts, h->inst_of, io);
+    colo::count_step_launch(COLO_STEP_KIND_MIXED_SUCC);
+    return colo::check_launch("env_step_succ_mixed_kernel");
+  }
+  const int grid = colo::grid_for(colo::kStepThreads / 32, (io.N + 31) / 32);
+  if (h->mode == 0)
+    colo::env_step_dense_mixed_kernel<float, 8><<<grid, colo::kStepThreads, 0, st>>>(h->insts, h->inst_of, io);
+  else
+    colo::env_step_dense_mixed_kernel<double, 8><<<grid, colo::kStepThreads, 0, st>>>(h->insts, h->inst_of, io);
+  colo::count_step_launch(COLO_STEP_KIND_MIXED_DENSE);
+  return colo::check_launch("env_step_dense_mixed_kernel");
+}
+
+int colo_mixed_env_step(const colo_mixed_tables* h, const colo_env_batch* batch, int random_actions,
+                        const void* u_next, const float* u_rew, unsigned long long t, int auto_reset, void* stream) {
+  colo::StepIO io;
+  const int r = make_mixed_io(h, batch, random_actions, u_next, u_rew, t, auto_reset, &io);
+  if (r != COLO_OK) return r;
+  return launch_mixed(h, io, stream);
+}
+
+int colo_mixed_env_random_steps(const colo_mixed_tables* h, const colo_env_batch* batch, int n_steps,
+                                unsigned long long t0, int auto_reset, void* stream) {
+  COLO_ARG_CHECK(n_steps >= 1, "n_steps >= 1");
+  colo::StepIO io;
+  const int r = make_mixed_io(h, batch, 1, nullptr, nullptr, t0, auto_reset, &io);
+  if (r != COLO_OK) return r;
+  io.n_steps = n_steps;
+  return launch_mixed(h, io, stream);
 }
 
 struct colo_env_stepper {

@@ -65,7 +65,9 @@ unsigned long long colo_backup_tma_sweeps(void);
 #define COLO_STEP_KIND_SHORT 2 /* env_step_dense_short_kernel: the warp-cooperative kernel (COLO_STEP_KERNEL=coop) */
 #define COLO_STEP_KIND_LONG 3  /* env_step_dense_kernel: rows of more than 1024 states (or ld % 128 != 0)      */
 #define COLO_STEP_KIND_SUCC 4  /* env_step_succ_kernel: successor-list tables                                  */
-#define COLO_STEP_KINDS 5
+#define COLO_STEP_KIND_MIXED_SUCC 5  /* env_step_succ_mixed_kernel: a mixed batch, successor-list tables       */
+#define COLO_STEP_KIND_MIXED_DENSE 6 /* env_step_dense_mixed_kernel: a mixed batch, dense rows (f32 or f64)   */
+#define COLO_STEP_KINDS 7
 unsigned long long colo_step_kernel_launches(int kind);
 
 /* ---------------------------------------------------------------- (B) Bellman backups ------------------- */
@@ -574,6 +576,41 @@ int colo_emit_noise_correlated(float* out, const unsigned char* step_type, const
 int colo_env_step_succ(const colo_mdp_tables* tb, const colo_env_batch* batch, int random_actions,
                        const double* u_next, const float* u_rew, unsigned long long t, int auto_reset,
                        void* stream);
+
+/*
+ * Mixed batches -- one batch whose envs belong to different MDP instances (e.g. a benchmark's parameter sets x seeds),
+ * advanced by ONE launch per reset / step / fused random steps whatever the number of instances.
+ *   Layout: instance i owns the contiguous envs [start_i, start_i + n_envs[i]), in instance order; N = sum n_envs[i].
+ *   Semantics: per env, those of colo_env_reset / colo_env_step_* / colo_env_random_steps on the env's OWN instance
+ *   (start distribution, sampler, reward classes and quantiles, rewards_range, H -- episodic and continuous instances
+ *   may share a batch --, auto-reset, obs = state index within the instance, random actions in [0, A_i)).
+ *   Philox: env e of instance i uses key seeds[i] and counter (e - start_i, t): segment i is bit-identical to a
+ *   single-MDP batch of instance i with seed = seeds[i], env0 = 0, driven by the same calls.
+ *   colo_env_batch is reused as is: N must equal sum n_envs[i] (COLO_ERR_ARG otherwise); its `seed` and `env0` are NOT
+ *   used (the seeds live in the handle); io_compact must be 0.  Visitation counters: visits_s [copies][sum S] and
+ *   visits_sa [copies][sum S*A], instance i's columns starting at sum_{j<i} S_j (sum_{j<i} S_j*A_j) --
+ *   colo_mixed_visits_size gives one copy's length (pairs = 0: sum S, pairs != 0: sum S*A).
+ *   An action outside [0, A_i) sets COLO_BAD_ACTION in `status` and leaves that env untouched.
+ * colo_mixed_tables_create -- host_tables[n_inst]: each instance's tables (device pointers inside, as for the
+ *   single-MDP calls; they must outlive the handle); n_envs[n_inst] >= 1; seeds[n_inst]; mode 0 dense f32 rows, 1 dense
+ *   f64 rows (rows may have a different ld per instance), 2 successor tables (every instance needs the mode's tables).
+ *   Validates every instance before touching the device (COLO_ERR_ARG, colo_last_error names the instance), then
+ *   uploads the per-instance descriptors and an env -> instance map on `stream` and synchronises it.
+ * colo_mixed_env_step -- u_next: float[N] for mode 0, double[N] otherwise, or NULL; u_rew float[N] or NULL.
+ * Dense mixed batches use the general warp-per-env search (the short-row specialisations are single-MDP); host I/O,
+ * the pipelines, the step server and emission maps are single-MDP only.
+ */
+typedef struct colo_mixed_tables colo_mixed_tables;
+int colo_mixed_tables_create(const colo_mdp_tables* host_tables, int n_inst, const long long* n_envs,
+                             const unsigned long long* seeds, int mode, void* stream, colo_mixed_tables** out);
+void colo_mixed_tables_destroy(colo_mixed_tables* h);
+long long colo_mixed_visits_size(const colo_mixed_tables* h, int pairs);
+int colo_mixed_env_reset(const colo_mixed_tables* h, const colo_env_batch* batch, const double* u_next,
+                         unsigned long long t, void* stream);
+int colo_mixed_env_step(const colo_mixed_tables* h, const colo_env_batch* batch, int random_actions,
+                        const void* u_next, const float* u_rew, unsigned long long t, int auto_reset, void* stream);
+int colo_mixed_env_random_steps(const colo_mixed_tables* h, const colo_env_batch* batch, int n_steps,
+                                unsigned long long t0, int auto_reset, void* stream);
 
 /*
  * Prepared step -- the same launch as colo_env_step_* (auto_reset on, in-kernel Philox uniforms, supplied actions) with
