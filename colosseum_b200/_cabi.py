@@ -15,6 +15,7 @@ STEP_FIRST, STEP_MID, STEP_LAST = 0, 1, 2
 # step-kernel variants of colo_step_kernel_launches (include/colosseum_b200.h, COLO_STEP_KIND_*)
 STEP_KIND_LEAN, STEP_KIND_KARY, STEP_KIND_SHORT, STEP_KIND_LONG, STEP_KIND_SUCC = 0, 1, 2, 3, 4
 STEP_KIND_MIXED_SUCC, STEP_KIND_MIXED_DENSE = 5, 6
+STEP_KIND_BREAKS, STEP_KIND_BREAKS_GENERAL = 7, 8
 
 
 class ColosseumB200Error(RuntimeError):
@@ -54,6 +55,7 @@ class MdpTables(C.Structure):
         ("rmin", C.c_float), ("rmax", C.c_float),
         ("start_cum", C.c_void_p), ("start_idx", C.c_void_p), ("n_start", C.c_int),
         ("cdf_mid", C.c_void_p), ("cdf_coarse", C.c_void_p), ("rew_cls_pad", C.c_void_p),
+        ("cdf_breaks", C.c_void_p), ("cdf_breaks_k", C.c_int),
     ]
 
 
@@ -270,6 +272,8 @@ PROTOTYPES = {
     "colo_emit_observations": (_I, [_P, _P, _P, _P, _LL, _I, _I, _I, _P, _P]),
     "colo_build_dense_cdf": (_I, [_P, _I, _I, _I, _P, _I, _P]),
     "colo_build_cdf_index": (_I, [_P, _I, _I, _I, _I, _P, _P, _P]),
+    "colo_count_cdf_breaks": (_I, [_P, _I, _I, _I, C.POINTER(C.c_int), _P]),
+    "colo_build_cdf_breaks": (_I, [C.POINTER(MdpTables), _I, _P, _P]),
     "colo_extended_vi_work_bytes": (C.c_size_t, [_I, _I]),
     "colo_extended_vi_f32": (_I, [_P, _P, _P, _P, _I, _I, _D, _D, _LL, _P, _P, _P, _P, _P]),
     "colo_extended_vi_f64acc": (_I, [_P, _P, _P, _P, _I, _I, _D, _D, _LL, _P, _P, _P, _P, _P]),

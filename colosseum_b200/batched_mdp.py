@@ -25,9 +25,15 @@ _MODES = {"dense_f32": 0, "dense_f64": 1, "succ": 2}
 
 
 class DeviceTables:
-    """MDPTables uploaded to the current CUDA device + the `colo_mdp_tables` struct pointing at them."""
+    """MDPTables uploaded to the current CUDA device + the `colo_mdp_tables` struct pointing at them.
 
-    def __init__(self, tb: MDPTables, mode: str):
+    breaks=True: for dense_f32 rows of <= 1024 states with at most 16 breakpoints each (CDF entries above their
+    predecessor) and at most one per 8 states, also the breakpoint table the f32 step kernels search in one round
+    instead of the row (`colo_mdp_tables.cdf_breaks`); `breaks_k` is its entries per row (0: none)."""
+
+    BREAKS_K = (2, 4, 8, 16)
+
+    def __init__(self, tb: MDPTables, mode: str, breaks: bool = True):
         import torch
 
         _cabi.require_cuda()
@@ -82,6 +88,19 @@ class DeviceTables:
         for name in ("cdf", "succ_cum", "succ_idx", "succ_len", "rew_cls_sas", "rew_cls_sa", "rew_cls_succ", "rew_q",
                      "start_cum", "start_idx", "cdf_mid", "cdf_coarse", "rew_cls_pad"):
             setattr(c, name, _cabi.ptr(k.get(name)))
+        self.breaks_k = 0
+        if breaks and mode == "dense_f32" and short_rows:
+            m = C.c_int(0)
+            rc = _cabi.lib().colo_count_cdf_breaks(_cabi.ptr(k["cdf"]), tb.S, tb.A, ld, C.byref(m), _cabi.current_stream())
+            _cabi.check(rc, "colo_count_cdf_breaks")
+            # the density rule of the compressed-row kernels: rows denser than 1 in 8 keep the k-ary row search
+            if m.value <= self.BREAKS_K[-1] and 8 * m.value <= tb.S:
+                K = next(x for x in self.BREAKS_K if x >= m.value)
+                k["cdf_breaks"] = torch.empty((tb.S, tb.A, K, 4), dtype=torch.int32, device=dev)
+                rc = _cabi.lib().colo_build_cdf_breaks(C.byref(c), K, _cabi.ptr(k["cdf_breaks"]), _cabi.current_stream())
+                _cabi.check(rc, "colo_build_cdf_breaks")
+                c.cdf_breaks, c.cdf_breaks_k = _cabi.ptr(k["cdf_breaks"]), K
+                self.breaks_k = K
         self.keep = k
         self.c = c
 
@@ -638,11 +657,12 @@ class MixedBatchedMDP:
         self._sa_off = np.concatenate([[0], np.cumsum(self.n_states * self.n_actions)]).astype(np.int64)
         # the single-MDP upload, reused as is: in the dense modes it also builds the short-row search index (cdf_mid,
         # cdf_coarse, rew_cls_pad) for rows of <= 1024 states, which the mixed kernels do not read -- a few build
-        # launches per instance at construction and up to about half the bytes of an f32 dense CDF again
+        # launches per instance at construction and up to about half the bytes of an f32 dense CDF again.  The
+        # breakpoint table, which they do not read either, is not built.
         self.dev = []
         for i, tb in enumerate(self.tables):
             try:
-                self.dev.append(DeviceTables(tb, mode))
+                self.dev.append(DeviceTables(tb, mode, breaks=False))
             except AssertionError as e:
                 raise AssertionError(f"instance {i}: {e}") from None
         self._c_tables = (_cabi.MdpTables * n)(*[d.c for d in self.dev])

@@ -250,9 +250,10 @@ __device__ __forceinline__ EnvIn load_env(const StepIO& io, const colo_mdp_table
 
 // epilogue of a regular step for one env held by this thread.  off_s / off_sa: where the env's MDP starts in the
 // counter rows (non-zero in a mixed batch, whose instances share one concatenated [copies][sum S] / [copies][sum S*A])
+// have_rew: `rew` is the reward of the step (a constant class resolved by the breakpoint table), no draw needed
 __device__ __forceinline__ void finish_env(const StepIO& io, const colo_mdp_tables& tb, long long e, const EnvIn& in,
                                            int nxt, int cls, bool stepping, bool resetting, long long off_s = 0,
-                                           long long off_sa = 0) {
+                                           long long off_sa = 0, bool have_rew = false, float rew = 0.f) {
   if (resetting) {  // auto_reset path == BaseMDP.reset(): the action is ignored, reward is None (NaN here)
     nxt = sample_start(tb, in.un64);
     io.state[e] = nxt;
@@ -266,7 +267,7 @@ __device__ __forceinline__ void finish_env(const StepIO& io, const colo_mdp_tabl
     const int hh = in.h + 1;
     io.h[e] = hh;
     io.state[e] = nxt;
-    io.reward[e] = reward_draw(tb, cls, in.ur);
+    io.reward[e] = have_rew ? rew : reward_draw(tb, cls, in.ur);
     if (io.random_actions) io.action[e] = in.a;
     const bool last = tb.H > 0 && hh >= tb.H;
     const unsigned char st = last ? COLO_STEP_LAST : COLO_STEP_MID;
@@ -480,6 +481,54 @@ __global__ void __launch_bounds__(kStepThreads) env_step_dense_short_kernel(cons
   }
 }
 
+// ---- breakpoint table (colo_mdp_tables.cdf_breaks) ----------------------------------------------------------------------
+// Most benchmark rows have a handful of successors, so the CDF row is a step function with a few breakpoints p_k (where
+// c[p_k] > c[p_k - 1]).  For x >= 0 the count of entries <= x over the whole padded row, with the clamp to the first
+// index reaching the total, is p_min(k*, m-1), k* = #{k : v_k <= x}: one 16-byte entry per breakpoint carries the whole
+// step (next state, its reward class, and the reward itself when the class's quantile row is constant).  A row of K
+// entries is read in ONE round of K independent loads (K = 2: one 32-byte sector), instead of the three dependent rounds
+// of the two-level index plus a fourth for the reward quantiles.
+struct CdfBreak {
+  float v;             // c[p]
+  int p;               // the breakpoint: the next state
+  unsigned cls_flags;  // reward class of (s, a, p) | kBreakInline
+  float r;             // the reward, when kBreakInline
+};
+constexpr unsigned kBreakInline = 0x80000000u;
+
+struct BreakStep {
+  int nxt, cls;
+  float rew;
+  bool have_cls, have_rew;
+};
+
+// the step of row r for uniform u (x = u * total, total = v of the last entry), from its K breakpoint entries; x not >= 0
+// (supplied uniforms: negative, NaN) finds no entry <= x, i.e. state 0, whose class the caller looks up (have_cls false)
+template <int K>
+__device__ __forceinline__ BreakStep breaks_step(const void* table, unsigned r, float u) {
+  const int4* __restrict__ row = reinterpret_cast<const int4*>(table) + (size_t)r * K;
+  int4 e[K];
+#pragma unroll
+  for (int k = 0; k < K; ++k) e[k] = __ldg(row + k);
+  const float x = u * __int_as_float(e[K - 1].x);
+  BreakStep b;
+  b.nxt = 0; b.cls = 0; b.rew = 0.f; b.have_cls = false; b.have_rew = false;
+  if (!(x >= 0.f)) return b;
+  int ks = 0;
+#pragma unroll
+  for (int k = 0; k < K; ++k) ks += __int_as_float(e[k].x) <= x;
+  ks = min(ks, K - 1);  // x >= total: the last breakpoint (the padding repeats it)
+  int4 sel = e[0];
+#pragma unroll
+  for (int k = 1; k < K; ++k) sel = k == ks ? e[k] : sel;
+  b.nxt = sel.y;
+  b.cls = (int)((unsigned)sel.z & ~kBreakInline);
+  b.have_cls = true;
+  b.have_rew = ((unsigned)sel.z & kBreakInline) != 0u;
+  b.rew = __int_as_float(sel.w);
+  return b;
+}
+
 // SHORT rows, one THREAD per env: a three-round k-ary search instead of reading the whole row.  The last entries of
 // the row's quads are monotone, so the number G of quads lying entirely at or below x is found from (1) the last entry
 // of every 8th quad (4*NCH independent 4-byte loads, all issued before any is consumed), (2) the last entries of the 8
@@ -492,7 +541,8 @@ __global__ void __launch_bounds__(kStepThreads) env_step_dense_short_kernel(cons
 // -- 5.58 us per step instead of 5.17: four sectors cost more than one extra round; fetching the reward quantiles of
 // every class before the search -- 5.50 us instead of 5.26.)  With 65,536 envs every warp is resident at once, so the step time IS the length of
 // that dependency chain.  Same comparisons against the same x => the same index, bit for bit.
-template <typename TC, int NCH, bool SERVER>
+// KB > 0 (f32): the search is one round over the KB-entry breakpoint row instead (NCH is then unused).
+template <typename TC, int NCH, bool SERVER, int KB = 0>
 __global__ void __launch_bounds__(kStepThreads) env_step_dense_kary_kernel(const colo_mdp_tables tb, const StepIO io) {
   const long long n_thr = (long long)gridDim.x * kStepThreads;
   const long long n_pad = (io.N + 31) & ~31LL;  // whole warps: finish_env uses warp collectives
@@ -519,72 +569,84 @@ __global__ void __launch_bounds__(kStepThreads) env_step_dense_kary_kernel(const
     const bool stepping = valid && !is_last && !in.bad;
     if (is_last && !io.auto_reset && io.status) *io.status = COLO_NEEDS_RESET;
     int nxt = 0, cls = 0;
+    bool have_rew = false;
+    float rew = 0.f;
     if (stepping) {
-      const TC* row = cdf + (size_t)(unsigned)(in.s * A + in.a) * (unsigned)ld;
-      TC total, x;
-      int blk = 0, G = 0;
       bool have_cls = false;
-      uint4 c0 = make_uint4(0, 0, 0, 0), c1 = c0;
-      nxt = ld;
-      if (coarse) {  // two-level index: NCH 128-bit loads of a small hot table, then the 8 quad ends of one block
-        const unsigned r = (unsigned)(in.s * A + in.a);
-        Quad<TC> cq[NCH];
-#pragma unroll
-        for (int k = 0; k < NCH; ++k) cq[k].load(coarse + (size_t)r * NB + 4 * k);
-        total = cq[NCH - 1].v[3];  // row[ld-1]: the padding [S, ld) holds the row total, i.e. the value of row[S-1]
-        x = (F32U ? (TC)in.un32 : (TC)in.un64) * total;
-#pragma unroll
-        for (int k = 0; k < NCH; ++k) blk += (cq[k].v[0] <= x) + (cq[k].v[1] <= x) + (cq[k].v[2] <= x) + (cq[k].v[3] <= x);
-        if (blk < NB) {
-          // round 2: the 8 quad ends of the block (one 32-byte sector of cdf_mid) and, in the same round, the reward
-          // classes of the block's 32 candidate next states (rew_cls_pad: rew_cls_sas with rows padded to ld, so the
-          // slice is one aligned 32-byte sector): the class lookup no longer waits for the search to finish
-          Quad<TC> m0, m1;
-          const TC* mp = mid + (size_t)r * (32 * NCH) + 8 * blk;
-          m0.load(mp);
-          m1.load(mp + 4);
-          if (tb.rew_cls_pad) {
-            const uint4* cp = reinterpret_cast<const uint4*>(tb.rew_cls_pad + (size_t)r * ld + 32 * blk);
-            c0 = __ldg(cp);
-            c1 = __ldg(cp + 1);
-          }
-          G = 8 * blk + (m0.v[0] <= x) + (m0.v[1] <= x) + (m0.v[2] <= x) + (m0.v[3] <= x) + (m1.v[0] <= x) +
-              (m1.v[1] <= x) + (m1.v[2] <= x) + (m1.v[3] <= x);
-        }
+      if constexpr (KB > 0) {
+        const BreakStep b = breaks_step<KB>(tb.cdf_breaks, (unsigned)(in.s * A + in.a), in.un32);
+        nxt = b.nxt;
+        cls = b.cls;
+        have_cls = b.have_cls;
+        // a constant class gives its reward at every uniform in [0, 1] (supplied ones may lie outside)
+        have_rew = b.have_rew && in.ur >= 0.f && in.ur <= 1.f;
+        rew = b.rew;
       } else {
-        total = __ldg(row + S - 1);
-        x = (F32U ? (TC)in.un32 : (TC)in.un64) * total;
-        TC c[NB];
+        const TC* row = cdf + (size_t)(unsigned)(in.s * A + in.a) * (unsigned)ld;
+        TC total, x;
+        int blk = 0, G = 0;
+        uint4 c0 = make_uint4(0, 0, 0, 0), c1 = c0;
+        nxt = ld;
+        if (coarse) {  // two-level index: NCH 128-bit loads of a small hot table, then the 8 quad ends of one block
+          const unsigned r = (unsigned)(in.s * A + in.a);
+          Quad<TC> cq[NCH];
 #pragma unroll
-        for (int k = 0; k < NB; ++k) c[k] = __ldg(row + 32 * k + 31);  // last entry of quad 8k+7
+          for (int k = 0; k < NCH; ++k) cq[k].load(coarse + (size_t)r * NB + 4 * k);
+          total = cq[NCH - 1].v[3];  // row[ld-1]: the padding [S, ld) holds the row total, i.e. the value of row[S-1]
+          x = (F32U ? (TC)in.un32 : (TC)in.un64) * total;
 #pragma unroll
-        for (int k = 0; k < NB; ++k) blk += c[k] <= x ? 1 : 0;
+          for (int k = 0; k < NCH; ++k) blk += (cq[k].v[0] <= x) + (cq[k].v[1] <= x) + (cq[k].v[2] <= x) + (cq[k].v[3] <= x);
+          if (blk < NB) {
+            // round 2: the 8 quad ends of the block (one 32-byte sector of cdf_mid) and, in the same round, the reward
+            // classes of the block's 32 candidate next states (rew_cls_pad: rew_cls_sas with rows padded to ld, so the
+            // slice is one aligned 32-byte sector): the class lookup no longer waits for the search to finish
+            Quad<TC> m0, m1;
+            const TC* mp = mid + (size_t)r * (32 * NCH) + 8 * blk;
+            m0.load(mp);
+            m1.load(mp + 4);
+            if (tb.rew_cls_pad) {
+              const uint4* cp = reinterpret_cast<const uint4*>(tb.rew_cls_pad + (size_t)r * ld + 32 * blk);
+              c0 = __ldg(cp);
+              c1 = __ldg(cp + 1);
+            }
+            G = 8 * blk + (m0.v[0] <= x) + (m0.v[1] <= x) + (m0.v[2] <= x) + (m0.v[3] <= x) + (m1.v[0] <= x) +
+                (m1.v[1] <= x) + (m1.v[2] <= x) + (m1.v[3] <= x);
+          }
+        } else {
+          total = __ldg(row + S - 1);
+          x = (F32U ? (TC)in.un32 : (TC)in.un64) * total;
+          TC c[NB];
+#pragma unroll
+          for (int k = 0; k < NB; ++k) c[k] = __ldg(row + 32 * k + 31);  // last entry of quad 8k+7
+#pragma unroll
+          for (int k = 0; k < NB; ++k) blk += c[k] <= x ? 1 : 0;
+          if (blk < NB) {
+            const TC* b = row + 32 * blk;
+            TC q[8];
+#pragma unroll
+            for (int k = 0; k < 8; ++k) q[k] = __ldg(b + 4 * k + 3);
+            G = 8 * blk;
+#pragma unroll
+            for (int k = 0; k < 8; ++k) G += q[k] <= x ? 1 : 0;
+          }
+        }
         if (blk < NB) {
-          const TC* b = row + 32 * blk;
-          TC q[8];
-#pragma unroll
-          for (int k = 0; k < 8; ++k) q[k] = __ldg(b + 4 * k + 3);
-          G = 8 * blk;
-#pragma unroll
-          for (int k = 0; k < 8; ++k) G += q[k] <= x ? 1 : 0;
+          Quad<TC> qq;
+          qq.load(row + 4 * G);  // the crossing quad: its last entry is > x, its first three decide
+          nxt = 4 * G + (qq.v[0] <= x) + (qq.v[1] <= x) + (qq.v[2] <= x);
+          if (coarse && tb.rew_cls_pad && nxt < S) {
+            const int pos = nxt - 32 * blk;
+            const unsigned w = pos < 16 ? (pos < 8 ? (pos < 4 ? c0.x : c0.y) : (pos < 12 ? c0.z : c0.w))
+                                        : (pos < 24 ? (pos < 20 ? c1.x : c1.y) : (pos < 28 ? c1.z : c1.w));
+            cls = (int)((w >> (8 * (pos & 3))) & 0xffu);
+            have_cls = true;
+          }
         }
-      }
-      if (blk < NB) {
-        Quad<TC> qq;
-        qq.load(row + 4 * G);  // the crossing quad: its last entry is > x, its first three decide
-        nxt = 4 * G + (qq.v[0] <= x) + (qq.v[1] <= x) + (qq.v[2] <= x);
-        if (coarse && tb.rew_cls_pad && nxt < S) {
-          const int pos = nxt - 32 * blk;
-          const unsigned w = pos < 16 ? (pos < 8 ? (pos < 4 ? c0.x : c0.y) : (pos < 12 ? c0.z : c0.w))
-                                      : (pos < 24 ? (pos < 20 ? c1.x : c1.y) : (pos < 28 ? c1.z : c1.w));
-          cls = (int)((w >> (8 * (pos & 3))) & 0xffu);
-          have_cls = true;
+        if (nxt >= S) {  // x >= total (rounding): bisect's hi = n-1 clamp == first index where the row reaches total
+          nxt = 0;
+          while (nxt < S - 1 && __ldg(row + nxt) < total) ++nxt;
+          have_cls = false;
         }
-      }
-      if (nxt >= S) {  // x >= total (rounding): bisect's hi = n-1 clamp == first index where the row reaches total
-        nxt = 0;
-        while (nxt < S - 1 && __ldg(row + nxt) < total) ++nxt;
-        have_cls = false;
       }
       if (!have_cls) {
         if (tb.rew_cls_sas)
@@ -593,7 +655,7 @@ __global__ void __launch_bounds__(kStepThreads) env_step_dense_kary_kernel(const
           cls = tb.rew_cls_sa[(size_t)in.s * A + in.a];
       }
     }
-    finish_env(io, tb, valid ? e : 0, in, nxt, cls, stepping, resetting);
+    finish_env(io, tb, valid ? e : 0, in, nxt, cls, stepping, resetting, 0, 0, have_rew, rew);
   }
   if (!SERVER) return;
   server_done(io, pass);
@@ -608,33 +670,85 @@ __global__ void __launch_bounds__(kStepThreads) env_step_dense_kary_kernel(const
 // 4 Mi envs: 505 warp instructions per env-step, issue slots 68 % busy, DRAM 11 % -- the kernel is ISSUE bound once
 // the batch fills the machine, so instructions are what the asymptotic env-steps/s is made of.
 constexpr int kLeanThreads = 128;
+
+// prologue and epilogue of the lean kernels: env scalars in, Philox words, the action check; stores and counters out
+struct LeanEnv {
+  int st, s, h, a;
+  bool resetting, stepping;
+  Philox4 w;
+};
+
+template <bool COMPACT>
+__device__ __forceinline__ LeanEnv lean_load(const colo_mdp_tables& tb, const StepIO& io, unsigned e) {
+  LeanEnv v;
+  const bool valid = e < (unsigned)io.N;
+  v.st = COLO_STEP_MID; v.s = 0; v.h = 0; v.a = 0;
+  if (valid) {
+    v.st = io.step_type[e];
+    v.s = io.state[e];
+    v.h = io.h[e];
+    if (COMPACT)
+      v.a = reinterpret_cast<const unsigned char*>(io.action)[e];
+    else
+      v.a = io.srv_go ? __ldcv(io.action + e) : io.action[e];
+  }
+  v.w = philox4x32_10(io.seed, io.env0 + (uint64_t)e, step_t0(io));
+  bool bad = false;
+  if ((unsigned)v.a >= (unsigned)tb.A) {
+    if (io.status) *io.status = COLO_BAD_ACTION;
+    v.a = 0;
+    bad = true;
+  }
+  v.resetting = valid && v.st == COLO_STEP_LAST;
+  v.stepping = valid && v.st != COLO_STEP_LAST && !bad;
+  return v;
+}
+
+// have_rew: `rew` is the step's reward (no draw from class `cls`)
+template <bool COMPACT>
+__device__ __forceinline__ void lean_store(const colo_mdp_tables& tb, const StepIO& io, unsigned e, const LeanEnv& v,
+                                           int nxt, int cls, bool have_rew, float rew) {
+  if (v.resetting) {  // auto_reset path == BaseMDP.reset(): the action is ignored, reward is None (NaN here)
+    nxt = sample_start(tb, u53(v.w.w[0], v.w.w[1]));
+    io.state[e] = nxt;
+    io.h[e] = 0;
+    io.step_type[e] = COLO_STEP_FIRST;
+    if (io.step_type_mirror) io.step_type_mirror[e] = COLO_STEP_FIRST;
+    io.reward[e] = __int_as_float(0x7fc00000);
+    if (io.discount) io.discount[e] = __int_as_float(0x7fc00000);
+    if (COMPACT)
+      reinterpret_cast<short*>(io.obs)[e] = (short)nxt;
+    else
+      io.obs[e] = nxt;
+  } else if (v.stepping) {
+    const int hh = v.h + 1;
+    const bool last = tb.H > 0 && hh >= tb.H;
+    const unsigned char nst = last ? COLO_STEP_LAST : COLO_STEP_MID;
+    io.h[e] = hh;
+    io.state[e] = nxt;
+    io.reward[e] = have_rew ? rew : reward_draw(tb, cls, u24(v.w.w[2]));
+    io.step_type[e] = nst;
+    if (io.step_type_mirror) io.step_type_mirror[e] = nst;
+    if (io.discount) io.discount[e] = last ? 0.f : 1.f;
+    if (COMPACT)
+      reinterpret_cast<short*>(io.obs)[e] = last ? (short)-1 : (short)nxt;
+    else
+      io.obs[e] = last ? -1 : nxt;
+  }
+  const unsigned copy = blockIdx.x & (unsigned)io.visits_mask;
+  aggregated_inc(io.visits_s + (size_t)copy * io.n_s, nxt, v.stepping || v.resetting);
+  aggregated_inc(io.visits_sa + (size_t)copy * io.n_sa, (long long)nxt * tb.A + v.a, v.stepping);
+}
+
 template <int NCH, bool COMPACT>
 __global__ void __launch_bounds__(kLeanThreads) env_step_kary_lean_kernel(const colo_mdp_tables tb, const StepIO io) {
   constexpr int ld = 128 * NCH, NB = 4 * NCH;
   const unsigned e = blockIdx.x * kLeanThreads + threadIdx.x;
-  const bool valid = e < (unsigned)io.N;
   const int S = tb.S, A = tb.A;
-  int st = COLO_STEP_MID, s = 0, h = 0, a = 0;
-  if (valid) {
-    st = io.step_type[e];
-    s = io.state[e];
-    h = io.h[e];
-    if (COMPACT)
-      a = reinterpret_cast<const unsigned char*>(io.action)[e];
-    else
-      a = io.srv_go ? __ldcv(io.action + e) : io.action[e];
-  }
-  const Philox4 w = philox4x32_10(io.seed, io.env0 + (uint64_t)e, step_t0(io));
-  bool bad = false;
-  if ((unsigned)a >= (unsigned)A) {
-    if (io.status) *io.status = COLO_BAD_ACTION;
-    a = 0;
-    bad = true;
-  }
-  const bool resetting = valid && st == COLO_STEP_LAST;
-  const bool stepping = valid && st != COLO_STEP_LAST && !bad;
+  const LeanEnv v = lean_load<COMPACT>(tb, io, e);
+  const int s = v.s, a = v.a;
   int nxt = 0, cls = 0;
-  if (stepping) {
+  if (v.stepping) {
     const unsigned r = (unsigned)(s * A + a);
     const float* __restrict__ coarse = reinterpret_cast<const float*>(tb.cdf_coarse) + (size_t)r * NB;
     const float* __restrict__ row = reinterpret_cast<const float*>(tb.cdf) + (size_t)r * ld;
@@ -642,7 +756,7 @@ __global__ void __launch_bounds__(kLeanThreads) env_step_kary_lean_kernel(const 
 #pragma unroll
     for (int k = 0; k < NCH; ++k) cq[k] = __ldg(reinterpret_cast<const float4*>(coarse) + k);
     const float total = cq[NCH - 1].w;
-    const float x = u24(w.w[0]) * total;
+    const float x = u24(v.w.w[0]) * total;
     int blk = 0;
 #pragma unroll
     for (int k = 0; k < NCH; ++k) blk += (cq[k].x <= x) + (cq[k].y <= x) + (cq[k].z <= x) + (cq[k].w <= x);
@@ -671,36 +785,28 @@ __global__ void __launch_bounds__(kLeanThreads) env_step_kary_lean_kernel(const 
     }
     if (!have_cls) cls = tb.rew_cls_sas ? tb.rew_cls_sas[((size_t)s * A + a) * S + nxt] : (tb.rew_cls_sa ? tb.rew_cls_sa[(size_t)s * A + a] : 0);
   }
-  if (resetting) {  // auto_reset path == BaseMDP.reset(): the action is ignored, reward is None (NaN here)
-    nxt = sample_start(tb, u53(w.w[0], w.w[1]));
-    io.state[e] = nxt;
-    io.h[e] = 0;
-    io.step_type[e] = COLO_STEP_FIRST;
-    if (io.step_type_mirror) io.step_type_mirror[e] = COLO_STEP_FIRST;
-    io.reward[e] = __int_as_float(0x7fc00000);
-    if (io.discount) io.discount[e] = __int_as_float(0x7fc00000);
-    if (COMPACT)
-      reinterpret_cast<short*>(io.obs)[e] = (short)nxt;
-    else
-      io.obs[e] = nxt;
-  } else if (stepping) {
-    const int hh = h + 1;
-    const bool last = tb.H > 0 && hh >= tb.H;
-    const unsigned char nst = last ? COLO_STEP_LAST : COLO_STEP_MID;
-    io.h[e] = hh;
-    io.state[e] = nxt;
-    io.reward[e] = reward_draw(tb, cls, u24(w.w[2]));
-    io.step_type[e] = nst;
-    if (io.step_type_mirror) io.step_type_mirror[e] = nst;
-    if (io.discount) io.discount[e] = last ? 0.f : 1.f;
-    if (COMPACT)
-      reinterpret_cast<short*>(io.obs)[e] = last ? (short)-1 : (short)nxt;
-    else
-      io.obs[e] = last ? -1 : nxt;
+  lean_store<COMPACT>(tb, io, e, v, nxt, cls, false, 0.f);
+}
+
+// The lean call on the breakpoint table: env scalars -> one K-entry breakpoint row (one round of K independent 16-byte
+// loads) -> stores, plus a reward-quantile round only where the class is not constant.  Same Philox words, same x, same
+// result and reward bits as env_step_kary_lean_kernel.
+template <int K, bool COMPACT>
+__global__ void __launch_bounds__(kLeanThreads) env_step_breaks_lean_kernel(const colo_mdp_tables tb, const StepIO io) {
+  const unsigned e = blockIdx.x * kLeanThreads + threadIdx.x;
+  const LeanEnv v = lean_load<COMPACT>(tb, io, e);
+  int nxt = 0, cls = 0;
+  bool have_rew = false;
+  float rew = 0.f;
+  if (v.stepping) {
+    // x = u24 * total >= 0 (the builder refuses negative and NaN rows): the entry always carries the class
+    const BreakStep b = breaks_step<K>(tb.cdf_breaks, (unsigned)(v.s * tb.A + v.a), u24(v.w.w[0]));
+    nxt = b.nxt;
+    cls = b.cls;
+    have_rew = b.have_rew;
+    rew = b.rew;
   }
-  const unsigned copy = blockIdx.x & (unsigned)io.visits_mask;
-  aggregated_inc(io.visits_s + (size_t)copy * io.n_s, nxt, stepping || resetting);
-  aggregated_inc(io.visits_sa + (size_t)copy * io.n_sa, (long long)nxt * A + a, stepping);
+  lean_store<COMPACT>(tb, io, e, v, nxt, cls, have_rew, rew);
 }
 
 // one step of one env from successor-list tables (every lane of the warp calls it: finish_env uses warp collectives);
@@ -897,6 +1003,65 @@ __global__ void build_cdf_index_kernel(const TC* __restrict__ cdf, long long row
   }
 }
 
+// the breakpoints of one f32 cdf row c[0..S) (c[-1] := 0): calls at(k, p_k, v_k) for each, returns their number, or -1 when
+// the row decreases somewhere or holds a NaN (no step function to tabulate)
+template <typename F>
+__device__ __forceinline__ int row_breaks(const float* __restrict__ row, int S, F at) {
+  float prev = 0.f;
+  int m = 0;
+  for (int j = 0; j < S; ++j) {
+    const float c = row[j];
+    if (!(c >= prev)) return -1;
+    if (c > prev) at(m++, j, c);
+    prev = c;
+  }
+  return m;
+}
+
+__global__ void count_cdf_breaks_kernel(const float* __restrict__ cdf, long long rows, int S, int ld, int* __restrict__ out) {
+  const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= rows) return;
+  const int m = row_breaks(cdf + r * ld, S, [](int, int, float) {});
+  atomicMax(out, m < 0 ? S + 1 : m);
+}
+
+// one thread per (s, a) row: the row's breakpoints, padded with copies of the last, then every entry's reward class and,
+// for a class whose quantile row is bitwise constant and finite, its reward as reward_draw computes it (the same bits at
+// every uniform in [0, 1]: fmaf(f, +0, q0) == q0 + 0)
+__global__ void build_cdf_breaks_kernel(const colo_mdp_tables tb, int K, CdfBreak* __restrict__ out, int* __restrict__ err) {
+  const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= (long long)tb.S * tb.A) return;
+  CdfBreak* b = out + r * K;
+  int m = row_breaks(reinterpret_cast<const float*>(tb.cdf) + r * tb.ld, tb.S, [&](int k, int p, float v) {
+    if (k < K) {
+      b[k].v = v;
+      b[k].p = p;
+    }
+  });
+  if (m < 0 || m > K) {
+    atomicExch(err, 1);
+    m = m < 0 ? 0 : K;
+  }
+  if (m == 0) {  // an all-zero row: its search returns state 0
+    b[0].v = 0.f;
+    b[0].p = 0;
+    m = 1;
+  }
+  for (int k = m; k < K; ++k) {
+    b[k].v = b[m - 1].v;
+    b[k].p = b[m - 1].p;
+  }
+  for (int k = 0; k < K; ++k) {
+    const int p = b[k].p;
+    const int cls = tb.rew_cls_sas ? tb.rew_cls_sas[r * tb.S + p] : (tb.rew_cls_sa ? tb.rew_cls_sa[r] : 0);
+    const float* q = tb.rew_q + (size_t)cls * tb.nq;
+    bool constant = isfinite(q[0]);
+    for (int i = 1; i < tb.nq && constant; ++i) constant = __float_as_uint(q[i]) == __float_as_uint(q[0]);
+    b[k].cls_flags = (unsigned)cls | (constant ? kBreakInline : 0u);
+    b[k].r = constant ? reward_draw(tb, cls, 0.f) : 0.f;
+  }
+}
+
 // Non-tabular observations: EmissionMap.get_observation (colosseum/emission_maps/base.py:110-140) is a row gather from
 // the precomputed table all_observations[h, s, ...] (:56-76); past the horizon (in_episode_time >= H, i.e. the LAST
 // step of an episode) the reference returns zeros (:131-132).  One warp per env copies the D floats of its row.
@@ -973,10 +1138,30 @@ static int launch_dense(const colo_mdp_tables* tb, const StepIO& io, void* strea
     // thread-per-env k-ary search (default) or the warp-cooperative full-row count (COLO_STEP_KERNEL=coop)
     static const bool coop = getenv("COLO_STEP_KERNEL") && !strcmp(getenv("COLO_STEP_KERNEL"), "coop");
     static const bool no_lean = getenv("COLO_STEP_KERNEL") && !strcmp(getenv("COLO_STEP_KERNEL"), "general");
+    // the breakpoint table (f32 only) replaces the row search and the index in both thread-per-env kernels
+    const int kb = sizeof(TC) == 4 && tb->cdf_breaks ? tb->cdf_breaks_k : 0;
+    COLO_ARG_CHECK(kb == 0 || kb == 2 || kb == 4 || kb == 8 || kb == 16, "cdf_breaks_k must be 2, 4, 8 or 16");
+    COLO_ARG_CHECK(kb == 0 || (uintptr_t)tb->cdf_breaks % 16 == 0, "cdf_breaks must be 16-byte aligned");
     if (!coop && !no_lean && !SERVER && sizeof(TC) == 4 && io.n_steps == 1 && !io.random_actions && io.u_next == nullptr &&
-        io.u_rew == nullptr && io.auto_reset && tb->cdf_mid && tb->cdf_coarse && tb->rew_cls_pad && io.visits_s &&
+        io.u_rew == nullptr && io.auto_reset && (kb || (tb->cdf_mid && tb->cdf_coarse && tb->rew_cls_pad)) && io.visits_s &&
         io.visits_sa && io.N < (1LL << 31) - kLeanThreads) {
       const int gl = (int)((io.N + kLeanThreads - 1) / kLeanThreads);
+      if (kb) {
+#define COLO_BREAKS_LEAN(K)                                                                          \
+  case K:                                                                                            \
+    if (io.io_compact) env_step_breaks_lean_kernel<K, true><<<gl, kLeanThreads, 0, st>>>(*tb, io);   \
+    else env_step_breaks_lean_kernel<K, false><<<gl, kLeanThreads, 0, st>>>(*tb, io);                 \
+    break
+        switch (kb) {
+          COLO_BREAKS_LEAN(2);
+          COLO_BREAKS_LEAN(4);
+          COLO_BREAKS_LEAN(8);
+          COLO_BREAKS_LEAN(16);
+        }
+#undef COLO_BREAKS_LEAN
+        count_step_launch(COLO_STEP_KIND_BREAKS);
+        return check_launch("env_step_breaks_lean_kernel");
+      }
 #define COLO_LEAN(NCH)                                                              \
   case NCH:                                                                         \
     if (io.io_compact) env_step_kary_lean_kernel<NCH, true><<<gl, kLeanThreads, 0, st>>>(*tb, io);   \
@@ -1000,6 +1185,16 @@ static int launch_dense(const colo_mdp_tables* tb, const StepIO& io, void* strea
                                    "in-kernel uniforms, auto_reset, CDF index present, counters on, no server)");
     if (!coop) {
       const int gk = grid_for(kStepThreads, io.N);
+      if (kb) {
+        switch (kb) {
+          case 2: launch_step(env_step_dense_kary_kernel<float, 1, SERVER, 2>, gk, SERVER, share, tb, io, st); break;
+          case 4: launch_step(env_step_dense_kary_kernel<float, 1, SERVER, 4>, gk, SERVER, share, tb, io, st); break;
+          case 8: launch_step(env_step_dense_kary_kernel<float, 1, SERVER, 8>, gk, SERVER, share, tb, io, st); break;
+          case 16: launch_step(env_step_dense_kary_kernel<float, 1, SERVER, 16>, gk, SERVER, share, tb, io, st); break;
+        }
+        count_step_launch(COLO_STEP_KIND_BREAKS_GENERAL);
+        return check_launch("env_step_dense_kary_kernel");
+      }
 #define COLO_KARY(NCH)                                                                              \
   case NCH:                                                                                         \
     launch_step(env_step_dense_kary_kernel<TC, NCH, SERVER>, gk, SERVER, share, tb, io, st);        \
@@ -1743,6 +1938,57 @@ int colo_build_cdf_index(const void* cdf, int S, int A, int ld, int is_f64, void
     colo::build_cdf_index_kernel<float><<<grid, 256, 0, (cudaStream_t)stream>>>((const float*)cdf, rows, ld, (float*)cdf_mid,
                                                                              (float*)cdf_coarse);
   return colo::check_launch("build_cdf_index_kernel");
+}
+
+int colo_count_cdf_breaks(const float* cdf, int S, int A, int ld, int* max_breaks, void* stream) {
+  COLO_ARG_CHECK(cdf && max_breaks && S > 0 && A > 0 && ld >= S, "cdf, max_breaks, S, A, ld");
+  cudaStream_t st = (cudaStream_t)stream;
+  const long long rows = (long long)S * A;
+  int* d = nullptr;
+  COLO_CUDA_TRY(cudaMalloc((void**)&d, sizeof(int)));
+  cudaError_t e = cudaMemsetAsync(d, 0, sizeof(int), st);
+  if (e == cudaSuccess) {
+    colo::count_cdf_breaks_kernel<<<(unsigned)((rows + 127) / 128), 128, 0, st>>>(cdf, rows, S, ld, d);
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) e = cudaMemcpyAsync(max_breaks, d, sizeof(int), cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  cudaFree(d);
+  if (e != cudaSuccess) {
+    colo::set_error("colo_count_cdf_breaks: %s", cudaGetErrorString(e));
+    return COLO_ERR_CUDA;
+  }
+  return COLO_OK;
+}
+
+int colo_build_cdf_breaks(const colo_mdp_tables* tb, int k, void* cdf_breaks, void* stream) {
+  int r = colo::check_tables_common(tb);
+  if (r != COLO_OK) return r;
+  COLO_ARG_CHECK(tb->cdf && tb->ld >= tb->S && cdf_breaks && (uintptr_t)cdf_breaks % 16 == 0,
+                 "f32 cdf and a 16-byte aligned cdf_breaks");
+  COLO_ARG_CHECK(k == 2 || k == 4 || k == 8 || k == 16, "k must be 2, 4, 8 or 16");
+  cudaStream_t st = (cudaStream_t)stream;
+  const long long rows = (long long)tb->S * tb->A;
+  int* d = nullptr;
+  int err = 0;
+  COLO_CUDA_TRY(cudaMalloc((void**)&d, sizeof(int)));
+  cudaError_t e = cudaMemsetAsync(d, 0, sizeof(int), st);
+  if (e == cudaSuccess) {
+    colo::build_cdf_breaks_kernel<<<(unsigned)((rows + 127) / 128), 128, 0, st>>>(*tb, k, (colo::CdfBreak*)cdf_breaks, d);
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) e = cudaMemcpyAsync(&err, d, sizeof(int), cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  cudaFree(d);
+  if (e != cudaSuccess) {
+    colo::set_error("colo_build_cdf_breaks: %s", cudaGetErrorString(e));
+    return COLO_ERR_CUDA;
+  }
+  if (err) {
+    colo::set_error("colo_build_cdf_breaks: a row has more than %d breakpoints, decreases or holds a NaN", k);
+    return COLO_ERR_ARG;
+  }
+  return COLO_OK;
 }
 
 int colo_build_dense_cdf(const float* T, int S, int A, int ld, void* cdf, int out_is_f64, void* stream) {

@@ -67,7 +67,9 @@ unsigned long long colo_backup_tma_sweeps(void);
 #define COLO_STEP_KIND_SUCC 4  /* env_step_succ_kernel: successor-list tables                                  */
 #define COLO_STEP_KIND_MIXED_SUCC 5  /* env_step_succ_mixed_kernel: a mixed batch, successor-list tables       */
 #define COLO_STEP_KIND_MIXED_DENSE 6 /* env_step_dense_mixed_kernel: a mixed batch, dense rows (f32 or f64)   */
-#define COLO_STEP_KINDS 7
+#define COLO_STEP_KIND_BREAKS 7 /* env_step_breaks_lean_kernel: the common dense f32 call, breakpoint table set     */
+#define COLO_STEP_KIND_BREAKS_GENERAL 8 /* env_step_dense_kary_kernel searching the breakpoint table (other f32 calls) */
+#define COLO_STEP_KINDS 9
 unsigned long long colo_step_kernel_launches(int kind);
 
 /* ---------------------------------------------------------------- (B) Bellman backups ------------------- */
@@ -474,6 +476,15 @@ typedef struct {
   const void* cdf_mid;
   const void* cdf_coarse;
   const unsigned char* rew_cls_pad;
+  /* optional breakpoint table of an f32 cdf with short rows (ld % 128 == 0, ld <= 1024), built by colo_build_cdf_breaks:
+   * [S,A,cdf_breaks_k] 16-byte entries {float v; int p; unsigned cls_flags; float r}, cdf_breaks_k in {2, 4, 8, 16}.
+   * The breakpoints of row c[0..S) (c[-1] := 0) are the p with c[p] > c[p-1], in order, v = c[p]; entries past the
+   * row's last breakpoint repeat it (a row without one holds {0, 0}).  cls_flags: bits 0-30 the reward class of
+   * (s, a, p) (rew_cls_sas, else rew_cls_sa, else 0); bit 31 set when that class's quantile row is bitwise constant
+   * and finite, r then being its reward.  Searching it returns exactly what searching the row returns; the dense f32
+   * steps use it in place of the row and the index.  NULL: not used. */
+  const void* cdf_breaks;
+  int cdf_breaks_k;
 } colo_mdp_tables;
 
 /*
@@ -514,7 +525,8 @@ typedef struct {
   int io_compact;  /* != 0: compact host I/O -- `action` is read as u8[N] and `obs` written as i16[N] (-1 = the terminal
                       observation), 8 instead of 13 bytes per env-step over PCIe (reward f32, step_type u8 unchanged).
                       Needs S <= 32767, A <= 256 and the common call of the dense f32 step (supplied actions, in-kernel
-                      uniforms, auto_reset, CDF index present, counters on); COLO_ERR_ARG otherwise. */
+                      uniforms, auto_reset, CDF index or breakpoint table present, counters on); COLO_ERR_ARG
+                      otherwise. */
 } colo_env_batch;
 
 /*
@@ -899,6 +911,13 @@ int colo_build_dense_cdf(const float* T, int S, int A, int ld, void* cdf, int ou
  * plain copies of entries of the row, so searching through the index returns exactly what searching the row returns. */
 int colo_build_cdf_index(const void* cdf, int S, int A, int ld, int is_f64, void* cdf_mid, void* cdf_coarse,
                          void* stream);
+/* The largest number of breakpoints (entries c[j] > c[j-1], c[-1] := 0) over the rows of an f32 cdf [S,A,ld], into
+ * *max_breaks (host).  A row that decreases somewhere or holds a NaN counts as S + 1.  Synchronises `stream`. */
+int colo_count_cdf_breaks(const float* cdf, int S, int A, int ld, int* max_breaks, void* stream);
+/* The breakpoint table of colo_mdp_tables (cdf_breaks [S,A,k], see there) from tb->cdf (f32) and tb's reward classes
+ * and quantiles; k in {2, 4, 8, 16} must be at least colo_count_cdf_breaks of the cdf (rows with more are refused
+ * with COLO_ERR_ARG after the build, the table then being unusable).  Synchronises `stream`. */
+int colo_build_cdf_breaks(const colo_mdp_tables* tb, int k, void* cdf_breaks, void* stream);
 
 /* ---------------------------------------------------------------- multi-GPU ---------------------------- */
 /*
