@@ -16,6 +16,9 @@ STEP_FIRST, STEP_MID, STEP_LAST = 0, 1, 2
 STEP_KIND_LEAN, STEP_KIND_KARY, STEP_KIND_SHORT, STEP_KIND_LONG, STEP_KIND_SUCC = 0, 1, 2, 3, 4
 STEP_KIND_MIXED_SUCC, STEP_KIND_MIXED_DENSE = 5, 6
 STEP_KIND_BREAKS, STEP_KIND_BREAKS_GENERAL = 7, 8
+# Bellman-solver paths of colo_solver_path_launches (include/colosseum_b200.h, COLO_PATH_*)
+PATH_KINDS = ["SPARSE_VI", "SPARSE_SWEEP", "RESIDENT", "BACKUP_WARP", "BACKUP_CTA", "EPI_BATCHED", "SPARSE_HIT",
+              "SPARSE_EPI", "HIT_GEMM", "HIT_UMMA", "GS_TMA", "GS_LDG", "GS_SPARSE"]
 
 
 class ColosseumB200Error(RuntimeError):
@@ -197,6 +200,7 @@ PROTOTYPES = {
     "colo_reset_launch_count": (None, []),
     "colo_backup_tma_sweeps": (_ULL, []),
     "colo_step_kernel_launches": (_ULL, [_I]),
+    "colo_solver_path_launches": (_ULL, [_I]),
     "colo_stream_synchronize": (_I, [_P]),
     "colo_backup_f32": (_I, [C.POINTER(BackupArgs), _P]),
     "colo_backup_f64acc": (_I, [C.POINTER(BackupArgs), _P]),

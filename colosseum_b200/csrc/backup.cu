@@ -392,10 +392,12 @@ static int launch_backup_2(const colo_backup_args& p, bool group_cta, cudaStream
   const int cap = sm_count() * 32;
   if (group_cta) {
     int grid = (int)(items < cap ? items : cap);
+    count_solver_path(COLO_PATH_BACKUP_CTA);
     backup_kernel<TV, FOLD, VEC, true><<<grid, kThreads, 0, st>>>(p);
   } else {
     long long blocks = (items + kWarps - 1) / kWarps;
     int grid = (int)(blocks < cap ? blocks : cap);
+    count_solver_path(COLO_PATH_BACKUP_WARP);
     backup_kernel<TV, FOLD, VEC, false><<<grid, kThreads, 0, st>>>(p);
   }
   return check_launch("backup_kernel");
@@ -883,6 +885,7 @@ static int episodic_batched_launch(const float* T, const float* R, const float* 
   const int grid = (int)(B < cap ? B : cap);
   (void)shared_mdp;
   const long long ts = shared_mdp ? 0 : (long long)S * A * S, rs = shared_mdp ? 0 : (long long)S * A;
+  count_solver_path(COLO_PATH_EPI_BATCHED);
   if (vec4) {
     auto k = episodic_batched_kernel<TV, L, true>;
     { const int _es = ensure_dynamic_smem((const void*)k, smem); if (_es != COLO_OK) return _es; }

@@ -12,6 +12,7 @@ namespace colo {
 void set_error(const char* fmt, ...);
 void count_launch(unsigned long long n = 1);
 int check_launch(const char* what);  // cudaGetLastError -> COLO_OK / COLO_ERR_CUDA (+ counts one launch)
+void count_solver_path(int kind);    // one launch of a Bellman-solver path (COLO_PATH_*, colo_solver_path_launches)
 
 #define COLO_CUDA_TRY(expr)                                                                  \
   do {                                                                                       \

@@ -475,6 +475,7 @@ static int gs_launch(GsArgs a, void* stream) {
   const int grid = (a.B + W - 1) / W;
   cudaStream_t st = (cudaStream_t)stream;
   if (a.cv_rm != nullptr) {
+    count_solver_path(COLO_PATH_GS_SPARSE);
     if (a.A * a.KMp <= 32) {
       auto k = gs_sparse_kernel<TV, true>;
       { const int _es = ensure_dynamic_smem((const void*)k, smem); if (_es != COLO_OK) return _es; }
@@ -517,11 +518,13 @@ static int gs_launch(GsArgs a, void* stream) {
     const int grid_t = (int)(want < (long long)sm_count() ? want : (long long)sm_count());  // one CTA per SM, persistent
     auto k = gs_solve_tma_kernel<TV>;
     { const int _es = ensure_dynamic_smem((const void*)k, smem_t); if (_es != COLO_OK) return _es; }
+    count_solver_path(COLO_PATH_GS_TMA);
     k<<<grid_t, Wt * 32, smem_t, st>>>(a, counter);
     const int r = check_launch("gs_solve_tma_kernel");
     cudaFreeAsync(counter, st);
     return r;
   }
+  count_solver_path(COLO_PATH_GS_LDG);
   if (vec) {
     auto k = gs_solve_kernel<TV, true>;
     { const int _es = ensure_dynamic_smem((const void*)k, smem); if (_es != COLO_OK) return _es; }

@@ -612,6 +612,7 @@ int hitting_umma_sweep(UmmaPlan* pl, const float* E_in, float* E_out, long long 
     return COLO_OK;
   };
   int r;
+  count_solver_path(COLO_PATH_HIT_UMMA);
   if (pl->BN == 128) r = pl->mc ? launch(hitting_umma_kernel<128, true>, UmmaCfg<128>::SMEM) : launch(hitting_umma_kernel<128, false>, UmmaCfg<128>::SMEM);
   else r = pl->mc ? launch(hitting_umma_kernel<64, true>, UmmaCfg<64>::SMEM) : launch(hitting_umma_kernel<64, false>, UmmaCfg<64>::SMEM);
   if (r != COLO_OK) return r;

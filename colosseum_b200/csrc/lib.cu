@@ -11,6 +11,8 @@ namespace colo {
 
 static thread_local char g_err[512] = "";
 static std::atomic<unsigned long long> g_launches{0};
+// launches per Bellman-solver path (colo_solver_path_launches), counted on the host where the path is chosen
+static std::atomic<unsigned long long> g_path_launches[COLO_PATH_KINDS];
 
 void set_error(const char* fmt, ...) {
   va_list ap;
@@ -20,6 +22,7 @@ void set_error(const char* fmt, ...) {
 }
 
 void count_launch(unsigned long long n) { g_launches.fetch_add(n, std::memory_order_relaxed); }
+void count_solver_path(int kind) { g_path_launches[kind].fetch_add(1, std::memory_order_relaxed); }
 
 int check_launch(const char* what) {
   count_launch(1);
@@ -70,6 +73,9 @@ const char* colo_last_error(void) { return colo::g_err; }
 int colo_version(void) { return 100; }
 unsigned long long colo_launch_count(void) { return colo::g_launches.load(); }
 void colo_reset_launch_count(void) { colo::g_launches.store(0); }
+unsigned long long colo_solver_path_launches(int kind) {
+  return kind >= 0 && kind < COLO_PATH_KINDS ? colo::g_path_launches[kind].load(std::memory_order_relaxed) : 0ULL;
+}
 int colo_stream_synchronize(void* stream) {
   COLO_CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));
   return COLO_OK;

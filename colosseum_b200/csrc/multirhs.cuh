@@ -242,6 +242,7 @@ static int launch_hitting_gemm(const HittingGemmArgs& a, cudaStream_t st) {
   constexpr int BN = 64, TM = 4, TN = 4;
   constexpr int BK = sizeof(TV) == 8 ? 16 : 32;
   const long long tiles64 = (long long)((a.K + BN - 1) / BN) * ((a.S + 63) / 64);
+  count_solver_path(COLO_PATH_HIT_GEMM);
   if (tiles64 >= (long long)sm_count()) {  // measured: at 225 tiles (S = 948) the 64 x 64 tile is 15 % faster, at 49 (S = 400) slower
     constexpr int BM = 64;
     dim3 grid((a.K + BN - 1) / BN, (a.S + BM - 1) / BM);

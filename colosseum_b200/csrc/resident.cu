@@ -289,6 +289,7 @@ static int launch_resident_3(const ResidentArgs& a, size_t smem, cudaStream_t st
     set_error("resident solver: a cluster of %d CTAs with %zu B of shared memory cannot be scheduled", a.C, smem);
     return COLO_ERR_ARG;
   }
+  count_solver_path(COLO_PATH_RESIDENT);
   COLO_CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, a));
   return check_launch("resident_solve_kernel");
 }

@@ -599,7 +599,8 @@ int sparse_diameter_continuous(const float* T, const int* targets, int K, int S,
   a.targets = targets; a.eps = (float)eps; a.max_value = max_value; a.max_iter = max_iter;
   a.tile_max = d_max; a.iters = d_it; a.status = d_st;
   const int threads = block_threads(S);
-#define COLO_SPHIT(N)                                                                                       \
+  count_solver_path(COLO_PATH_SPARSE_HIT);
+#define COLO_SPHIT(N)                                                                                     \
   {                                                                                                         \
     auto kern = sparse_hitting_kernel<TV, N>;                                                               \
     { const int _es = ensure_dynamic_smem((const void*)kern, smem); if (_es != COLO_OK) return _es; }      \
@@ -643,6 +644,7 @@ int sparse_diameter_episodic(const float* T_epi, const int* targets, int K, int 
   a.max_iter = max_iter; a.out = d_out; a.iters = d_it; a.status = d_st;
   auto kern = sparse_episodic_kernel<TV>;
   { const int _es = ensure_dynamic_smem((const void*)kern, smem); if (_es != COLO_OK) return _es; }
+  count_solver_path(COLO_PATH_SPARSE_EPI);
   kern<<<K, block_threads(S), smem, st>>>(a);
   r = check_launch("sparse_episodic_kernel");
   if (r == COLO_OK) r = collect<TV>(d_out, d_it, d_st, K, out_host, st);
@@ -710,7 +712,8 @@ int sparse_solve_resident(const SparseRows& h, const float* R, const float* pi, 
   a.normalize = normalize ? 1 : 0;
   a.iters = d_it; a.status = d_st;
   const int threads = block_threads(S);
-#define COLO_SPVI(FOLD)                                                                                     \
+  count_solver_path(COLO_PATH_SPARSE_VI);
+#define COLO_SPVI(FOLD)                                                                                   \
   {                                                                                                         \
     auto kern = sparse_vi_kernel<TV, FOLD>;                                                                 \
     { const int _es = ensure_dynamic_smem((const void*)kern, smem); if (_es != COLO_OK) return _es; }      \
@@ -752,6 +755,7 @@ int sparse_sweep_launch(const SparseRows& h, const float* R, const float* pi, in
   const int threads = lanes >= 148LL * 1024 ? 256 : 128;
   dim3 grid((unsigned)((lanes + threads - 1) / threads), B);
   cudaStream_t st = (cudaStream_t)stream;
+  count_solver_path(COLO_PATH_SPARSE_SWEEP);
   if (fold == COLO_FOLD_MAX) sparse_sweep_kernel<TV, COLO_FOLD_MAX><<<grid, threads, 0, st>>>(a);
   else if (fold == COLO_FOLD_PI) sparse_sweep_kernel<TV, COLO_FOLD_PI><<<grid, threads, 0, st>>>(a);
   else sparse_sweep_kernel<TV, COLO_FOLD_MIN><<<grid, threads, 0, st>>>(a);

@@ -71,6 +71,25 @@ unsigned long long colo_backup_tma_sweeps(void);
 #define COLO_STEP_KIND_BREAKS_GENERAL 8 /* env_step_dense_kary_kernel searching the breakpoint table (other f32 calls) */
 #define COLO_STEP_KINDS 9
 unsigned long long colo_step_kernel_launches(int kind);
+/* Bellman-solver launches since load that went to each solver path (`kind`: COLO_PATH_*; 0 for any other value): the
+ * solvers of (B) pick their kernel from the tensor's shape and sparsity, and this tells a caller which one served a
+ * call.  Counted on the host when the launch is enqueued, one count per launch (a solve of n sweeps on a per-sweep
+ * path counts n), as colo_step_kernel_launches. */
+#define COLO_PATH_SPARSE_VI 0    /* sparse_vi_kernel: compressed rows, a whole discounted solve in one CTA (S <= 2048) */
+#define COLO_PATH_SPARSE_SWEEP 1 /* sparse_sweep_kernel: compressed rows, one launch per discounted sweep              */
+#define COLO_PATH_RESIDENT 2     /* resident_solve_kernel: T in a cluster's shared memory, a whole solve in one launch */
+#define COLO_PATH_BACKUP_WARP 3  /* backup_kernel, one warp per (instance, state)                                     */
+#define COLO_PATH_BACKUP_CTA 4   /* backup_kernel, one CTA per (instance, state): few, long rows                      */
+#define COLO_PATH_EPI_BATCHED 5  /* episodic_batched_kernel: one CTA per instance, all layers in one launch           */
+#define COLO_PATH_SPARSE_HIT 6   /* sparse_hitting_kernel: compressed rows, a whole continuous diameter in one launch */
+#define COLO_PATH_SPARSE_EPI 7   /* sparse_episodic_kernel: compressed rows, a whole episodic diameter in one launch  */
+#define COLO_PATH_HIT_GEMM 8     /* hitting_gemm_kernel: one tiled multi-target GEMM per diameter sweep or layer      */
+#define COLO_PATH_HIT_UMMA 9     /* hitting_umma_kernel: the same sweep on the tensor cores (f32)                     */
+#define COLO_PATH_GS_TMA 10      /* gs_solve_tma_kernel: in-place sweeps, dense rows staged by the TMA               */
+#define COLO_PATH_GS_LDG 11      /* gs_solve_kernel: in-place sweeps, dense rows through plain loads                  */
+#define COLO_PATH_GS_SPARSE 12   /* gs_sparse_kernel: in-place sweeps on compressed rows                              */
+#define COLO_PATH_KINDS 13
+unsigned long long colo_solver_path_launches(int kind);
 
 /* ---------------------------------------------------------------- (B) Bellman backups ------------------- */
 /*

@@ -99,11 +99,15 @@ def test_umma_large_dense_2048():
 
 
 def test_diameter_dense_through_umma(monkeypatch):
-    """get_diameter (f32 mode) on a dense synthetic MDP takes the tensor-core path and meets the f32 bar against the
-    fp64 fixed-point oracle; forcing the SIMT GEMM gives the same number to rounding"""
+    """get_diameter (f32 mode) on a dense synthetic MDP takes the tensor-core path, one hitting_umma launch per sweep
+    and no other solver path, and meets the f32 bar against the fp64 fixed-point oracle.  (The forced SIMT GEMM is
+    compared with this path in test_gpu_solver_paths.py: COLO_DIAM_PATH is read once per process.)"""
     import colosseum_b200.hardness as hd
 
     from colosseum_b200 import _cabi
+
+    def paths():
+        return np.array([_cabi.lib().colo_solver_path_launches(k) for k in range(len(_cabi.PATH_KINDS))], np.int64)
 
     T = dirichlet_T(384, 8, 0.02, 11)  # 4.7 MB: too large for the on-chip resident solver, dense rows
     # fp64 fixed point of the multi-target recurrence (SURVEY App. B.5), all targets side by side
@@ -119,9 +123,12 @@ def test_diameter_dense_through_umma(monkeypatch):
     d_ref = float(E.max())
     assert abs(orc.diameter_continuous_f64(T, targets=np.arange(4, dtype=np.int32)) - E[:4].max()) < 1e-6  # same recurrence
     n0 = _cabi.lib().colo_launch_count()
+    p0 = paths()
     d, sweeps = hd.get_diameter(T, False, precision="f32", epsilon=2e-5, return_sweeps=True)
     assert abs(d - d_ref) < 1e-4 * d_ref, (d, d_ref)
     assert sweeps > 3 and _cabi.lib().colo_launch_count() - n0 >= sweeps
+    ran = {_cabi.PATH_KINDS[k]: int(v) for k, v in enumerate(paths() - p0) if v}
+    assert ran == {"HIT_UMMA": sweeps}, ran
 
 
 @pytest.mark.parametrize("cluster", ["0", "1"])
