@@ -118,6 +118,13 @@ class QLearningArgs(C.Structure):
     ]
 
 
+class QLearningInst(C.Structure):
+    """mirror of `colo_qlearning_inst`"""
+
+    _fields_ = [("log_term", C.c_double), ("sqrt_h7sa", C.c_double), ("H_eff", C.c_double), ("gamma", C.c_double),
+                ("span_approx", C.c_double)]
+
+
 class PsrlArgs(C.Structure):
     """mirror of `colo_psrl_args`"""
 
@@ -263,6 +270,10 @@ PROTOTYPES = {
     "colo_env_server_stop": (_I, [C.POINTER(EnvServer), _P]),
     "colo_qlearning_episodic_steps": (_I, [C.POINTER(MdpTables), C.POINTER(QLearningArgs), _I, _ULL, _P]),
     "colo_qlearning_continuous_steps": (_I, [C.POINTER(MdpTables), C.POINTER(QLearningArgs), _I, _ULL, _P]),
+    "colo_mixed_qlearning_create": (_I, [_P, _I, C.POINTER(QLearningInst), _P, C.POINTER(C.c_void_p)]),
+    "colo_mixed_qlearning_sizes": (_I, [_P, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]),
+    "colo_mixed_qlearning_steps": (_I, [_P, C.POINTER(QLearningArgs), _I, _ULL, _P]),
+    "colo_mixed_qlearning_destroy": (None, [_P]),
     "colo_psrl_episodic_steps": (_I, [C.POINTER(MdpTables), C.POINTER(PsrlArgs), _I, _ULL, _P]),
     "colo_ucrl2_steps": (_I, [C.POINTER(MdpTables), C.POINTER(Ucrl2Args), _LL, _P]),
     "colo_ucrl2_bounds": (_I, [C.POINTER(Ucrl2Args), _I, _I, _P, _I, _D, _D, _D, _I, _P, _P, _P]),

@@ -9,6 +9,8 @@ body execute per launch.  Classes keep the reference's names and constructor arg
     QLearningContinuous colosseum/agent/agents/infinite_horizon/q_learning.py:114-255 (Wei et al. 2020)
     BatchedMDPLoop.run(T, log_every)  MDPLoop.run: cumulative reward per loop, and at every log tick the expected
                         regret of each loop's greedy policy (experiment/indicators.py:29-45 / markov_chain.py:12-31)
+    MixedQLearningEpisodic, MixedQLearningContinuous, MixedBatchedMDPLoop
+                        the same loops on many MDP instances at once (a benchmark's instances x seeds), one launch
 
 `mdp_specs` is replaced by the `MDPTables` of the MDP (the kernel needs the sampler tables, not only the sizes).
 `epsilon_greedy` and `boltzmann_temperature` are constants or, as in the reference, functions of the actor's interaction
@@ -668,6 +670,18 @@ def agents_load_state_dict(agents, d):
     agents.torch.cuda.current_stream().synchronize()
 
 
+def _normalised_indicators(rec, cum_regret, base, done):
+    """the normalised indicators of MDPLoop._update_performance_logs (agent_mdp_interaction.py:395-428) from the
+    episodic baselines `base` (scalars, or one value per loop)"""
+    span = base["optimal"] - base["worst"]
+    rec["normalized_cumulative_regret"] = cum_regret / span
+    rec["normalized_cumulative_reward"] = (rec["cumulative_reward"] - done * base["worst"]) / span
+    for k in ("optimal", "worst", "random"):
+        rec[f"{k}_cumulative_expected_reward"] = base[k] * done
+    rec["random_cumulative_regret"] = (base["optimal"] - base["random"]) * done
+    rec["worst_cumulative_regret"] = span * done
+
+
 class BatchedMDPLoop:
     """MDPLoop for N loops at once.  `T`, `R` (numpy float32) are only needed for the regret indicators."""
 
@@ -869,17 +883,241 @@ class BatchedMDPLoop:
                 reg = self._expected_regret_all() if all_loops else self._expected_regret(regret_for)
                 cum_regret = cum_regret + reg * n  # agent_mdp_interaction.py:503-506
                 rec["regret"], rec["cumulative_regret"] = reg, cum_regret.copy()
-                if base is not None:  # the normalised indicators of MDPLoop._update_performance_logs (:395-428)
-                    span = base["optimal"] - base["worst"]
-                    rec["normalized_cumulative_regret"] = cum_regret / span
-                    rec["normalized_cumulative_reward"] = (rec["cumulative_reward"] - done * base["worst"]) / span
-                    for k in ("optimal", "worst", "random"):
-                        rec[f"{k}_cumulative_expected_reward"] = base[k] * done
-                    rec["random_cumulative_regret"] = (base["optimal"] - base["random"]) * done
-                    rec["worst_cumulative_regret"] = span * done
+                if base is not None:
+                    _normalised_indicators(rec, cum_regret, base, done)
                 if all_loops:
                     cum_expected = cum_expected + self._agent_average_reward * n
                     rec["cumulative_expected_reward"] = cum_expected.copy()
+            rec["steps_per_second"] = done * ag.n_loops / (time.perf_counter() - t_start)
+            self.logs.append(rec)
+        return self.logs
+
+
+class _MixedQLearningBatch:
+    """Q-learning loops on many MDP instances, all advanced by one launch per `steps` (colo_mixed_qlearning_*).
+    Instance i owns the contiguous loops `segment(i)`; they are bit-identical to the single-MDP class built with
+    tables[i], seed[i] and n_loops[i].  The flat tables keep the single-MDP names (N, Q, V, ...; state, h,
+    cumulative_reward, n_episodes are flat [n_loops]); `table(name, i)` is instance i's view, shaped as the single-MDP
+    class's table ([n_i, H_i, S_i, A_i], V [n_i, H_i + 1, S_i]; continuous [n_i, S_i, A_i], V [n_i, S_i])."""
+    episodic = None
+
+    def _alloc(self, tables, n_loops, seed, epsilon_greedy, boltzmann_temperature):
+        import torch
+
+        from .batched_mdp import MixedBatchedMDP
+
+        _cabi.require_cuda()
+        self._explore = (epsilon_greedy, boltzmann_temperature)
+        tables = list(tables)
+        for i, tb in enumerate(tables):
+            assert (tb.H > 0) == self.episodic, f"instance {i}: episodic agents need an episodic MDP and vice versa"
+        self.torch = torch
+        self._handle = None
+        # the env handle (successor tables, per-instance seeds and segments) and the resets
+        self.env = MixedBatchedMDP(tables, n_loops, "succ", seed, track_visits=False)
+        self.tables = self.env.tables
+        self.sizes, self.seeds = self.env.sizes, self.env.seeds
+        self.n_loops = N = self.env.n_envs
+        self.t = 0
+        self.state, self.h = self.env.state, self.env.h
+        self.cumulative_reward = torch.zeros(N, dtype=torch.float64, device="cuda")
+        self.n_episodes = torch.zeros(N, dtype=torch.int64, device="cuda")
+        a = _cabi.QLearningArgs()
+        a.N = N  # seed, env0 and the per-instance constants live in the handle
+        a.state, a.h = self.state.data_ptr(), self.h.data_ptr()
+        a.cum_reward, a.n_episodes = self.cumulative_reward.data_ptr(), self.n_episodes.data_ptr()
+        self._args = a
+        self.reset_envs()
+
+    def _make_handle(self, insts):
+        """uploads the per-instance constants; returns the element counts of the Q-shaped and V-shaped flat tables"""
+        n = len(self.tables)
+        lib = _cabi.lib()
+        out = C.c_void_p()
+        rc = lib.colo_mixed_qlearning_create(self.env._handle, int(self.episodic), (_cabi.QLearningInst * n)(*insts),
+                                             _cabi.current_stream(), C.byref(out))
+        _cabi.check(rc, "colo_mixed_qlearning_create")
+        self._handle = out.value
+        nq, nv = C.c_longlong(), C.c_longlong()
+        _cabi.check(lib.colo_mixed_qlearning_sizes(self._handle, C.byref(nq), C.byref(nv)), "colo_mixed_qlearning_sizes")
+        ep = self.episodic
+        self._shapes = {"q": [(int(m), tb.H, tb.S, tb.A) if ep else (int(m), tb.S, tb.A) for m, tb in zip(self.sizes, self.tables)],
+                        "v": [(int(m), tb.H + 1, tb.S) if ep else (int(m), tb.S) for m, tb in zip(self.sizes, self.tables)]}
+        self._region = {k: [int(np.prod(sh)) for sh in v] for k, v in self._shapes.items()}
+        self._off = {k: np.concatenate([[0], np.cumsum(v)]).astype(np.int64) for k, v in self._region.items()}
+        assert (self._off["q"][-1], self._off["v"][-1]) == (nq.value, nv.value), "table layout of the library"
+        return nq.value, nv.value
+
+    def _per_instance(self, kind, dtype, values):
+        """a flat table whose region of instance i is filled with values[i]"""
+        torch = self.torch
+        counts = torch.tensor(self._region[kind], dtype=torch.int64, device="cuda")
+        return torch.repeat_interleave(torch.tensor(values, dtype=dtype, device="cuda"), counts,
+                                       output_size=int(self._off[kind][-1]))
+
+    def __del__(self):
+        try:
+            if getattr(self, "_handle", None):
+                _cabi.lib().colo_mixed_qlearning_destroy(self._handle)
+                self._handle = None
+        except Exception:
+            pass
+
+    @property
+    def n_instances(self):
+        return len(self.tables)
+
+    def segment(self, i: int) -> slice:
+        """the loops of instance i"""
+        return self.env.segment(i)
+
+    def table(self, name: str, i: int):
+        """instance i's view of the flat table `name`, shaped as the single-MDP class's"""
+        kind = "v" if name == "V" else "q"
+        lo, hi = int(self._off[kind][i]), int(self._off[kind][i + 1])
+        return getattr(self, name)[lo:hi].view(self._shapes[kind][i])
+
+    def reset_envs(self):
+        """mdp.reset() for every loop, as the single-MDP classes: start states drawn at counter t, then t += 1"""
+        self.env.t = self.t
+        self.env.reset()
+        self.t += 1
+        self.torch.cuda.current_stream().synchronize()
+
+    def steps(self, n_steps: int, trace: bool = False):
+        """n_steps iterations of the interaction loop for every loop of every instance, one launch.  trace=True returns
+        i32 [n_steps, n_loops, 4] = (s_t, a_t, obs_tp1, reward bits)."""
+        torch = self.torch
+        tr = torch.empty((n_steps, self.n_loops, 4), dtype=torch.int32, device="cuda") if trace else None
+        self._args.trace = None if tr is None else tr.data_ptr()
+        _set_actor(self, self.t, n_steps)
+        rc = _cabi.lib().colo_mixed_qlearning_steps(self._handle, C.byref(self._args), int(n_steps), self.t,
+                                                    _cabi.current_stream())
+        _cabi.check(rc, "colo_mixed_qlearning_steps")
+        self.t += int(n_steps)
+        return tr
+
+
+class MixedQLearningEpisodic(_MixedQLearningBatch):
+    """QLearningEpisodic's loops on many episodic MDPs: `tables` a list, `seed` and `n_loops` one value or one per
+    instance"""
+    episodic = True
+
+    def __init__(self, seed, tables, optimization_horizon: int, p: float, c_1: float, c_2: float = None,
+                 min_at: float = 0, UCB_type="hoeffding", epsilon_greedy=None, boltzmann_temperature=None, *,
+                 n_loops=1):
+        UCB_type = UCB_type.lower()
+        assert 0 <= min_at < 0.99 and 0 < p < 1 and c_1 > 0 and UCB_type in ("hoeffding", "bernstein")
+        if UCB_type == "bernstein":
+            assert c_2 is not None and c_2 > 0
+        self._alloc(tables, n_loops, seed, epsilon_greedy, boltzmann_temperature)
+        torch = self.torch
+        insts = [_cabi.QLearningInst(log_term=float(np.log(tb.S * tb.A * optimization_horizon / p)),  # q_learning.py:43
+                                     sqrt_h7sa=float(np.sqrt(tb.H ** 7 * tb.S * tb.A))) for tb in self.tables]
+        nq, nv = self._make_handle(insts)
+        self.N = torch.ones(nq, dtype=torch.int32, device="cuda")                              # q_learning.py:44
+        self.Q = self._per_instance("q", torch.float32, [float(tb.H) for tb in self.tables])   # :45-47
+        self.V = torch.zeros(nv, dtype=torch.float32, device="cuda")                          # :48
+        a = self._args
+        a.cnt, a.Q, a.V = self.N.data_ptr(), self.Q.data_ptr(), self.V.data_ptr()
+        a.ucb_type = 0
+        if UCB_type == "bernstein":
+            self.mu = torch.zeros(nq, dtype=torch.float32, device="cuda")
+            self.sigma = torch.zeros_like(self.mu)
+            self.beta = torch.zeros_like(self.mu)
+            a.mu, a.sigma, a.beta = self.mu.data_ptr(), self.sigma.data_ptr(), self.beta.data_ptr()
+            a.ucb_type = 1
+            a.c_2 = float(c_2)
+        a.c_1, a.min_at = float(c_1), float(min_at)
+
+
+class MixedQLearningContinuous(_MixedQLearningBatch):
+    """QLearningContinuous's loops on many continuous MDPs: `tables` a list, `seed` and `n_loops` one value or one per
+    instance; H, gamma and span_approx are lists, one value per instance"""
+    episodic = False
+
+    def __init__(self, seed, tables, optimization_horizon: int, min_at: float = 0, confidence: float = 0.95,
+                 span_approx_weight: float = 1, get_span_approx=None, h_weight: float = 1, get_H=get_H,
+                 epsilon_greedy=None, boltzmann_temperature=None, *, n_loops=1):
+        assert 0 <= min_at < 0.99 and 0 < confidence < 1 and span_approx_weight > 0 and h_weight > 0
+        self._alloc(tables, n_loops, seed, epsilon_greedy, boltzmann_temperature)
+        torch = self.torch
+        self.min_at = min_at if min_at > 0.009 else 0                                # q_learning.py:62
+        log_term = float(np.log(2 * optimization_horizon / confidence))
+        self.span_approx, self.H, self.gamma, insts = [], [], [], []
+        for tb in self.tables:
+            span = span_approx_weight
+            if get_span_approx is not None:
+                span *= get_span_approx(tb.S, tb.A)
+            H = float(h_weight * get_H(tb.S, tb.A, optimization_horizon, span, confidence))
+            self.span_approx.append(span)
+            self.H.append(H)
+            self.gamma.append(1 - 1 / H)
+            insts.append(_cabi.QLearningInst(log_term=log_term, H_eff=H, gamma=float(1 - 1 / H), span_approx=float(span)))
+        nq, nv = self._make_handle(insts)
+        self.N = torch.zeros(nq, dtype=torch.int32, device="cuda")
+        self.Q = self._per_instance("q", torch.float32, self.H)
+        self.Q_main = self.Q.clone()
+        self.V = self._per_instance("v", torch.float32, self.H)
+        a = self._args
+        a.cnt, a.Q, a.Q_main, a.V = self.N.data_ptr(), self.Q.data_ptr(), self.Q_main.data_ptr(), self.V.data_ptr()
+        a.min_at = float(self.min_at)
+
+
+class _SegmentView:
+    """instance i of a mixed agent batch, with the attributes BatchedMDPLoop's regret evaluation reads"""
+
+    def __init__(self, agents, i):
+        self.torch, self.episodic = agents.torch, agents.episodic
+        self.tables = agents.tables[i]
+        self.n_loops = int(agents.sizes[i])
+        self.Q = agents.table("Q", i)
+        self.state = agents.state[agents.segment(i)]
+
+
+class MixedBatchedMDPLoop:
+    """BatchedMDPLoop for a mixed agent batch.  `T`, `R` (lists, one numpy float32 pair per instance) are only needed
+    for the regret indicators.  The record has BatchedMDPLoop.run's fields, each as a flat per-loop array.
+    regret_for="all" evaluates the greedy policies instance by instance, through one BatchedMDPLoop per instance over a
+    view of its segment: a log tick costs a few launches and a host synchronisation per instance (one ragged launch
+    over every instance is not offered)."""
+
+    def __init__(self, agents: _MixedQLearningBatch, T=None, R=None):
+        self.agents = agents
+        self.T, self.R = T, R
+        self.loops = None if T is None else [BatchedMDPLoop(_SegmentView(agents, i), T[i], R[i])
+                                             for i in range(agents.n_instances)]
+        self.logs = []
+
+    def run(self, T: int, log_every: int = -1, regret_for=None):
+        """T interaction steps for every loop, `log_every` steps per launch; regret_for None or "all"."""
+        assert regret_for in (None, "all"), "a mixed batch evaluates the regret of every loop or of none"
+        ag = self.agents
+        log_every = T if log_every in (0, -1, None) else int(log_every)
+        regret = regret_for == "all"
+        assert not regret or self.loops is not None, "regret_for='all' needs T, R"
+        cum_regret = np.zeros(ag.n_loops)
+        cum_expected = np.zeros(ag.n_loops)
+        base = None
+        if regret and ag.episodic:
+            per = [lp.episodic_baselines() for lp in self.loops]
+            base = {k: np.repeat([b[k] for b in per], ag.sizes) for k in ("optimal", "worst", "random")}
+        t_start = time.perf_counter()
+        done = 0
+        while done < T:
+            n = min(log_every, T - done)
+            ag.steps(n)
+            done += n
+            rec = {"steps": done, "cumulative_reward": ag.cumulative_reward.cpu().numpy(),
+                   "n_episodes": ag.n_episodes.cpu().numpy()}
+            if regret:
+                reg = np.concatenate([lp._expected_regret_all() for lp in self.loops])
+                cum_regret = cum_regret + reg * n
+                rec["regret"], rec["cumulative_regret"] = reg, cum_regret.copy()
+                if base is not None:
+                    _normalised_indicators(rec, cum_regret, base, done)
+                cum_expected = cum_expected + np.concatenate([lp._agent_average_reward for lp in self.loops]) * n
+                rec["cumulative_expected_reward"] = cum_expected.copy()
             rec["steps_per_second"] = done * ag.n_loops / (time.perf_counter() - t_start)
             self.logs.append(rec)
         return self.logs

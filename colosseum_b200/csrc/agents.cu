@@ -16,36 +16,44 @@
 //
 // Memory: the tables of a loop are contiguous ([N][H,S,A]); accesses are 4-byte gathers at (h, s, a) -- latency
 // bound, hidden by running one thread per loop with as many loops as the caller has seeds.
+#include <cmath>
+#include <vector>
+
 #include "agent_device.cuh"
+#include "mixed.cuh"
 
 namespace colo {
 
+// Loop i of a batch: it is loop j of the region of the flat tables that starts base_q (Q-shaped tables) / base_v (V)
+// elements in; it draws with Philox key `seed` (agent: seed ^ kAgentKey) and counter (ctr, t), and its MDP's constants
+// are `c`.  The flat per-loop arrays of p (state, h, cum_reward, n_episodes, trace) are indexed by i.
 template <bool EPISODIC>
-__global__ void __launch_bounds__(128) qlearning_steps_kernel(const colo_mdp_tables tb, const colo_qlearning_args p,
-                                                              int n_steps, unsigned long long t0) {
-  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= p.N) return;
+__device__ __forceinline__ void qlearning_loop(const colo_mdp_tables& tb, const colo_qlearning_args& p,
+                                               const colo_qlearning_inst& c, size_t base_q, size_t base_v, long long j,
+                                               unsigned long long seed, unsigned long long ctr, long long i,
+                                               int n_steps, unsigned long long t0) {
   const int S = tb.S, A = tb.A, H = tb.H;
   const size_t per_q = (size_t)(EPISODIC ? H : 1) * S * A, per_v = (size_t)(EPISODIC ? H + 1 : 1) * S;
-  int* cnt = p.cnt + i * per_q;
-  float* Q = p.Q + i * per_q;
-  float* V = p.V + i * per_v;
-  float* Qm = EPISODIC ? nullptr : p.Q_main + i * per_q;
-  float* mu = p.mu ? p.mu + i * per_q : nullptr;
-  float* sg = p.sigma ? p.sigma + i * per_q : nullptr;
-  float* be = p.beta ? p.beta + i * per_q : nullptr;
+  const size_t off_q = base_q + j * per_q, off_v = base_v + j * per_v;
+  int* cnt = p.cnt + off_q;
+  float* Q = p.Q + off_q;
+  float* V = p.V + off_v;
+  float* Qm = EPISODIC ? nullptr : p.Q_main + off_q;
+  float* mu = p.mu ? p.mu + off_q : nullptr;
+  float* sg = p.sigma ? p.sigma + off_q : nullptr;
+  float* be = p.beta ? p.beta + off_q : nullptr;
   int s = p.state[i], h = p.h[i];
   double cum = p.cum_reward[i];
   long long episodes = p.n_episodes ? p.n_episodes[i] : 0;
-  const double Hd = EPISODIC ? (double)H : p.H_eff;
+  const double Hd = EPISODIC ? (double)H : c.H_eff;
   const double H3 = (double)H * H * H;  // exact: H**3 is a python int in the reference
 
   for (int step = 0; step < n_steps; ++step) {
     const unsigned long long t = t0 + step;
-    const Philox4 we = philox4x32_10(p.seed, p.env0 + (uint64_t)i, t);
-    const Philox4 wa = philox4x32_10(p.seed ^ kAgentKey, p.env0 + (uint64_t)i, t);
+    const Philox4 we = philox4x32_10(seed, ctr, t);
+    const Philox4 wa = philox4x32_10(seed ^ kAgentKey, ctr, t);
     const size_t row = ((size_t)(EPISODIC ? h : 0) * S + s) * A;
-    const int a = actor_select(Q + row, A, A, p.epsilon_greedy, p.actor, (long long)t, wa, p.seed, p.env0 + (uint64_t)i);
+    const int a = actor_select(Q + row, A, A, p.epsilon_greedy, p.actor, (long long)t, wa, seed, ctr);
     const size_t idx = row + a;
     // every table entry the update needs is requested as soon as its address is known, and consumed only after the
     // sampler's own (dependent) table walk: the loop body is a chain of cold gathers, the fewer in series the better
@@ -85,7 +93,7 @@ __global__ void __launch_bounds__(128) qlearning_steps_kernel(const colo_mdp_tab
       float b32 = 0.f;
       bool b_is_f32 = false;
       if (p.ucb_type == 0) {
-        b = __dmul_rn(p.c_1, __dsqrt_rn(__ddiv_rn(__dmul_rn(H3, p.log_term), (double)n)));
+        b = __dmul_rn(p.c_1, __dsqrt_rn(__ddiv_rn(__dmul_rn(H3, c.log_term), (double)n)));
       } else {
         const float m = __fadd_rn(mu0, vnext);
         const float g = __fadd_rn(sg0, __fmul_rn(vnext, vnext));
@@ -96,10 +104,10 @@ __global__ void __launch_bounds__(128) qlearning_steps_kernel(const colo_mdp_tab
         const float hd2 = __fmul_rn((float)H, __fmul_rn(d, d));
         const int n2 = (int)((unsigned)n * (unsigned)n);  // np.int32 ** 2 wraps
         const double x = __dadd_rn(__ddiv_rn((double)hd2, (double)n2), (double)H);
-        const double first = __dsqrt_rn(__dmul_rn(x, p.log_term));
-        const double second = __ddiv_rn(__dmul_rn(p.sqrt_h7sa, p.log_term), (double)n);
+        const double first = __dsqrt_rn(__dmul_rn(x, c.log_term));
+        const double second = __ddiv_rn(__dmul_rn(c.sqrt_h7sa, c.log_term), (double)n);
         const double v1 = __dmul_rn(p.c_1, __dadd_rn(first, second));
-        const double v2 = __dmul_rn(p.c_2, __dsqrt_rn(__ddiv_rn(__dmul_rn(H3, p.log_term), (double)n)));
+        const double v2 = __dmul_rn(p.c_2, __dsqrt_rn(__ddiv_rn(__dmul_rn(H3, c.log_term), (double)n)));
         const float nb = (float)(v2 < v1 ? v2 : v1);  // python min(v1, v2)
         be[idx] = nb;
         if (py_alpha) {  // every operand is float32 or a python scalar: the whole bonus is float32 arithmetic
@@ -123,9 +131,9 @@ __global__ void __launch_bounds__(128) qlearning_steps_kernel(const colo_mdp_tab
       for (int k = 1; k < A; ++k) mx = fmaxf(mx, Q[row + k]);
       V[(size_t)h * S + s] = fminf((float)H, mx);
     } else {
-      const double b = __dmul_rn(__dmul_rn(4.0, p.span_approx),
-                                 __dsqrt_rn(__dmul_rn(__ddiv_rn(Hd, (double)n), p.log_term)));
-      const double target = __dadd_rn(__dadd_rn((double)r, __dmul_rn(p.gamma, (double)v_sp)), b);
+      const double b = __dmul_rn(__dmul_rn(4.0, c.span_approx),
+                                 __dsqrt_rn(__dmul_rn(__ddiv_rn(Hd, (double)n), c.log_term)));
+      const double target = __dadd_rn(__dadd_rn((double)r, __dmul_rn(c.gamma, (double)v_sp)), b);
       const float qm = (float)__dadd_rn(__dmul_rn(om, (double)q_old), __dmul_rn(alpha, target));
       Qm[idx] = qm;
       const float q_new = fminf(q_old, qm);
@@ -159,6 +167,39 @@ __global__ void __launch_bounds__(128) qlearning_steps_kernel(const colo_mdp_tab
   p.h[i] = h;
   p.cum_reward[i] = cum;
   if (p.n_episodes) p.n_episodes[i] = episodes;
+}
+
+template <bool EPISODIC>
+__global__ void __launch_bounds__(128) qlearning_steps_kernel(const colo_mdp_tables tb, const colo_qlearning_args p,
+                                                              int n_steps, unsigned long long t0) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= p.N) return;
+  const colo_qlearning_inst c = {p.log_term, p.sqrt_h7sa, p.H_eff, p.gamma, p.span_approx};
+  qlearning_loop<EPISODIC>(tb, p, c, 0, 0, i, p.seed, p.env0 + (uint64_t)i, i, n_steps, t0);
+}
+
+// a mixed agent batch's instance: its constants and where its region of the flat tables starts
+struct MixedQInst {
+  colo_qlearning_inst c;
+  long long off_q, off_v;
+};
+
+// one loop per thread over the instances of a mixed batch: loop i is env i of the batch, on its instance's tables,
+// keys and constants, with counter i - start (bit-identical to the instance's single-MDP batch)
+template <bool EPISODIC>
+__global__ void __launch_bounds__(128) qlearning_mixed_steps_kernel(const MixedInst* __restrict__ insts,
+                                                                    const MixedQInst* __restrict__ qinsts,
+                                                                    const int* __restrict__ inst_of,
+                                                                    const colo_qlearning_args p, int n_steps,
+                                                                    unsigned long long t0) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= p.N) return;
+  const int k = __ldg(inst_of + i);
+  const MixedInst& d = insts[k];
+  const MixedQInst& q = qinsts[k];
+  const long long j = i - d.start;
+  qlearning_loop<EPISODIC>(d.tb, p, q.c, (size_t)q.off_q, (size_t)q.off_v, j, d.seed, (unsigned long long)j, i, n_steps,
+                           t0);
 }
 
 // PSRLEpisodic between two posterior samples (colosseum/agent/agents/episodic/posterior_sampling.py:142-147): act
@@ -228,6 +269,19 @@ __global__ void __launch_bounds__(128) psrl_steps_kernel(const colo_mdp_tables t
   if (p.n_episodes) p.n_episodes[i] = episodes;
 }
 
+// the buffers and shared hyper-parameters of a non-empty batch (single-MDP and mixed)
+static int check_loop_args(const colo_qlearning_args* a, bool episodic) {
+  COLO_ARG_CHECK(a->state && a->h && a->cnt && a->Q && a->V && a->cum_reward, "state, h, cnt, Q, V, cum_reward");
+  if (episodic) {
+    COLO_ARG_CHECK(a->ucb_type == 0 || (a->ucb_type == 1 && a->mu && a->sigma && a->beta && a->c_2 > 0),
+                   "ucb_type 0 (hoeffding) or 1 (bernstein with mu, sigma, beta, c_2)");
+    COLO_ARG_CHECK(a->c_1 > 0, "c_1 > 0");
+  } else {
+    COLO_ARG_CHECK(a->Q_main, "Q_main");
+  }
+  return COLO_OK;
+}
+
 static int check_args(const colo_mdp_tables* tb, const colo_qlearning_args* a, int n_steps, bool episodic) {
   COLO_ARG_CHECK(tb && a, "tables / args are NULL");
   COLO_ARG_CHECK(tb->S > 0 && tb->A > 0 && tb->rew_q && tb->n_cls > 0 && tb->nq >= 2, "tables");
@@ -236,14 +290,9 @@ static int check_args(const colo_mdp_tables* tb, const colo_qlearning_args* a, i
   COLO_ARG_CHECK(episodic ? tb->H > 0 : tb->H == 0, "episodic agents need H > 0, continuous agents H == 0");
   COLO_ARG_CHECK(a->N >= 0 && n_steps >= 1, "N >= 0, n_steps >= 1");
   if (a->N == 0) return COLO_OK;
-  COLO_ARG_CHECK(a->state && a->h && a->cnt && a->Q && a->V && a->cum_reward, "state, h, cnt, Q, V, cum_reward");
-  if (episodic) {
-    COLO_ARG_CHECK(a->ucb_type == 0 || (a->ucb_type == 1 && a->mu && a->sigma && a->beta && a->c_2 > 0),
-                   "ucb_type 0 (hoeffding) or 1 (bernstein with mu, sigma, beta, c_2)");
-    COLO_ARG_CHECK(a->c_1 > 0, "c_1 > 0");
-  } else {
-    COLO_ARG_CHECK(a->Q_main && a->H_eff > 0, "Q_main, H_eff");
-  }
+  const int r = check_loop_args(a, episodic);
+  if (r != COLO_OK) return r;
+  if (!episodic) COLO_ARG_CHECK(a->H_eff > 0, "Q_main, H_eff");
   return COLO_OK;
 }
 
@@ -283,6 +332,102 @@ int colo_psrl_episodic_steps(const colo_mdp_tables* tb, const colo_psrl_args* a,
   const int grid = (int)((a->N + 127) / 128);
   colo::psrl_steps_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(*tb, *a, n_steps, t0);
   return colo::check_launch("psrl_steps_kernel");
+}
+
+// ---- mixed agent batches ------------------------------------------------------------------------------------------------
+struct colo_mixed_qlearning {
+  const colo_mixed_tables* tables;
+  int episodic;
+  long long q_elems, v_elems;
+  colo::MixedQInst* insts;  // device [n_inst]
+};
+
+void colo_mixed_qlearning_destroy(colo_mixed_qlearning* q) {
+  if (!q) return;
+  if (q->insts) cudaFree(q->insts);
+  free(q);
+}
+
+int colo_mixed_qlearning_create(const colo_mixed_tables* tables, int episodic, const colo_qlearning_inst* host_insts,
+                                void* stream, colo_mixed_qlearning** out) {
+  COLO_ARG_CHECK(out && tables && host_insts, "tables, host_insts, out");
+  COLO_ARG_CHECK(episodic == 0 || episodic == 1, "episodic 0 or 1");
+  COLO_ARG_CHECK(tables->mode == 2, "colo_mixed_qlearning_create: the mixed tables must be made in successor mode (2)");
+  const int n_inst = tables->n_inst;
+  std::vector<colo::MixedQInst> insts((size_t)n_inst);
+  long long q_elems = 0, v_elems = 0;
+  for (int k = 0; k < n_inst; ++k) {
+    const colo::MixedInst& d = tables->host_insts[k];
+    const colo_qlearning_inst& c = host_insts[k];
+    const char* why = nullptr;
+    if (episodic ? d.tb.H <= 0 : d.tb.H != 0)
+      why = episodic ? "episodic agents need H > 0" : "continuous agents need H == 0";
+    else if (!(std::isfinite(c.log_term) && std::isfinite(c.sqrt_h7sa) && std::isfinite(c.H_eff) &&
+               std::isfinite(c.gamma) && std::isfinite(c.span_approx)))
+      why = "non-finite constant";
+    else if (!(c.sqrt_h7sa >= 0))
+      why = "sqrt_h7sa < 0";
+    else if (!episodic && !(c.H_eff > 0 && c.span_approx >= 0))
+      why = "continuous agents need H_eff > 0 and span_approx >= 0";
+    if (why) {
+      colo::set_error("colo_mixed_qlearning_create: instance %d: %s", k, why);
+      return COLO_ERR_ARG;
+    }
+    const long long n = (k + 1 < n_inst ? tables->host_insts[k + 1].start : tables->N) - d.start;
+    const long long S = d.tb.S, A = d.tb.A, H = d.tb.H;
+    insts[(size_t)k].c = c;
+    insts[(size_t)k].off_q = q_elems;
+    insts[(size_t)k].off_v = v_elems;
+    q_elems += n * (episodic ? H : 1) * S * A;
+    v_elems += n * (episodic ? H + 1 : 1) * S;
+  }
+  colo_mixed_qlearning* q = (colo_mixed_qlearning*)calloc(1, sizeof(colo_mixed_qlearning));
+  COLO_ARG_CHECK(q != nullptr, "out of host memory");
+  q->tables = tables;
+  q->episodic = episodic;
+  q->q_elems = q_elems;
+  q->v_elems = v_elems;
+  cudaStream_t st = (cudaStream_t)stream;
+  cudaError_t e = cudaMalloc((void**)&q->insts, sizeof(colo::MixedQInst) * (size_t)n_inst);
+  if (e == cudaSuccess)
+    e = cudaMemcpyAsync(q->insts, insts.data(), sizeof(colo::MixedQInst) * (size_t)n_inst, cudaMemcpyHostToDevice, st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);  // the host staging vector dies with this call
+  if (e != cudaSuccess) {
+    colo::set_error("colo_mixed_qlearning_create: %s", cudaGetErrorString(e));
+    colo_mixed_qlearning_destroy(q);
+    return COLO_ERR_CUDA;
+  }
+  *out = q;
+  return COLO_OK;
+}
+
+int colo_mixed_qlearning_sizes(const colo_mixed_qlearning* q, long long* q_elems, long long* v_elems) {
+  COLO_ARG_CHECK(q && q_elems && v_elems, "handle, q_elems, v_elems");
+  *q_elems = q->q_elems;
+  *v_elems = q->v_elems;
+  return COLO_OK;
+}
+
+int colo_mixed_qlearning_steps(const colo_mixed_qlearning* q, const colo_qlearning_args* a, int n_steps,
+                               unsigned long long t0, void* stream) {
+  COLO_ARG_CHECK(q && a, "handle / args are NULL");
+  COLO_ARG_CHECK(n_steps >= 1, "n_steps >= 1");
+  if (a->N != q->tables->N) {
+    colo::set_error("bad argument: args N = %lld, the mixed tables hold %lld loops", a->N, q->tables->N);
+    return COLO_ERR_ARG;
+  }
+  const int r = colo::check_loop_args(a, q->episodic);
+  if (r != COLO_OK) return r;
+  const int grid = (int)((a->N + 127) / 128);
+  const colo_mixed_tables* m = q->tables;
+  if (q->episodic) {
+    colo::qlearning_mixed_steps_kernel<true><<<grid, 128, 0, (cudaStream_t)stream>>>(m->insts, q->insts, m->inst_of,
+                                                                                     *a, n_steps, t0);
+    return colo::check_launch("qlearning_mixed_steps_kernel<episodic>");
+  }
+  colo::qlearning_mixed_steps_kernel<false><<<grid, 128, 0, (cudaStream_t)stream>>>(m->insts, q->insts, m->inst_of,
+                                                                                    *a, n_steps, t0);
+  return colo::check_launch("qlearning_mixed_steps_kernel<continuous>");
 }
 
 }  // extern "C"

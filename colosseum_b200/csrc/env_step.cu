@@ -22,6 +22,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "mixed.cuh"
 
 namespace colo {
 
@@ -892,17 +893,7 @@ __global__ void __launch_bounds__(kStepThreads) env_reset_kernel(const colo_mdp_
   }
 }
 
-// ---- mixed batches (colo_mixed_tables): envs of different MDP instances in one launch ---------------------------------
-// Instance i owns the contiguous envs [start, start + n_i).  Env e looks up its instance in inst_of[e] and then runs the
-// per-env code above on that instance's tables, Philox key and counter (seed_i; e - start), and counter offsets.  Envs of
-// one instance are contiguous, so the lanes of a warp almost always read the same descriptor (one broadcast load).
-struct MixedInst {
-  colo_mdp_tables tb;
-  unsigned long long seed;
-  long long start;          // first env of the instance
-  long long off_s, off_sa;  // sum of S, of S*A over the instances before it: its columns in the counter rows
-};
-
+// ---- mixed batches (colo_mixed_tables, mixed.cuh): envs of different MDP instances in one launch -----------------------
 __device__ __forceinline__ int mixed_inst_of(const int* __restrict__ inst_of, long long e, bool valid) {
   return valid ? __ldg(inst_of + e) : 0;  // lanes past the batch take part in the warp collectives as instance 0
 }
@@ -1337,13 +1328,6 @@ int colo_env_random_steps(const colo_mdp_tables* tb, const colo_env_batch* batch
 }
 
 // ---- mixed batches ------------------------------------------------------------------------------------------------------
-struct colo_mixed_tables {
-  int n_inst, mode;
-  long long N, sum_s, sum_sa;
-  colo::MixedInst* insts;  // device [n_inst]
-  int* inst_of;            // device [N]: instance of every env
-};
-
 static int mixed_check_instance(const colo_mdp_tables* tb, int mode) {
   int r = colo::check_tables_common(tb);
   if (r != COLO_OK) return r;
@@ -1360,6 +1344,7 @@ void colo_mixed_tables_destroy(colo_mixed_tables* h) {
   if (!h) return;
   if (h->insts) cudaFree(h->insts);
   if (h->inst_of) cudaFree(h->inst_of);
+  free(h->host_insts);
   free(h);
 }
 
@@ -1403,6 +1388,12 @@ int colo_mixed_tables_create(const colo_mdp_tables* host_tables, int n_inst, con
   h->N = N;
   h->sum_s = sum_s;
   h->sum_sa = sum_sa;
+  h->host_insts = (colo::MixedInst*)malloc(sizeof(colo::MixedInst) * (size_t)n_inst);
+  if (h->host_insts == nullptr) {
+    colo_mixed_tables_destroy(h);
+    COLO_ARG_CHECK(false, "out of host memory");
+  }
+  memcpy(h->host_insts, insts.data(), sizeof(colo::MixedInst) * (size_t)n_inst);
   cudaStream_t st = (cudaStream_t)stream;
   cudaError_t e = cudaMalloc((void**)&h->insts, sizeof(colo::MixedInst) * (size_t)n_inst);
   if (e == cudaSuccess) e = cudaMalloc((void**)&h->inst_of, sizeof(int) * (size_t)N);

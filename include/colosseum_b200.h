@@ -799,6 +799,39 @@ int colo_qlearning_continuous_steps(const colo_mdp_tables* tb, const colo_qlearn
                                     unsigned long long t0, void* stream);
 
 /*
+ * Mixed agent batches -- Q-learning loops on the instances of a mixed batch (colo_mixed_tables, successor mode), all
+ * advanced by ONE launch per colo_mixed_qlearning_steps whatever the number of instances: a benchmark's whole suite of
+ * instances x seeds at once.  Loop i is env i of the mixed batch: it belongs to instance k with start_k <= i <
+ * start_k + n_k and runs colo_qlearning_{episodic,continuous}_steps' body on instance k's tables with env key seeds[k],
+ * agent key seeds[k] ^ 0x9E3779B97F4A7C15, Boltzmann key seeds[k] ^ 0x94D049BB133111EB and counter (i - start_k, t):
+ * instance k's loops are bit-identical to a single-MDP batch of n_k loops with seed = seeds[k], env0 = 0.
+ *   colo_qlearning_inst: instance k's constants, derived from its S, A, H as the single-MDP calls' fields of the same
+ *   names (episodic: log_term, sqrt_h7sa; continuous: log_term, H_eff, gamma = 1 - 1/H_eff, span_approx).
+ *   Layout of the flat tables (colo_qlearning_args' cnt, Q, Q_main, mu, sigma, beta; V): instance k's region holds its
+ *   loops as [n_k, H_k, S_k, A_k] (continuous [n_k, S_k, A_k]); V [n_k, H_k + 1, S_k] (continuous [n_k, S_k]); the
+ *   regions follow each other in instance order.  colo_mixed_qlearning_sizes gives the element counts of the Q-shaped
+ *   and the V-shaped tables.  state, h, cum_reward, n_episodes are flat [N]; trace is [n_steps, N, 4].
+ * colo_mixed_qlearning_create -- episodic 1 (every instance needs H > 0) or 0 (every instance H == 0);
+ *   host_insts[n_inst].  Checks the handle (successor mode) and every instance on the host before any CUDA call
+ *   (COLO_ERR_ARG, colo_last_error names the instance): H against `episodic`, constants finite, sqrt_h7sa >= 0,
+ *   continuous H_eff > 0 and span_approx >= 0.  Then uploads the per-instance descriptors on `stream` and synchronises
+ *   it.  `tables` must outlive the handle.
+ * colo_mixed_qlearning_steps -- args as for the single-MDP calls, except that N must equal the mixed batch's env count
+ *   and that seed, env0, log_term, sqrt_h7sa, H_eff, gamma and span_approx are taken from the handle (the shared
+ *   hyper-parameters ucb_type, c_1, c_2, min_at, epsilon_greedy and the actor come from args).  Does not synchronise.
+ */
+typedef struct {
+  double log_term, sqrt_h7sa, H_eff, gamma, span_approx;
+} colo_qlearning_inst;
+typedef struct colo_mixed_qlearning colo_mixed_qlearning;
+int colo_mixed_qlearning_create(const colo_mixed_tables* tables, int episodic, const colo_qlearning_inst* host_insts,
+                                void* stream, colo_mixed_qlearning** out);
+int colo_mixed_qlearning_sizes(const colo_mixed_qlearning* q, long long* q_elems, long long* v_elems);
+int colo_mixed_qlearning_steps(const colo_mixed_qlearning* q, const colo_qlearning_args* a, int n_steps,
+                               unsigned long long t0, void* stream);
+void colo_mixed_qlearning_destroy(colo_mixed_qlearning* q);
+
+/*
  * colo_psrl_episodic_steps -- PSRLEpisodic between two posterior samples (agent/agents/episodic/posterior_sampling.py:
  * 142-147) for N independent loops: greedy / epsilon-greedy action on Q f32[N,H+1,S,A] (the episodic value iteration of
  * each loop's sampled model), BaseMDP.step, BayesianMDPModel.step_update (agent/mdp_models/bayesian_model.py:78-92):
