@@ -13,7 +13,7 @@ OK, OVERFLOW, MAX_ITER, NEEDS_RESET, SERVER_LAPSED, BAD_ACTION = 0, 1, 2, 3, 4, 
 FOLD_MAX, FOLD_PI, FOLD_MIN = 0, 1, 2
 STEP_FIRST, STEP_MID, STEP_LAST = 0, 1, 2
 # step-kernel variants of colo_step_kernel_launches (include/colosseum_b200.h, COLO_STEP_KIND_*)
-STEP_KIND_LEAN, STEP_KIND_KARY, STEP_KIND_SHORT, STEP_KIND_LONG, STEP_KIND_SUCC = 0, 1, 2, 3, 4
+STEP_KIND_LEAN, STEP_KIND_KARY, STEP_KIND_LONG, STEP_KIND_SUCC = 0, 1, 3, 4  # kind 2 is retired
 STEP_KIND_MIXED_SUCC, STEP_KIND_MIXED_DENSE = 5, 6
 STEP_KIND_BREAKS, STEP_KIND_BREAKS_GENERAL = 7, 8
 # Bellman-solver paths of colo_solver_path_launches (include/colosseum_b200.h, COLO_PATH_*)

@@ -7,7 +7,8 @@
     ts, actions = env.random_step()   # BaseMDP.random_step for every env
 
 With n_envs=1, `ts.scalar()` is the reference's scalar dm_env.TimeStep.  Modes:
-  dense_f32 / dense_f64   warp-cooperative inverse-CDF search over the dense CDF row of T[s,a,:]
+  dense_f32 / dense_f64   inverse-CDF search over the dense CDF row of T[s,a,:] (a k-ary search or the row's
+                          breakpoint table; a warp-cooperative count for rows of more than 1024 states)
   succ                    successor-list tables in the reference sampler's own order: bit-exact with
                           NextStateSampler.sample for the same fp64 uniform (mdp/utils/custom_samplers.py:49-72)
 Uniforms may be supplied (`u_next`, `u_reward`) or come from the in-kernel Philox4x32-10 stream keyed by

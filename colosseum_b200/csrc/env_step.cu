@@ -7,10 +7,10 @@
 //                 tabulated quantile function, then the reference's rescale r*(max-min) - min (sic)
 //   bookkeeping : h, episodic termination (LAST, obs -1), auto-reset, visitation counts on the NEXT node (sic).
 //
-// Dense kernel: a warp owns a tile of 32 consecutive envs.  Env scalars are loaded / stored coalesced (lane i <->
-// env i); the search over the dense CDF row T[s,a,:] is warp-cooperative: the row is read with 128-bit coalesced
-// loads, all issued before any is consumed, and because the row is monotone the bisect position is simply the
-// COUNT of entries <= x, i.e. one integer warp reduction, no branches and no early exit.
+// Dense rows of at most 1024 states: one thread per env, a three-round k-ary search of the row or one round over the
+// row's breakpoint table (env_step_dense_kary_kernel); the common call takes the lean form of either
+// (env_step_kary_lean_kernel, env_step_breaks_lean_kernel).  Longer rows (env_step_dense_kernel): a warp owns a tile of
+// 32 envs and searches each env's row together, counting the entries <= x with one ballot per chunk.
 #include <stdlib.h>
 #include <string.h>
 #include <time.h>
@@ -392,96 +392,6 @@ __global__ void __launch_bounds__(kStepThreads) env_step_dense_kernel(const colo
   }
 }
 
-// SHORT rows (ld == 128 * NCH, NCH <= 8; the host pads rows of S <= 1024 to whole 128-entry chunks):
-// branch-free, software-pipelined variant.  For U envs at a time the warp issues every row load (U * NCH 128-bit
-// loads per lane in flight), then finds for each env the number G of quads lying entirely at or below x with one
-// ballot + popc per chunk.  The within-quad step is deferred to the epilogue, where lane i finishes env i on its
-// own (one 16-byte gather of quad G, which the warp has just pulled into L1), i.e. it is vectorised over the 32
-// envs of the tile instead of costing shuffles and selects inside the per-env loop.
-template <typename TC, int NCH, int U, int TILE, bool SERVER>
-__global__ void __launch_bounds__(kStepThreads) env_step_dense_short_kernel(const colo_mdp_tables tb, const StepIO io) {
-  // TILE envs per warp (lanes >= TILE idle in the per-lane phases): smaller tiles = more warps in flight when the
-  // batch alone cannot fill the machine (65,536 envs / 32 = 14 warps per SM)
-  const int lane = threadIdx.x & 31;
-  const long long warp_global = ((long long)blockIdx.x * kStepThreads + threadIdx.x) >> 5;
-  const long long n_warps = ((long long)gridDim.x * kStepThreads) >> 5;
-  const long long n_tiles = (io.N + TILE - 1) / TILE;
-  const int S = tb.S, A = tb.A;
-  constexpr int ld = 128 * NCH;
-  const TC* __restrict__ cdf = reinterpret_cast<const TC*>(tb.cdf);
-  constexpr bool F32U = sizeof(TC) == 4;
-
-  for (unsigned long long pass = io.srv_seq0 + 1;; ++pass) {  // SERVER: one pass per doorbell; else exactly one pass
-  unsigned long long t_pass = step_t0(io);
-  if (SERVER) {
-    if (!server_wait(io, pass)) return;
-    t_pass += pass - io.srv_seq0 - 1;
-  }
-  for (long long tile = warp_global; tile < n_tiles; tile += n_warps)
-  for (int step = 0; step < io.n_steps; ++step) {  // an env is owned by the same lane for every step of the launch
-    const long long e = tile * TILE + lane;
-    const bool valid = lane < TILE && e < io.N;
-    EnvIn in;
-    in.s = 0; in.a = 0; in.st = COLO_STEP_MID; in.h = 0; in.bad = 0; in.un64 = 0.0; in.un32 = 0.f; in.ur = 0.f;
-    if (valid) in = load_env<F32U>(io, tb, e, t_pass + step);
-    const bool is_last = valid && in.st == COLO_STEP_LAST;
-    const bool resetting = is_last && io.auto_reset;
-    const bool stepping = valid && !is_last && !in.bad;
-    if (is_last && !io.auto_reset && io.status) *io.status = COLO_NEEDS_RESET;
-    // lanes that do not step take part with row 0 (keeps the loop branch-free); 32-bit element offsets
-    // (the host checks S*A*ld < 2^31)
-    const unsigned off_l = stepping ? (unsigned)(in.s * A + in.a) * (unsigned)ld : 0u;
-    const TC u_l = F32U ? (TC)in.un32 : (TC)in.un64;
-
-    int my_G = 0;
-    for (int i0 = 0; i0 < TILE; i0 += U) {
-      Quad<TC> q[U][NCH];
-      TC x[U];
-#pragma unroll
-      for (int k = 0; k < U; ++k) {
-        const unsigned off = __shfl_sync(FULL, off_l, i0 + k);
-        const TC u = __shfl_sync(FULL, u_l, i0 + k);
-        const TC* row = cdf + off;
-        x[k] = u * __ldg(row + S - 1);
-#pragma unroll
-        for (int c = 0; c < NCH; ++c) q[k][c].load(row + c * 128 + lane * 4);
-      }
-#pragma unroll
-      for (int k = 0; k < U; ++k) {
-        int G = 0;
-#pragma unroll
-        for (int c = 0; c < NCH; ++c) G += __popc(__ballot_sync(FULL, q[k][c].v[3] <= x[k]));
-        my_G = (lane == i0 + k) ? G : my_G;
-      }
-    }
-    // per-lane finish: env `lane` of the tile
-    int nxt = 0, cls = 0;
-    if (stepping) {
-      const TC* row = cdf + off_l;
-      const TC total = __ldg(row + S - 1);
-      const TC xl = u_l * total;  // same operands, same product as in the search above
-      nxt = ld;
-      if (my_G < 32 * NCH) {
-        Quad<TC> qq;
-        qq.load(row + 4 * my_G);  // the crossing quad: its last entry is > x, its first three decide
-        nxt = 4 * my_G + (qq.v[0] <= xl) + (qq.v[1] <= xl) + (qq.v[2] <= xl);
-      }
-      if (nxt >= S) {  // x >= total (rounding): bisect's hi = n-1 clamp == first index where the row reaches total
-        nxt = 0;
-        while (nxt < S - 1 && __ldg(row + nxt) < total) ++nxt;
-      }
-      if (tb.rew_cls_sas)
-        cls = tb.rew_cls_sas[((size_t)in.s * A + in.a) * S + nxt];
-      else if (tb.rew_cls_sa)
-        cls = tb.rew_cls_sa[(size_t)in.s * A + in.a];
-    }
-    finish_env(io, tb, valid ? e : 0, in, nxt, cls, stepping, resetting);
-  }
-  if (!SERVER) return;
-  server_done(io, pass);
-  }
-}
-
 // ---- breakpoint table (colo_mdp_tables.cdf_breaks) ----------------------------------------------------------------------
 // Most benchmark rows have a handful of successors, so the CDF row is a step function with a few breakpoints p_k (where
 // c[p_k] > c[p_k - 1]).  For x >= 0 the count of entries <= x over the whole padded row, with the clamp to the first
@@ -530,18 +440,17 @@ __device__ __forceinline__ BreakStep breaks_step(const void* table, unsigned r, 
   return b;
 }
 
-// SHORT rows, one THREAD per env: a three-round k-ary search instead of reading the whole row.  The last entries of
-// the row's quads are monotone, so the number G of quads lying entirely at or below x is found from (1) the last entry
-// of every 8th quad (4*NCH independent 4-byte loads, all issued before any is consumed), (2) the last entries of the 8
-// quads of the block that holds the crossing, (3) the crossing quad itself (the same 16-byte gather the warp-
-// cooperative kernel ends with).  With the two-level index of colo_mdp_tables (cdf_coarse / cdf_mid: copies of exactly
-// those entries, contiguous) round 1 is NCH 128-bit loads of a 60 KB table and also yields the row total; round 2 is
-// one 32-byte sector of cdf_mid plus, in the same round, the 32-byte sector of reward classes of the block's candidate
-// next states (rew_cls_pad); round 3 the crossing quad.  Three dependent rounds per env after the env scalars, instead
-// of 32/U per tile plus two.  (Tried on one box each: reading the whole 128-byte block in round 2 and skipping round 3
-// -- 5.58 us per step instead of 5.17: four sectors cost more than one extra round; fetching the reward quantiles of
-// every class before the search -- 5.50 us instead of 5.26.)  With 65,536 envs every warp is resident at once, so the step time IS the length of
-// that dependency chain.  Same comparisons against the same x => the same index, bit for bit.
+// Rows of at most 1024 states, one THREAD per env: a three-round k-ary search instead of reading the whole row.  The last
+// entries of the row's quads are monotone, so the number G of quads lying entirely at or below x is found from (1) the
+// last entry of every 8th quad (4*NCH independent 4-byte loads, all issued before any is consumed), (2) the last entries
+// of the 8 quads of the block that holds the crossing, (3) the crossing quad itself.  With the two-level index of
+// colo_mdp_tables (cdf_coarse / cdf_mid: copies of exactly those entries, contiguous) round 1 is NCH 128-bit loads of a
+// 60 KB table and also yields the row total; round 2 is one 32-byte sector of cdf_mid plus, in the same round, the
+// 32-byte sector of reward classes of the block's candidate next states (rew_cls_pad); round 3 the crossing quad: three
+// dependent rounds per env after the env scalars.  (Tried on one box each: reading the whole 128-byte block in round 2
+// and skipping round 3 -- 5.58 us per step instead of 5.17: four sectors cost more than one extra round; fetching the
+// reward quantiles of every class before the search -- 5.50 us instead of 5.26.)  With 65,536 envs every warp is
+// resident at once, so the step time IS the length of that dependency chain.  Same comparisons against the same x => the same index, bit for bit.
 // KB > 0 (f32): the search is one round over the KB-entry breakpoint row instead (NCH is then unused).
 template <typename TC, int NCH, bool SERVER, int KB = 0>
 __global__ void __launch_bounds__(kStepThreads) env_step_dense_kary_kernel(const colo_mdp_tables tb, const StepIO io) {
@@ -1120,20 +1029,13 @@ static int launch_dense(const colo_mdp_tables* tb, const StepIO& io, void* strea
   const int ld = tb->ld;
   const bool short_rows = ld % 128 == 0 && ld <= 1024 && (long long)tb->S * tb->A * ld < (1LL << 31);
   if (short_rows) {
-    // envs per warp: 32 when the batch alone fills the machine, fewer (more warps in flight) otherwise
-    static const int forced = getenv("COLO_STEP_TILE") ? atoi(getenv("COLO_STEP_TILE")) : 0;
-    const long long warps32 = (io.N + 31) / 32;
-    // measured on B200 at N=65,536 (14 warps/SM with 32-env tiles): 32 -> 14.1 us, 16 -> 14.4 us, 8 -> 16.6 us
-    int tile = warps32 >= (long long)sm_count() * 8 ? 32 : (warps32 >= (long long)sm_count() * 4 ? 16 : 8);
-    if (forced == 8 || forced == 16 || forced == 32) tile = forced;
-    // thread-per-env k-ary search (default) or the warp-cooperative full-row count (COLO_STEP_KERNEL=coop)
-    static const bool coop = getenv("COLO_STEP_KERNEL") && !strcmp(getenv("COLO_STEP_KERNEL"), "coop");
+    // COLO_STEP_KERNEL=general sends the common call to the general kernel too, so that tests can pin it there
     static const bool no_lean = getenv("COLO_STEP_KERNEL") && !strcmp(getenv("COLO_STEP_KERNEL"), "general");
     // the breakpoint table (f32 only) replaces the row search and the index in both thread-per-env kernels
     const int kb = sizeof(TC) == 4 && tb->cdf_breaks ? tb->cdf_breaks_k : 0;
     COLO_ARG_CHECK(kb == 0 || kb == 2 || kb == 4 || kb == 8 || kb == 16, "cdf_breaks_k must be 2, 4, 8 or 16");
     COLO_ARG_CHECK(kb == 0 || (uintptr_t)tb->cdf_breaks % 16 == 0, "cdf_breaks must be 16-byte aligned");
-    if (!coop && !no_lean && !SERVER && sizeof(TC) == 4 && io.n_steps == 1 && !io.random_actions && io.u_next == nullptr &&
+    if (!no_lean && !SERVER && sizeof(TC) == 4 && io.n_steps == 1 && !io.random_actions && io.u_next == nullptr &&
         io.u_rew == nullptr && io.auto_reset && (kb || (tb->cdf_mid && tb->cdf_coarse && tb->rew_cls_pad)) && io.visits_s &&
         io.visits_sa && io.N < (1LL << 31) - kLeanThreads) {
       const int gl = (int)((io.N + kLeanThreads - 1) / kLeanThreads);
@@ -1174,61 +1076,39 @@ static int launch_dense(const colo_mdp_tables* tb, const StepIO& io, void* strea
     }
     COLO_ARG_CHECK(!io.io_compact, "io_compact is offered by the common call of the dense f32 step only (supplied actions, "
                                    "in-kernel uniforms, auto_reset, CDF index present, counters on, no server)");
-    if (!coop) {
-      const int gk = grid_for(kStepThreads, io.N);
-      if (kb) {
-        switch (kb) {
-          case 2: launch_step(env_step_dense_kary_kernel<float, 1, SERVER, 2>, gk, SERVER, share, tb, io, st); break;
-          case 4: launch_step(env_step_dense_kary_kernel<float, 1, SERVER, 4>, gk, SERVER, share, tb, io, st); break;
-          case 8: launch_step(env_step_dense_kary_kernel<float, 1, SERVER, 8>, gk, SERVER, share, tb, io, st); break;
-          case 16: launch_step(env_step_dense_kary_kernel<float, 1, SERVER, 16>, gk, SERVER, share, tb, io, st); break;
-        }
-        count_step_launch(COLO_STEP_KIND_BREAKS_GENERAL);
-        return check_launch("env_step_dense_kary_kernel");
+    const int gk = grid_for(kStepThreads, io.N);
+    if (kb) {
+      switch (kb) {
+        case 2: launch_step(env_step_dense_kary_kernel<float, 1, SERVER, 2>, gk, SERVER, share, tb, io, st); break;
+        case 4: launch_step(env_step_dense_kary_kernel<float, 1, SERVER, 4>, gk, SERVER, share, tb, io, st); break;
+        case 8: launch_step(env_step_dense_kary_kernel<float, 1, SERVER, 8>, gk, SERVER, share, tb, io, st); break;
+        case 16: launch_step(env_step_dense_kary_kernel<float, 1, SERVER, 16>, gk, SERVER, share, tb, io, st); break;
       }
+      count_step_launch(COLO_STEP_KIND_BREAKS_GENERAL);
+      return check_launch("env_step_dense_kary_kernel");
+    }
 #define COLO_KARY(NCH)                                                                              \
   case NCH:                                                                                         \
     launch_step(env_step_dense_kary_kernel<TC, NCH, SERVER>, gk, SERVER, share, tb, io, st);        \
     break
-      switch (ld / 128) {
-        COLO_KARY(1);
-        COLO_KARY(2);
-        COLO_KARY(3);
-        COLO_KARY(4);
-        COLO_KARY(5);
-        COLO_KARY(6);
-        COLO_KARY(7);
-        COLO_KARY(8);
-      }
-#undef COLO_KARY
-      count_step_launch(COLO_STEP_KIND_KARY);
-      return check_launch("env_step_dense_kary_kernel");
-    }
-    const int grid = grid_for(kStepThreads / 32, (io.N + tile - 1) / tile);
-#define COLO_SHORT(NCH, U)                                                                                        \
-  case NCH:                                                                                                       \
-    if (tile == 32) launch_step(env_step_dense_short_kernel<TC, NCH, U, 32, SERVER>, grid, SERVER, share, tb, io, st);      \
-    else if (tile == 16) launch_step(env_step_dense_short_kernel<TC, NCH, U, 16, SERVER>, grid, SERVER, share, tb, io, st); \
-    else launch_step(env_step_dense_short_kernel<TC, NCH, U, 8, SERVER>, grid, SERVER, share, tb, io, st);                  \
-    break
     switch (ld / 128) {
-      COLO_SHORT(1, 4);
-      COLO_SHORT(2, 4);
-      COLO_SHORT(3, 4);
-      COLO_SHORT(4, 4);
-      COLO_SHORT(5, 2);
-      COLO_SHORT(6, 2);
-      COLO_SHORT(7, 2);
-      COLO_SHORT(8, 2);
+      COLO_KARY(1);
+      COLO_KARY(2);
+      COLO_KARY(3);
+      COLO_KARY(4);
+      COLO_KARY(5);
+      COLO_KARY(6);
+      COLO_KARY(7);
+      COLO_KARY(8);
     }
-#undef COLO_SHORT
-    count_step_launch(COLO_STEP_KIND_SHORT);
-  } else {
-    COLO_ARG_CHECK(!io.io_compact, "io_compact needs rows of at most 1024 states");
-    const int grid = grid_for(kStepThreads / 32, (io.N + 31) / 32);
-    launch_step(env_step_dense_kernel<TC, 8, SERVER>, grid, SERVER, share, tb, io, st);
-    count_step_launch(COLO_STEP_KIND_LONG);
+#undef COLO_KARY
+    count_step_launch(COLO_STEP_KIND_KARY);
+    return check_launch("env_step_dense_kary_kernel");
   }
+  COLO_ARG_CHECK(!io.io_compact, "io_compact needs rows of at most 1024 states");
+  const int grid = grid_for(kStepThreads / 32, (io.N + 31) / 32);
+  launch_step(env_step_dense_kernel<TC, 8, SERVER>, grid, SERVER, share, tb, io, st);
+  count_step_launch(COLO_STEP_KIND_LONG);
   return check_launch("env_step_dense_kernel");
 }
 

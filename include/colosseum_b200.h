@@ -62,7 +62,7 @@ unsigned long long colo_backup_tma_sweeps(void);
  * Counted on the host when the launch is enqueued: a launch captured into a CUDA graph counts once. */
 #define COLO_STEP_KIND_LEAN 0  /* env_step_kary_lean_kernel: the common dense f32 call                         */
 #define COLO_STEP_KIND_KARY 1  /* env_step_dense_kary_kernel: rows of <= 1024 states, every other dense call    */
-#define COLO_STEP_KIND_SHORT 2 /* env_step_dense_short_kernel: the warp-cooperative kernel (COLO_STEP_KERNEL=coop) */
+/* kind 2 is retired: no kernel counts there                                                             */
 #define COLO_STEP_KIND_LONG 3  /* env_step_dense_kernel: rows of more than 1024 states (or ld % 128 != 0)      */
 #define COLO_STEP_KIND_SUCC 4  /* env_step_succ_kernel: successor-list tables                                  */
 #define COLO_STEP_KIND_MIXED_SUCC 5  /* env_step_succ_mixed_kernel: a mixed batch, successor-list tables       */

@@ -30,8 +30,7 @@ def timeit(env, steps=200, do_flush=False, random_actions=False, acts=None):
     b.record(); torch.cuda.synchronize()
     return a.elapsed_time(b) / steps * 1e3
 
-print("COLO_STEP_TILE =", os.environ.get("COLO_STEP_TILE"))
-for mode in (("dense_f32",) if os.environ.get("COLO_STEP_TILE") else ("dense_f32", "dense_f64", "succ")):
+for mode in ("dense_f32", "dense_f64", "succ"):
     for visits in (True, False):
         env = BatchedMDP(tb, N, mode=mode, seed=1, track_visits=visits)
         env.reset()

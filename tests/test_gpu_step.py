@@ -550,8 +550,7 @@ def test_correlated_emission_noises(bm):
 @pytest.mark.parametrize("mode", ["dense_f32", "dense_f64"])
 def test_step_without_search_index_is_identical(bm, mode):
     """colo_mdp_tables.cdf_mid / cdf_coarse / rew_cls_pad are optional: with NULL pointers the k-ary kernel samples the
-    same entries from the row itself -- bit-identical to the indexed default.  (Running this whole file with
-    COLO_STEP_KERNEL=coop exercises the warp-cooperative kernel against the same oracles.)"""
+    same entries from the row itself -- bit-identical to the indexed default."""
     import torch
 
     tb = MDPTables.from_golden(load_instance("c2_deepsea30_prand"))

@@ -1,10 +1,10 @@
 """GPU parity of every dense step-kernel variant at every row width it is compiled for.
 
 The dense step has one instantiation per row width NCH = ld / 128 = 1..8 (rows of at most 1024 states) for each of
-the lean kernel (the common f32 call), the general k-ary kernel (fp32 and fp64), the warp-cooperative kernel
-(COLO_STEP_KERNEL=coop, tiles of 8, 16 and 32 envs), plus the long-row kernel (more than 1024 states).  Every case here
-runs synthetic MDPs through one of them and compares state, h, step_type, observation, reward bits, discount and both
-visitation tables with the C oracle, bit for bit; `colo_step_kernel_launches` proves which variant ran.
+the lean kernel (the common f32 call) and the general k-ary kernel (fp32 and fp64), plus the long-row kernel (more
+than 1024 states).  Every case here runs synthetic MDPs through one of them and compares state, h, step_type,
+observation, reward bits, discount and both visitation tables with the C oracle, bit for bit;
+`colo_step_kernel_launches` proves which variant ran.
 
 The MDPs are built so that the search meets its hard cases: exact ties x == cdf[j] (bisect_right goes past j and past
 any flat run of zero-probability states after it) at quad, block and chunk ends, also inside the lean kernel, whose
@@ -28,9 +28,9 @@ pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
-LEAN, KARY, SHORT, LONG, SUCC = range(5)  # COLO_STEP_KIND_* of include/colosseum_b200.h
-KIND_NAMES = ["env_step_kary_lean_kernel", "env_step_dense_kary_kernel", "env_step_dense_short_kernel",
-              "env_step_dense_kernel", "env_step_succ_kernel"]
+LEAN, KARY, LONG, SUCC = 0, 1, 3, 4  # COLO_STEP_KIND_* of include/colosseum_b200.h (kind 2 is retired)
+KIND_NAMES = {LEAN: "env_step_kary_lean_kernel", KARY: "env_step_dense_kary_kernel", LONG: "env_step_dense_kernel",
+              SUCC: "env_step_succ_kernel"}
 
 # states of each row width: no padding, and one state in the last chunk (plus a few odd sizes)
 WIDTH_S = {k: [128 * k, 128 * (k - 1) + 1] for k in range(1, 9)}
@@ -175,8 +175,6 @@ def step_inputs(case, tb, dyadic, cdf, i, kind):
 def expected_kind(case, kind, stripped=False):
     if case["S"] > 1024:
         return LONG
-    if case.get("force") == "coop":
-        return SHORT
     lean_shaped = kind in ("lean_tie", "act")
     if lean_shaped and case["mode"] == "dense_f32" and case.get("force") != "general" and not stripped:
         return LEAN
@@ -393,26 +391,6 @@ def run_children(tmp_path, force, cases):
     for k, case in enumerate(cases):
         with np.load(tmp_path / f"{k}.npz") as z:
             check_case(case, dict(z))
-
-
-def test_warp_cooperative_kernel_matches_oracle(tmp_path):
-    """env_step_dense_short_kernel<TC, NCH, U, TILE> (COLO_STEP_KERNEL=coop) at every width in both precisions; the
-    tile follows from N: 37 envs -> 8, 4 x SMs x 32 -> 16, 8 x SMs x 32 -> 32"""
-    import torch
-
-    sms = torch.cuda.get_device_properties(0).multi_processor_count
-    cases = []
-    for nch in range(1, 9):
-        for m, mode in enumerate(["dense_f32", "dense_f64"]):
-            for j, N in enumerate([37, 4 * sms * 32, 8 * sms * 32]):
-                S = WIDTH_S[nch][(m + j) % 2]
-                plan = [("lean_tie", 1), ("u_tie", 1), ("u", 1), ("act", 1), ("rand", 1)]
-                if N == 37:
-                    plan += [("fused", 4)]
-                cases.append(dict(S=S, A=a_for(S, nch + j), H=[0, 3][j % 2], N=N, env0=17 * j,
-                                  seed=SEED + 1000 + 10 * nch + 3 * m + j, mode=mode, io="device", plan=plan,
-                                  force="coop"))
-    run_children(tmp_path, "coop", cases)
 
 
 def test_forced_general_kernel_matches_oracle(tmp_path):
