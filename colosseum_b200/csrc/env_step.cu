@@ -11,6 +11,13 @@
 // row's breakpoint table (env_step_dense_kary_kernel); the common call takes the lean form of either
 // (env_step_kary_lean_kernel, env_step_breaks_lean_kernel).  Longer rows (env_step_dense_kernel): a warp owns a tile of
 // 32 envs and searches each env's row together, counting the entries <= x with one ballot per chunk.
+//
+// The general per-env paths (dense, k-ary, successor lists, mixed batches) share one prologue (begin_env), one
+// epilogue (finish_env) and, where a persistent step server runs them, one pass loop (run_passes); the two warp-per-env
+// kernels share one tile search (warp_tile_next); finish_env and reset_env share the FIRST-TimeStep stores
+// (store_first).  The lean kernels keep their own prologue, epilogue and index rounds (lean_load, lean_store) and share
+// the class-word select and the clamp (block_cls, row_clamp) with the general k-ary kernel: calling the general helpers
+// from them changes their instructions (profiles/r3_step_refactor_sass.txt).
 #include <stdlib.h>
 #include <string.h>
 #include <time.h>
@@ -200,12 +207,13 @@ struct Quad<double> {
   }
 };
 
-// per-env prologue shared by all step kernels: resolves uniforms/actions, handles the reset path.
-// returns true when the env takes a regular step.
+// one env's inputs to a step: its scalars, uniforms and action; whether it resets (auto_reset of a LAST env) or takes a
+// regular step
 struct EnvIn {
   int s, a, st, h, bad;
   double un64;
   float un32, ur;
+  bool resetting, stepping;
 };
 
 // `seed` / `ctr`: the env's Philox key and counter -- (io.seed, io.env0 + e) in a single-MDP batch, (the instance's
@@ -243,27 +251,45 @@ __device__ __forceinline__ EnvIn load_env(const StepIO& io, const colo_mdp_table
   return in;
 }
 
+// the prologue of every general per-env step path; a lane past the batch (!valid) gets zero inputs and neither resets
+// nor steps.  A LAST env without auto_reset raises COLO_NEEDS_RESET.
 template <bool F32U>
-__device__ __forceinline__ EnvIn load_env(const StepIO& io, const colo_mdp_tables& tb, long long e,
-                                           unsigned long long t) {
-  return load_env<F32U>(io, tb, e, t, io.seed, io.env0 + (uint64_t)e);
+__device__ __forceinline__ EnvIn begin_env(const StepIO& io, const colo_mdp_tables& tb, long long e, bool valid,
+                                            unsigned long long t, unsigned long long seed, unsigned long long ctr) {
+  EnvIn in;
+  in.s = 0; in.a = 0; in.st = COLO_STEP_MID; in.h = 0; in.bad = 0; in.un64 = 0.0; in.un32 = 0.f; in.ur = 0.f;
+  if (valid) in = load_env<F32U>(io, tb, e, t, seed, ctr);
+  const bool is_last = valid && in.st == COLO_STEP_LAST;
+  in.resetting = is_last && io.auto_reset;
+  in.stepping = valid && !is_last && !in.bad;
+  if (is_last && !io.auto_reset && io.status) *io.status = COLO_NEEDS_RESET;
+  return in;
 }
 
-// epilogue of a regular step for one env held by this thread.  off_s / off_sa: where the env's MDP starts in the
-// counter rows (non-zero in a mixed batch, whose instances share one concatenated [copies][sum S] / [copies][sum S*A])
+// the stores of a FIRST TimeStep at start state s0 (BaseMDP.reset: the reference's reward is None, NaN here)
+__device__ __forceinline__ void store_first(const StepIO& io, long long e, int s0, bool compact) {
+  io.state[e] = s0;
+  io.h[e] = 0;
+  io.step_type[e] = COLO_STEP_FIRST;
+  if (io.step_type_mirror) io.step_type_mirror[e] = COLO_STEP_FIRST;
+  if (io.discount) io.discount[e] = __int_as_float(0x7fc00000);
+  if (io.reward) io.reward[e] = __int_as_float(0x7fc00000);
+  if (compact)
+    reinterpret_cast<short*>(io.obs)[e] = (short)s0;
+  else
+    io.obs[e] = s0;
+}
+
+// epilogue of a step for one env held by this thread.  off_s / off_sa: where the env's MDP starts in the counter rows
+// (non-zero in a mixed batch, whose instances share one concatenated [copies][sum S] / [copies][sum S*A])
 // have_rew: `rew` is the reward of the step (a constant class resolved by the breakpoint table), no draw needed
 __device__ __forceinline__ void finish_env(const StepIO& io, const colo_mdp_tables& tb, long long e, const EnvIn& in,
-                                           int nxt, int cls, bool stepping, bool resetting, long long off_s = 0,
-                                           long long off_sa = 0, bool have_rew = false, float rew = 0.f) {
+                                           int nxt, int cls, long long off_s = 0, long long off_sa = 0,
+                                           bool have_rew = false, float rew = 0.f) {
+  const bool resetting = in.resetting, stepping = in.stepping;
   if (resetting) {  // auto_reset path == BaseMDP.reset(): the action is ignored, reward is None (NaN here)
     nxt = sample_start(tb, in.un64);
-    io.state[e] = nxt;
-    io.h[e] = 0;
-    io.step_type[e] = COLO_STEP_FIRST;
-    if (io.step_type_mirror) io.step_type_mirror[e] = COLO_STEP_FIRST;
-    io.reward[e] = __int_as_float(0x7fc00000);
-    if (io.discount) io.discount[e] = __int_as_float(0x7fc00000);
-    io.obs[e] = nxt;
+    store_first(io, e, nxt, false);
   } else if (stepping) {
     const int hh = in.h + 1;
     io.h[e] = hh;
@@ -283,10 +309,9 @@ __device__ __forceinline__ void finish_env(const StepIO& io, const colo_mdp_tabl
 }
 
 // the dense reward class of a step s --a--> nxt
-__device__ __forceinline__ int dense_cls(const colo_mdp_tables& tb, const EnvIn& in, int nxt) {
-  if (tb.rew_cls_sas) return tb.rew_cls_sas[((size_t)in.s * tb.A + in.a) * tb.S + nxt];
-  if (tb.rew_cls_sa) return tb.rew_cls_sa[(size_t)in.s * tb.A + in.a];
-  return 0;
+__device__ __forceinline__ int dense_cls(const colo_mdp_tables& tb, int s, int a, int nxt) {
+  return tb.rew_cls_sas ? tb.rew_cls_sas[((size_t)s * tb.A + a) * tb.S + nxt]
+                        : (tb.rew_cls_sa ? tb.rew_cls_sa[(size_t)s * tb.A + a] : 0);
 }
 
 // Position of x in one monotone dense row, warp-cooperative.  The row is read as quads (4 consecutive entries per
@@ -339,57 +364,63 @@ __device__ __forceinline__ int warp_row_next(const TC* __restrict__ row, int S, 
 
 constexpr int kEnvUnroll = 4;  // independent row searches in flight per warp
 
+// The warp walks over the 32 envs of its tile and every lane helps searching env i's row: lane i hands the warp its
+// row, the row's S and ld and its uniform.  Returns the next state of this lane's env.
+template <typename TC, int NCH>
+__device__ __forceinline__ int warp_tile_next(const TC* row_l, int S_l, int ld_l, TC u_l, int lane) {
+  int my_next = 0;
+  for (int i0 = 0; i0 < 32; i0 += kEnvUnroll) {
+#pragma unroll
+    for (int k = 0; k < kEnvUnroll; ++k) {
+      const int i = i0 + k;
+      const TC* row = reinterpret_cast<const TC*>(__shfl_sync(FULL, (unsigned long long)row_l, i));
+      const int S_i = __shfl_sync(FULL, S_l, i), ld_i = __shfl_sync(FULL, ld_l, i);
+      const TC u_i = __shfl_sync(FULL, u_l, i);
+      const int nxt = warp_row_next<TC, NCH>(row, S_i, ld_i, u_i, lane);
+      if (lane == i) my_next = nxt;
+    }
+  }
+  return my_next;
+}
+
+// SERVER: the launch runs one pass per doorbell until the host retires the server; otherwise exactly one pass.
+// step_envs(t) steps the launch's envs once, t being the Philox step counter of the pass.  The kernel's loop-invariant
+// set-up stays outside the pass loop, in the kernel.
+template <bool SERVER, typename Pass>
+__device__ __forceinline__ void run_passes(const StepIO& io, const Pass& step_envs) {
+  for (unsigned long long pass = io.srv_seq0 + 1;; ++pass) {
+    unsigned long long t_pass = step_t0(io);
+    if (SERVER) {
+      if (!server_wait(io, pass)) return;
+      t_pass += pass - io.srv_seq0 - 1;
+    }
+    step_envs(t_pass);
+    if (!SERVER) return;
+    server_done(io, pass);
+  }
+}
+
 template <typename TC, int NCH, bool SERVER>
 __global__ void __launch_bounds__(kStepThreads) env_step_dense_kernel(const colo_mdp_tables tb, const StepIO io) {
   const int lane = threadIdx.x & 31;
   const long long warp_global = ((long long)blockIdx.x * kStepThreads + threadIdx.x) >> 5;
   const long long n_warps = ((long long)gridDim.x * kStepThreads) >> 5;
   const long long n_tiles = (io.N + 31) >> 5;
-  const int S = tb.S, A = tb.A, ld = tb.ld;
   const TC* __restrict__ cdf = reinterpret_cast<const TC*>(tb.cdf);
   constexpr bool F32U = sizeof(TC) == 4;
-
-  for (unsigned long long pass = io.srv_seq0 + 1;; ++pass) {  // SERVER: one pass per doorbell; else exactly one pass
-  unsigned long long t_pass = step_t0(io);
-  if (SERVER) {
-    if (!server_wait(io, pass)) return;
-    t_pass += pass - io.srv_seq0 - 1;
-  }
-  for (long long tile = warp_global; tile < n_tiles; tile += n_warps)
-  for (int step = 0; step < io.n_steps; ++step) {  // an env is owned by the same lane for every step of the launch
-    const long long e = tile * 32 + lane;
-    const bool valid = e < io.N;
-    EnvIn in;
-    in.s = 0; in.a = 0; in.st = COLO_STEP_MID; in.h = 0; in.bad = 0; in.un64 = 0.0; in.un32 = 0.f; in.ur = 0.f;
-    if (valid) in = load_env<F32U>(io, tb, e, t_pass + step);
-    const bool is_last = valid && in.st == COLO_STEP_LAST;
-    const bool resetting = is_last && io.auto_reset;
-    const bool stepping = valid && !is_last && !in.bad;
-    if (is_last && !io.auto_reset && io.status) *io.status = COLO_NEEDS_RESET;
-    // lanes that do not step still take part in the searches with a harmless row (keeps the loop branch-free)
-    const int s_l = stepping ? in.s : 0, a_l = stepping ? in.a : 0;
-    const TC u_l = F32U ? (TC)in.un32 : (TC)in.un64;
-
-    int my_next = 0;
-    // the warp walks over the 32 envs of its tile; every lane helps searching env i's row
-    for (int i0 = 0; i0 < 32; i0 += kEnvUnroll) {
-#pragma unroll
-      for (int k = 0; k < kEnvUnroll; ++k) {
-        const int i = i0 + k;
-        const int s_i = __shfl_sync(FULL, s_l, i);
-        const int a_i = __shfl_sync(FULL, a_l, i);
-        const TC u_i = __shfl_sync(FULL, u_l, i);
-        const TC* row = cdf + ((size_t)s_i * A + a_i) * ld;
-        const int nxt = warp_row_next<TC, NCH>(row, S, ld, u_i, lane);
-        if (lane == i) my_next = nxt;
-      }
+  run_passes<SERVER>(io, [&](unsigned long long t) {
+    for (long long tile = warp_global; tile < n_tiles; tile += n_warps)
+    for (int step = 0; step < io.n_steps; ++step) {  // an env is owned by the same lane for every step of the launch
+      const long long e = tile * 32 + lane;
+      const bool valid = e < io.N;
+      const EnvIn in = begin_env<F32U>(io, tb, e, valid, t + step, io.seed, io.env0 + (uint64_t)e);
+      // lanes that do not step still take part in the searches with a harmless row (keeps the loop branch-free)
+      const TC* row_l = cdf + (in.stepping ? ((size_t)in.s * tb.A + in.a) * tb.ld : 0);
+      const int nxt = warp_tile_next<TC, NCH>(row_l, tb.S, tb.ld, F32U ? (TC)in.un32 : (TC)in.un64, lane);
+      const int cls = in.stepping ? dense_cls(tb, in.s, in.a, nxt) : 0;
+      finish_env(io, tb, valid ? e : 0, in, nxt, cls);
     }
-    const int cls = stepping ? dense_cls(tb, in, my_next) : 0;
-    finish_env(io, tb, valid ? e : 0, in, my_next, cls, stepping, resetting);
-  }
-  if (!SERVER) return;
-  server_done(io, pass);
-  }
+  });
 }
 
 // ---- breakpoint table (colo_mdp_tables.cdf_breaks) ----------------------------------------------------------------------
@@ -440,6 +471,21 @@ __device__ __forceinline__ BreakStep breaks_step(const void* table, unsigned r, 
   return b;
 }
 
+// the reward class of candidate pos (0..31) of a block, from its 32-byte sector of rew_cls_pad
+__device__ __forceinline__ int block_cls(uint4 c0, uint4 c1, int pos) {
+  const unsigned w = pos < 16 ? (pos < 8 ? (pos < 4 ? c0.x : c0.y) : (pos < 12 ? c0.z : c0.w))
+                              : (pos < 24 ? (pos < 20 ? c1.x : c1.y) : (pos < 28 ? c1.z : c1.w));
+  return (int)((w >> (8 * (pos & 3))) & 0xffu);
+}
+
+// x >= total (rounding): bisect's hi = n-1 clamp == first index where the row reaches total
+template <typename TC>
+__device__ __forceinline__ int row_clamp(const TC* __restrict__ row, int S, TC total) {
+  int nxt = 0;
+  while (nxt < S - 1 && __ldg(row + nxt) < total) ++nxt;
+  return nxt;
+}
+
 // Rows of at most 1024 states, one THREAD per env: a three-round k-ary search instead of reading the whole row.  The last
 // entries of the row's quads are monotone, so the number G of quads lying entirely at or below x is found from (1) the
 // last entry of every 8th quad (4*NCH independent 4-byte loads, all issued before any is consumed), (2) the last entries
@@ -462,114 +508,97 @@ __global__ void __launch_bounds__(kStepThreads) env_step_dense_kary_kernel(const
   const TC* __restrict__ mid = reinterpret_cast<const TC*>(tb.cdf_mid);
   const TC* __restrict__ coarse = tb.cdf_mid ? reinterpret_cast<const TC*>(tb.cdf_coarse) : nullptr;
   constexpr bool F32U = sizeof(TC) == 4;
-  for (unsigned long long pass = io.srv_seq0 + 1;; ++pass) {  // SERVER: one pass per doorbell; else exactly one pass
-  unsigned long long t_pass = step_t0(io);
-  if (SERVER) {
-    if (!server_wait(io, pass)) return;
-    t_pass += pass - io.srv_seq0 - 1;
-  }
-  for (long long e = (long long)blockIdx.x * kStepThreads + threadIdx.x; e < n_pad; e += n_thr)
-  for (int step = 0; step < io.n_steps; ++step) {  // an env is owned by the same thread for every step of the launch
-    const bool valid = e < io.N;
-    EnvIn in;
-    in.s = 0; in.a = 0; in.st = COLO_STEP_MID; in.h = 0; in.bad = 0; in.un64 = 0.0; in.un32 = 0.f; in.ur = 0.f;
-    if (valid) in = load_env<F32U>(io, tb, e, t_pass + step);
-    const bool is_last = valid && in.st == COLO_STEP_LAST;
-    const bool resetting = is_last && io.auto_reset;
-    const bool stepping = valid && !is_last && !in.bad;
-    if (is_last && !io.auto_reset && io.status) *io.status = COLO_NEEDS_RESET;
-    int nxt = 0, cls = 0;
-    bool have_rew = false;
-    float rew = 0.f;
-    if (stepping) {
-      bool have_cls = false;
-      if constexpr (KB > 0) {
-        const BreakStep b = breaks_step<KB>(tb.cdf_breaks, (unsigned)(in.s * A + in.a), in.un32);
-        nxt = b.nxt;
-        cls = b.cls;
-        have_cls = b.have_cls;
-        // a constant class gives its reward at every uniform in [0, 1] (supplied ones may lie outside)
-        have_rew = b.have_rew && in.ur >= 0.f && in.ur <= 1.f;
-        rew = b.rew;
-      } else {
-        const TC* row = cdf + (size_t)(unsigned)(in.s * A + in.a) * (unsigned)ld;
-        TC total, x;
-        int blk = 0, G = 0;
-        uint4 c0 = make_uint4(0, 0, 0, 0), c1 = c0;
-        nxt = ld;
-        if (coarse) {  // two-level index: NCH 128-bit loads of a small hot table, then the 8 quad ends of one block
-          const unsigned r = (unsigned)(in.s * A + in.a);
-          Quad<TC> cq[NCH];
-#pragma unroll
-          for (int k = 0; k < NCH; ++k) cq[k].load(coarse + (size_t)r * NB + 4 * k);
-          total = cq[NCH - 1].v[3];  // row[ld-1]: the padding [S, ld) holds the row total, i.e. the value of row[S-1]
-          x = (F32U ? (TC)in.un32 : (TC)in.un64) * total;
-#pragma unroll
-          for (int k = 0; k < NCH; ++k) blk += (cq[k].v[0] <= x) + (cq[k].v[1] <= x) + (cq[k].v[2] <= x) + (cq[k].v[3] <= x);
-          if (blk < NB) {
-            // round 2: the 8 quad ends of the block (one 32-byte sector of cdf_mid) and, in the same round, the reward
-            // classes of the block's 32 candidate next states (rew_cls_pad: rew_cls_sas with rows padded to ld, so the
-            // slice is one aligned 32-byte sector): the class lookup no longer waits for the search to finish
-            Quad<TC> m0, m1;
-            const TC* mp = mid + (size_t)r * (32 * NCH) + 8 * blk;
-            m0.load(mp);
-            m1.load(mp + 4);
-            if (tb.rew_cls_pad) {
-              const uint4* cp = reinterpret_cast<const uint4*>(tb.rew_cls_pad + (size_t)r * ld + 32 * blk);
-              c0 = __ldg(cp);
-              c1 = __ldg(cp + 1);
-            }
-            G = 8 * blk + (m0.v[0] <= x) + (m0.v[1] <= x) + (m0.v[2] <= x) + (m0.v[3] <= x) + (m1.v[0] <= x) +
-                (m1.v[1] <= x) + (m1.v[2] <= x) + (m1.v[3] <= x);
-          }
+  run_passes<SERVER>(io, [&](unsigned long long t) {
+    for (long long e = (long long)blockIdx.x * kStepThreads + threadIdx.x; e < n_pad; e += n_thr)
+    for (int step = 0; step < io.n_steps; ++step) {  // an env is owned by the same thread for every step of the launch
+      const bool valid = e < io.N;
+      const EnvIn in = begin_env<F32U>(io, tb, e, valid, t + step, io.seed, io.env0 + (uint64_t)e);
+      int nxt = 0, cls = 0;
+      bool have_rew = false;
+      float rew = 0.f;
+      if (in.stepping) {
+        bool have_cls = false;
+        if constexpr (KB > 0) {
+          const BreakStep b = breaks_step<KB>(tb.cdf_breaks, (unsigned)(in.s * A + in.a), in.un32);
+          nxt = b.nxt;
+          cls = b.cls;
+          have_cls = b.have_cls;
+          // a constant class gives its reward at every uniform in [0, 1] (supplied ones may lie outside)
+          have_rew = b.have_rew && in.ur >= 0.f && in.ur <= 1.f;
+          rew = b.rew;
         } else {
-          total = __ldg(row + S - 1);
-          x = (F32U ? (TC)in.un32 : (TC)in.un64) * total;
-          TC c[NB];
+          const TC* row = cdf + (size_t)(unsigned)(in.s * A + in.a) * (unsigned)ld;
+          TC total, x;
+          int blk = 0, G = 0;
+          uint4 c0 = make_uint4(0, 0, 0, 0), c1 = c0;
+          nxt = ld;
+          if (coarse) {  // two-level index: NCH 128-bit loads of a small hot table, then the 8 quad ends of one block
+            const unsigned r = (unsigned)(in.s * A + in.a);
+            Quad<TC> cq[NCH];
 #pragma unroll
-          for (int k = 0; k < NB; ++k) c[k] = __ldg(row + 32 * k + 31);  // last entry of quad 8k+7
+            for (int k = 0; k < NCH; ++k) cq[k].load(coarse + (size_t)r * NB + 4 * k);
+            total = cq[NCH - 1].v[3];  // row[ld-1]: the padding [S, ld) holds the row total, i.e. the value of row[S-1]
+            x = (F32U ? (TC)in.un32 : (TC)in.un64) * total;
 #pragma unroll
-          for (int k = 0; k < NB; ++k) blk += c[k] <= x ? 1 : 0;
+            for (int k = 0; k < NCH; ++k) blk += (cq[k].v[0] <= x) + (cq[k].v[1] <= x) + (cq[k].v[2] <= x) + (cq[k].v[3] <= x);
+            if (blk < NB) {
+              // round 2: the 8 quad ends of the block (one 32-byte sector of cdf_mid) and, in the same round, the reward
+              // classes of the block's 32 candidate next states (rew_cls_pad: rew_cls_sas with rows padded to ld, so the
+              // slice is one aligned 32-byte sector): the class lookup does not wait for the search to finish
+              Quad<TC> m0, m1;
+              const TC* mp = mid + (size_t)r * (32 * NCH) + 8 * blk;
+              m0.load(mp);
+              m1.load(mp + 4);
+              if (tb.rew_cls_pad) {
+                const uint4* cp = reinterpret_cast<const uint4*>(tb.rew_cls_pad + (size_t)r * ld + 32 * blk);
+                c0 = __ldg(cp);
+                c1 = __ldg(cp + 1);
+              }
+              G = 8 * blk + (m0.v[0] <= x) + (m0.v[1] <= x) + (m0.v[2] <= x) + (m0.v[3] <= x) + (m1.v[0] <= x) +
+                  (m1.v[1] <= x) + (m1.v[2] <= x) + (m1.v[3] <= x);
+            }
+          } else {
+            total = __ldg(row + S - 1);
+            x = (F32U ? (TC)in.un32 : (TC)in.un64) * total;
+            TC c[NB];
+#pragma unroll
+            for (int k = 0; k < NB; ++k) c[k] = __ldg(row + 32 * k + 31);  // last entry of quad 8k+7
+#pragma unroll
+            for (int k = 0; k < NB; ++k) blk += c[k] <= x ? 1 : 0;
+            if (blk < NB) {
+              const TC* b = row + 32 * blk;
+              TC q[8];
+#pragma unroll
+              for (int k = 0; k < 8; ++k) q[k] = __ldg(b + 4 * k + 3);
+              G = 8 * blk;
+#pragma unroll
+              for (int k = 0; k < 8; ++k) G += q[k] <= x ? 1 : 0;
+            }
+          }
           if (blk < NB) {
-            const TC* b = row + 32 * blk;
-            TC q[8];
-#pragma unroll
-            for (int k = 0; k < 8; ++k) q[k] = __ldg(b + 4 * k + 3);
-            G = 8 * blk;
-#pragma unroll
-            for (int k = 0; k < 8; ++k) G += q[k] <= x ? 1 : 0;
+            Quad<TC> qq;
+            qq.load(row + 4 * G);  // the crossing quad: its last entry is > x, its first three decide
+            nxt = 4 * G + (qq.v[0] <= x) + (qq.v[1] <= x) + (qq.v[2] <= x);
+            if (coarse && tb.rew_cls_pad && nxt < S) {
+              cls = block_cls(c0, c1, nxt - 32 * blk);
+              have_cls = true;
+            }
+          }
+          if (nxt >= S) {
+            nxt = row_clamp(row, S, total);
+            have_cls = false;
           }
         }
-        if (blk < NB) {
-          Quad<TC> qq;
-          qq.load(row + 4 * G);  // the crossing quad: its last entry is > x, its first three decide
-          nxt = 4 * G + (qq.v[0] <= x) + (qq.v[1] <= x) + (qq.v[2] <= x);
-          if (coarse && tb.rew_cls_pad && nxt < S) {
-            const int pos = nxt - 32 * blk;
-            const unsigned w = pos < 16 ? (pos < 8 ? (pos < 4 ? c0.x : c0.y) : (pos < 12 ? c0.z : c0.w))
-                                        : (pos < 24 ? (pos < 20 ? c1.x : c1.y) : (pos < 28 ? c1.z : c1.w));
-            cls = (int)((w >> (8 * (pos & 3))) & 0xffu);
-            have_cls = true;
-          }
-        }
-        if (nxt >= S) {  // x >= total (rounding): bisect's hi = n-1 clamp == first index where the row reaches total
-          nxt = 0;
-          while (nxt < S - 1 && __ldg(row + nxt) < total) ++nxt;
-          have_cls = false;
+        if (!have_cls) {
+          if (tb.rew_cls_sas)
+            cls = tb.rew_cls_sas[((size_t)in.s * A + in.a) * S + nxt];
+          else if (tb.rew_cls_sa)
+            cls = tb.rew_cls_sa[(size_t)in.s * A + in.a];
         }
       }
-      if (!have_cls) {
-        if (tb.rew_cls_sas)
-          cls = tb.rew_cls_sas[((size_t)in.s * A + in.a) * S + nxt];
-        else if (tb.rew_cls_sa)
-          cls = tb.rew_cls_sa[(size_t)in.s * A + in.a];
-      }
+      finish_env(io, tb, valid ? e : 0, in, nxt, cls, 0, 0, have_rew, rew);
     }
-    finish_env(io, tb, valid ? e : 0, in, nxt, cls, stepping, resetting, 0, 0, have_rew, rew);
-  }
-  if (!SERVER) return;
-  server_done(io, pass);
-  }
+  });
 }
 
 // The LEAN form of the k-ary step for the common call: one step per launch, supplied actions, in-kernel Philox uniforms,
@@ -682,17 +711,11 @@ __global__ void __launch_bounds__(kLeanThreads) env_step_kary_lean_kernel(const 
       const float4 qq = __ldg(reinterpret_cast<const float4*>(row) + G);
       nxt = 4 * G + (qq.x <= x) + (qq.y <= x) + (qq.z <= x);
       if (nxt < S) {
-        const int pos = nxt - 32 * blk;
-        const unsigned wsel = pos < 16 ? (pos < 8 ? (pos < 4 ? c0.x : c0.y) : (pos < 12 ? c0.z : c0.w))
-                                       : (pos < 24 ? (pos < 20 ? c1.x : c1.y) : (pos < 28 ? c1.z : c1.w));
-        cls = (int)((wsel >> (8 * (pos & 3))) & 0xffu);
+        cls = block_cls(c0, c1, nxt - 32 * blk);
         have_cls = true;
       }
     }
-    if (nxt >= S) {  // x >= total (rounding): bisect's hi = n-1 clamp == first index where the row reaches total
-      nxt = 0;
-      while (nxt < S - 1 && __ldg(row + nxt) < total) ++nxt;
-    }
+    if (nxt >= S) nxt = row_clamp(row, S, total);
     if (!have_cls) cls = tb.rew_cls_sas ? tb.rew_cls_sas[((size_t)s * A + a) * S + nxt] : (tb.rew_cls_sa ? tb.rew_cls_sa[(size_t)s * A + a] : 0);
   }
   lean_store<COMPACT>(tb, io, e, v, nxt, cls, false, 0.f);
@@ -724,15 +747,9 @@ __global__ void __launch_bounds__(kLeanThreads) env_step_breaks_lean_kernel(cons
 __device__ __forceinline__ void succ_env_step(const StepIO& io, const colo_mdp_tables& tb, long long e, bool valid,
                                               unsigned long long t, unsigned long long seed, unsigned long long ctr,
                                               long long off_s, long long off_sa) {
-  EnvIn in;
-  in.s = 0; in.a = 0; in.st = COLO_STEP_MID; in.h = 0; in.bad = 0; in.un64 = 0.0; in.un32 = 0.f; in.ur = 0.f;
-  if (valid) in = load_env<false>(io, tb, e, t, seed, ctr);
-  const bool is_last = valid && in.st == COLO_STEP_LAST;
-  const bool resetting = is_last && io.auto_reset;
-  const bool stepping = valid && !is_last && !in.bad;
-  if (is_last && !io.auto_reset && io.status) *io.status = COLO_NEEDS_RESET;
+  const EnvIn in = begin_env<false>(io, tb, e, valid, t, seed, ctr);
   int nxt = 0, cls = 0;
-  if (stepping) {
+  if (in.stepping) {
     const size_t sa = (size_t)in.s * tb.A + in.a;
     const size_t base = sa * tb.Ksucc;
     const int n = __ldg(tb.succ_len + sa);
@@ -744,7 +761,7 @@ __device__ __forceinline__ void succ_env_step(const StepIO& io, const colo_mdp_t
     nxt = __ldg(tb.succ_idx + base + pos);
     cls = tb.rew_cls_succ ? __ldg(tb.rew_cls_succ + base + pos) : 0;
   }
-  finish_env(io, tb, valid ? e : 0, in, nxt, cls, stepping, resetting, off_s, off_sa);
+  finish_env(io, tb, valid ? e : 0, in, nxt, cls, off_s, off_sa);
 }
 
 template <bool SERVER>
@@ -752,18 +769,11 @@ __global__ void __launch_bounds__(kStepThreads) env_step_succ_kernel(const colo_
   const long long n_thr = (long long)gridDim.x * kStepThreads;
   // round the loop bound up to whole warps: finish_env uses warp collectives
   const long long n_pad = (io.N + 31) & ~31LL;
-  for (unsigned long long pass = io.srv_seq0 + 1;; ++pass) {  // SERVER: one pass per doorbell; else exactly one pass
-  unsigned long long t_pass = step_t0(io);
-  if (SERVER) {
-    if (!server_wait(io, pass)) return;
-    t_pass += pass - io.srv_seq0 - 1;
-  }
-  for (long long e = (long long)blockIdx.x * kStepThreads + threadIdx.x; e < n_pad; e += n_thr)
-  for (int step = 0; step < io.n_steps; ++step)  // an env is owned by the same thread for every step of the launch
-    succ_env_step(io, tb, e, e < io.N, t_pass + step, io.seed, io.env0 + (uint64_t)e, 0, 0);
-  if (!SERVER) return;
-  server_done(io, pass);
-  }
+  run_passes<SERVER>(io, [&](unsigned long long t) {
+    for (long long e = (long long)blockIdx.x * kStepThreads + threadIdx.x; e < n_pad; e += n_thr)
+    for (int step = 0; step < io.n_steps; ++step)  // an env is owned by the same thread for every step of the launch
+      succ_env_step(io, tb, e, e < io.N, t + step, io.seed, io.env0 + (uint64_t)e, 0, 0);
+  });
 }
 
 // BaseMDP.reset of one env (valid); returns its start state
@@ -778,16 +788,7 @@ __device__ __forceinline__ int reset_env(const StepIO& io, const colo_mdp_tables
     u = u53(w.w[0], w.w[1]);
   }
   const int s0 = sample_start(tb, u);
-  io.state[e] = s0;
-  io.h[e] = 0;
-  io.step_type[e] = COLO_STEP_FIRST;
-  if (io.step_type_mirror) io.step_type_mirror[e] = COLO_STEP_FIRST;
-  if (io.discount) io.discount[e] = __int_as_float(0x7fc00000);
-  if (io.reward) io.reward[e] = __int_as_float(0x7fc00000);  // the reference's reward of a FIRST TimeStep is None
-  if (io.io_compact)
-    reinterpret_cast<short*>(io.obs)[e] = (short)s0;
-  else
-    io.obs[e] = s0;
+  store_first(io, e, s0, io.io_compact);
   return s0;
 }
 
@@ -847,30 +848,12 @@ __global__ void __launch_bounds__(kStepThreads) env_step_dense_mixed_kernel(cons
     const MixedInst d = insts[mixed_inst_of(inst_of, e, valid)];
     const TC* __restrict__ cdf = reinterpret_cast<const TC*>(d.tb.cdf);
     for (int step = 0; step < io.n_steps; ++step) {
-      EnvIn in;
-      in.s = 0; in.a = 0; in.st = COLO_STEP_MID; in.h = 0; in.bad = 0; in.un64 = 0.0; in.un32 = 0.f; in.ur = 0.f;
-      if (valid) in = load_env<F32U>(io, d.tb, e, io.t + step, d.seed, (unsigned long long)(e - d.start));
-      const bool is_last = valid && in.st == COLO_STEP_LAST;
-      const bool resetting = is_last && io.auto_reset;
-      const bool stepping = valid && !is_last && !in.bad;
-      if (is_last && !io.auto_reset && io.status) *io.status = COLO_NEEDS_RESET;
-      // lanes that do not step search row 0 of their instance; every lane hands the warp its own row and shape
-      const TC* row_l = cdf + (stepping ? ((size_t)in.s * d.tb.A + in.a) * d.tb.ld : 0);
-      const TC u_l = F32U ? (TC)in.un32 : (TC)in.un64;
-      int my_next = 0;
-      for (int i0 = 0; i0 < 32; i0 += kEnvUnroll) {
-#pragma unroll
-        for (int k = 0; k < kEnvUnroll; ++k) {
-          const int i = i0 + k;
-          const TC* row = reinterpret_cast<const TC*>(__shfl_sync(FULL, (unsigned long long)row_l, i));
-          const int S_i = __shfl_sync(FULL, d.tb.S, i), ld_i = __shfl_sync(FULL, d.tb.ld, i);
-          const TC u_i = __shfl_sync(FULL, u_l, i);
-          const int nxt = warp_row_next<TC, NCH>(row, S_i, ld_i, u_i, lane);
-          if (lane == i) my_next = nxt;
-        }
-      }
-      const int cls = stepping ? dense_cls(d.tb, in, my_next) : 0;
-      finish_env(io, d.tb, valid ? e : 0, in, my_next, cls, stepping, resetting, d.off_s, d.off_sa);
+      const EnvIn in = begin_env<F32U>(io, d.tb, e, valid, io.t + step, d.seed, (unsigned long long)(e - d.start));
+      // lanes that do not step search row 0 of their instance
+      const TC* row_l = cdf + (in.stepping ? ((size_t)in.s * d.tb.A + in.a) * d.tb.ld : 0);
+      const int nxt = warp_tile_next<TC, NCH>(row_l, d.tb.S, d.tb.ld, F32U ? (TC)in.un32 : (TC)in.un64, lane);
+      const int cls = in.stepping ? dense_cls(d.tb, in.s, in.a, nxt) : 0;
+      finish_env(io, d.tb, valid ? e : 0, in, nxt, cls, d.off_s, d.off_sa);
     }
   }
 }
