@@ -207,6 +207,8 @@ PROTOTYPES = {
     "colo_reset_launch_count": (None, []),
     "colo_backup_tma_sweeps": (_ULL, []),
     "colo_step_kernel_launches": (_ULL, [_I]),
+    "colo_set_step_overlap": (_I, [_I]),
+    "colo_step_overlap_launches": (_ULL, []),
     "colo_solver_path_launches": (_ULL, [_I]),
     "colo_stream_synchronize": (_I, [_P]),
     "colo_backup_f32": (_I, [C.POINTER(BackupArgs), _P]),

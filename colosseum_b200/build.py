@@ -39,19 +39,26 @@ def _stale():
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build_library(force=False, verbose=False):
-    """Compile every CUDA source for sm_100a and link the shared library.  Returns its path."""
-    if not force and not _stale():
+def build_library(force=False, verbose=False, defines=None, out=None):
+    """Compile every CUDA source for sm_100a and link the shared library.  Returns its path.
+
+    defines: {name: value} passed as -D to every source, for kernel-variant probes; out: path of the library to link
+    (its objects go to a directory beside it).  A variant (either argument given) is always rebuilt."""
+    lib_path = os.path.abspath(out) if out else LIB_PATH
+    variant = bool(defines) or out is not None
+    if not force and not variant and not _stale():
         return LIB_PATH
-    os.makedirs(LIB_DIR, exist_ok=True)
-    obj_dir = os.path.join(LIB_DIR, "obj")
+    lib_dir = os.path.dirname(lib_path)
+    os.makedirs(lib_dir, exist_ok=True)
+    obj_dir = os.path.join(lib_dir, "obj" if not variant else os.path.basename(lib_path) + ".obj")
     os.makedirs(obj_dir, exist_ok=True)
     nvcc = _nvcc()
     env = dict(os.environ)
+    dflags = [f"-D{k}={v}" for k, v in (defines or {}).items()]
     procs = []
     for src in SOURCES:
         obj = os.path.join(obj_dir, src.replace(".cu", ".o"))
-        cmd = [nvcc] + NVCC_FLAGS + ["-I", INCLUDE, "-c", os.path.join(CSRC, src), "-o", obj]
+        cmd = [nvcc] + NVCC_FLAGS + dflags + ["-I", INCLUDE, "-c", os.path.join(CSRC, src), "-o", obj]
         if verbose:
             cmd.insert(1, "-Xptxas=-v")
         procs.append((src, obj, subprocess.Popen(cmd, env=env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT)))
@@ -63,9 +70,9 @@ def build_library(force=False, verbose=False):
         if p.returncode != 0:
             raise RuntimeError(f"nvcc failed on {src}")
         objs.append(obj)
-    cmd = [nvcc, "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-o", LIB_PATH] + objs
+    cmd = [nvcc, "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-o", lib_path] + objs
     subprocess.check_call(cmd, env=env)
-    return LIB_PATH
+    return lib_path
 
 
 if __name__ == "__main__":

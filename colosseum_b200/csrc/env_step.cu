@@ -610,6 +610,53 @@ __global__ void __launch_bounds__(kStepThreads) env_step_dense_kary_kernel(const
 // the batch fills the machine, so instructions are what the asymptotic env-steps/s is made of.
 constexpr int kLeanThreads = 128;
 
+// Launch overlap of the lean kernels (DESIGN 4.2).  The host launches them with programmatic dependent launch
+// (launch_lean), so a step's grid can be resident while the grid ahead of it on the stream still runs.  Before its
+// griddepcontrol.wait a lean kernel touches global memory only through L2 prefetches -- safe whatever the grid ahead
+// writes, since L2 is the device's point of coherence and a prefetch fills no L1 -- of the lines its loads and counter
+// atomics will need: the CTA's own env scalars, and a share of the batch's first table round and of all privatised
+// counter copies.  Without a predecessor grid (or the launch attribute) the wait returns at once.  Each kernel comes
+// with and without the prefetch (PF); the host takes the prefetching one only where a grid ahead can hide it
+// (launch_lean).
+// COLO_STEP_PDL_TRIGGER places griddepcontrol.launch_dependents: 0 before the wait (grids pile up as deep as the SMs
+// allow), 1 after it (at most one grid waits behind a running one), 2 after the stores.  COLO_STEP_PREFETCH=0 drops the
+// prefetches.  Both exist for scripts/step_overlap_probe.py, which builds the variants.
+#ifndef COLO_STEP_PDL_TRIGGER
+#define COLO_STEP_PDL_TRIGGER 1
+#endif
+#ifndef COLO_STEP_PREFETCH
+#define COLO_STEP_PREFETCH 1
+#endif
+
+template <int WHERE>
+__device__ __forceinline__ void lean_trigger() {
+  if (COLO_STEP_PDL_TRIGGER == WHERE) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+}
+
+// table / table_bytes: the batch's first table round (cdf_breaks, or cdf_coarse of the k-ary kernel).  Thread i < 6 of
+// each CTA prefetches from array i: thread 0-2 the CTA's own 128 envs of state, h and step_type; thread 3-5 4 KiB
+// chunk blockIdx.x of the table, visits_s and visits_sa (all copies), so that the CTAs of a grid share the batch-wide
+// arrays (one chunk per CTA: a small grid prefetches their first chunks only, since one CTA issuing many held its own
+// loads behind them).  Each chunk is shrunk to whole 16-byte units inside its array (the bulk prefetch's granule): no
+// address outside an array is touched.
+template <bool PF>
+__device__ __forceinline__ void lean_prologue(const StepIO& io, const void* table, size_t table_bytes) {
+  const unsigned i = threadIdx.x;
+  if (COLO_STEP_PREFETCH && PF && i < 6) {
+    const size_t N = (size_t)io.N, copies = (size_t)io.visits_mask + 1;
+    const void* p = i == 0 ? (const void*)io.state : i == 1 ? (const void*)io.h : i == 2 ? (const void*)io.step_type
+                  : i == 3 ? table : i == 4 ? (const void*)io.visits_s : (const void*)io.visits_sa;
+    const size_t bytes = i < 2 ? 4 * N : i == 2 ? N : i == 3 ? table_bytes : 8 * copies * (size_t)(i == 4 ? io.n_s : io.n_sa);
+    const size_t chunk = i < 2 ? 4 * kLeanThreads : i == 2 ? kLeanThreads : 4096;
+    const size_t lo = (size_t)blockIdx.x * chunk;
+    const uintptr_t a = ((uintptr_t)p + lo + 15) & ~(uintptr_t)15, b = ((uintptr_t)p + min(lo + chunk, bytes)) & ~(uintptr_t)15;
+    if (lo < bytes && b > a) asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a), "r"((unsigned)(b - a)) : "memory");
+  }
+  lean_trigger<0>();
+  asm volatile("griddepcontrol.wait;" ::: "memory");
+  lean_trigger<1>();
+}
+
 // prologue and epilogue of the lean kernels: env scalars in, Philox words, the action check; stores and counters out
 struct LeanEnv {
   int st, s, h, a;
@@ -679,11 +726,12 @@ __device__ __forceinline__ void lean_store(const colo_mdp_tables& tb, const Step
   aggregated_inc(io.visits_sa + (size_t)copy * io.n_sa, (long long)nxt * tb.A + v.a, v.stepping);
 }
 
-template <int NCH, bool COMPACT>
+template <int NCH, bool COMPACT, bool PF>
 __global__ void __launch_bounds__(kLeanThreads) env_step_kary_lean_kernel(const colo_mdp_tables tb, const StepIO io) {
   constexpr int ld = 128 * NCH, NB = 4 * NCH;
   const unsigned e = blockIdx.x * kLeanThreads + threadIdx.x;
   const int S = tb.S, A = tb.A;
+  lean_prologue<PF>(io, tb.cdf_coarse, (size_t)S * A * NB * sizeof(float));
   const LeanEnv v = lean_load<COMPACT>(tb, io, e);
   const int s = v.s, a = v.a;
   int nxt = 0, cls = 0;
@@ -719,14 +767,16 @@ __global__ void __launch_bounds__(kLeanThreads) env_step_kary_lean_kernel(const 
     if (!have_cls) cls = tb.rew_cls_sas ? tb.rew_cls_sas[((size_t)s * A + a) * S + nxt] : (tb.rew_cls_sa ? tb.rew_cls_sa[(size_t)s * A + a] : 0);
   }
   lean_store<COMPACT>(tb, io, e, v, nxt, cls, false, 0.f);
+  lean_trigger<2>();
 }
 
 // The lean call on the breakpoint table: env scalars -> one K-entry breakpoint row (one round of K independent 16-byte
 // loads) -> stores, plus a reward-quantile round only where the class is not constant.  Same Philox words, same x, same
 // result and reward bits as env_step_kary_lean_kernel.
-template <int K, bool COMPACT>
+template <int K, bool COMPACT, bool PF>
 __global__ void __launch_bounds__(kLeanThreads) env_step_breaks_lean_kernel(const colo_mdp_tables tb, const StepIO io) {
   const unsigned e = blockIdx.x * kLeanThreads + threadIdx.x;
+  lean_prologue<PF>(io, tb.cdf_breaks, (size_t)tb.S * tb.A * K * sizeof(int4));
   const LeanEnv v = lean_load<COMPACT>(tb, io, e);
   int nxt = 0, cls = 0;
   bool have_rew = false;
@@ -740,6 +790,7 @@ __global__ void __launch_bounds__(kLeanThreads) env_step_breaks_lean_kernel(cons
     rew = b.rew;
   }
   lean_store<COMPACT>(tb, io, e, v, nxt, cls, have_rew, rew);
+  lean_trigger<2>();
 }
 
 // one step of one env from successor-list tables (every lane of the warp calls it: finish_env uses warp collectives);
@@ -1000,8 +1051,49 @@ static void launch_step(K kernel, int grid, bool server, int share, const colo_m
   kernel<<<grid, kStepThreads, 0, st>>>(*tb, io);
 }
 
+// Programmatic dependent launch of the lean kernels (lean_prologue): a process-wide switch (colo_set_step_overlap,
+// default from COLO_STEP_OVERLAP, on unless "0"), the launches made with the attribute (colo_step_overlap_launches),
+// and whether the driver refused it once (then every later lean launch is plain)
+static std::atomic<int> g_step_overlap{[] {
+  const char* s = getenv("COLO_STEP_OVERLAP");
+  return s && !strcmp(s, "0") ? 0 : 1;
+}()};
+static std::atomic<unsigned long long> g_overlap_launches{0};
+static std::atomic<bool> g_overlap_refused{false};
+
+// The prefetch (lean_prologue) pays only where a grid ahead hides it (profiles/r4_step_overlap_probe.txt): an
+// overlapped launch of at most this many CTAs.  A plain launch has nothing ahead of it, and the prefetch immediately
+// followed by the loads of the same lines cost 12 % at 65,536 envs; a larger grid streams its env scalars at the issue
+// bound, where the prefetch cost 5-9 % at 1 Mi and 16 Mi envs and even the skipped prologue 2-3 % at 16 Mi.
+constexpr int kPrefetchCtas = 2048;  // 262,144 envs
+
+// kpf / kplain: the kernel with and without the prefetch.  overlap: the caller allows the attribute (the queued
+// pipeline and the steppers do not: their launches follow stream memory operations or a host synchronisation)
+template <typename K>
+static void launch_lean(K kpf, K kplain, int grid, bool overlap, const colo_mdp_tables* tb, const StepIO& io,
+                        cudaStream_t st) {
+  if (overlap && g_step_overlap.load(std::memory_order_relaxed) && !g_overlap_refused.load(std::memory_order_relaxed)) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(kLeanThreads);
+    cfg.stream = st;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    if (cudaLaunchKernelEx(&cfg, grid <= kPrefetchCtas ? kpf : kplain, *tb, io) == cudaSuccess) {
+      g_overlap_launches.fetch_add(1, std::memory_order_relaxed);
+      return;
+    }
+    cudaGetLastError();
+    g_overlap_refused.store(true, std::memory_order_relaxed);
+  }
+  kplain<<<grid, kLeanThreads, 0, st>>>(*tb, io);
+}
+
 template <typename TC, bool SERVER>
-static int launch_dense(const colo_mdp_tables* tb, const StepIO& io, void* stream, int share = 1) {
+static int launch_dense(const colo_mdp_tables* tb, const StepIO& io, void* stream, int share = 1, bool overlap = true) {
   int r = check_tables_common(tb);
   if (r != COLO_OK) return r;
   COLO_ARG_CHECK(tb->cdf && tb->ld >= tb->S && tb->ld % 4 == 0, "dense cdf with ld % 4 == 0 is required");
@@ -1023,10 +1115,14 @@ static int launch_dense(const colo_mdp_tables* tb, const StepIO& io, void* strea
         io.visits_sa && io.N < (1LL << 31) - kLeanThreads) {
       const int gl = (int)((io.N + kLeanThreads - 1) / kLeanThreads);
       if (kb) {
-#define COLO_BREAKS_LEAN(K)                                                                          \
-  case K:                                                                                            \
-    if (io.io_compact) env_step_breaks_lean_kernel<K, true><<<gl, kLeanThreads, 0, st>>>(*tb, io);   \
-    else env_step_breaks_lean_kernel<K, false><<<gl, kLeanThreads, 0, st>>>(*tb, io);                 \
+#define COLO_BREAKS_LEAN(K)                                                                               \
+  case K:                                                                                                 \
+    if (io.io_compact)                                                                                    \
+      launch_lean(env_step_breaks_lean_kernel<K, true, true>, env_step_breaks_lean_kernel<K, true, false>, gl, \
+                  overlap, tb, io, st);                                                                   \
+    else                                                                                                  \
+      launch_lean(env_step_breaks_lean_kernel<K, false, true>, env_step_breaks_lean_kernel<K, false, false>, gl, \
+                  overlap, tb, io, st);                                                                   \
     break
         switch (kb) {
           COLO_BREAKS_LEAN(2);
@@ -1038,10 +1134,14 @@ static int launch_dense(const colo_mdp_tables* tb, const StepIO& io, void* strea
         count_step_launch(COLO_STEP_KIND_BREAKS);
         return check_launch("env_step_breaks_lean_kernel");
       }
-#define COLO_LEAN(NCH)                                                              \
-  case NCH:                                                                         \
-    if (io.io_compact) env_step_kary_lean_kernel<NCH, true><<<gl, kLeanThreads, 0, st>>>(*tb, io);   \
-    else env_step_kary_lean_kernel<NCH, false><<<gl, kLeanThreads, 0, st>>>(*tb, io);                 \
+#define COLO_LEAN(NCH)                                                                             \
+  case NCH:                                                                                        \
+    if (io.io_compact)                                                                             \
+      launch_lean(env_step_kary_lean_kernel<NCH, true, true>, env_step_kary_lean_kernel<NCH, true, false>, gl, \
+                  overlap, tb, io, st);                                                            \
+    else                                                                                           \
+      launch_lean(env_step_kary_lean_kernel<NCH, false, true>, env_step_kary_lean_kernel<NCH, false, false>, gl, \
+                  overlap, tb, io, st);                                                            \
     break
       switch (ld / 128) {
         COLO_LEAN(1);
@@ -1372,8 +1472,9 @@ int colo_env_stepper_launch(colo_env_stepper* h, const int* action, unsigned lon
   if (h->io.N == 0) return COLO_OK;
   h->io.action = const_cast<int*>(action);
   h->io.t = t;
-  if (h->mode == 0) return colo::launch_dense<float, false>(&h->tb, h->io, h->stream);
-  if (h->mode == 1) return colo::launch_dense<double, false>(&h->tb, h->io, h->stream);
+  // no launch overlap: a stepper launches after the host has synchronised with its previous step
+  if (h->mode == 0) return colo::launch_dense<float, false>(&h->tb, h->io, h->stream, 1, false);
+  if (h->mode == 1) return colo::launch_dense<double, false>(&h->tb, h->io, h->stream, 1, false);
   return colo::launch_succ<false>(&h->tb, h->io, h->stream);
 }
 
@@ -1492,8 +1593,9 @@ static int pl_launch(colo_env_pipeline* p, int g, const int* action, unsigned lo
   io.action = const_cast<int*>(action);
   io.t = t;
   io.t_dev = t_dev;
-  if (h->mode == 0) return colo::launch_dense<float, false>(&h->tb, io, p->streams[g]);
-  if (h->mode == 1) return colo::launch_dense<double, false>(&h->tb, io, p->streams[g]);
+  // no launch overlap: the predecessor of each step is a stream memory operation, not a step kernel
+  if (h->mode == 0) return colo::launch_dense<float, false>(&h->tb, io, p->streams[g], 1, false);
+  if (h->mode == 1) return colo::launch_dense<double, false>(&h->tb, io, p->streams[g], 1, false);
   return colo::launch_succ<false>(&h->tb, io, p->streams[g]);
 }
 
@@ -1766,6 +1868,10 @@ int colo_env_server_stop(const colo_env_server* srv, void* stream) {
 unsigned long long colo_step_kernel_launches(int kind) {
   return kind >= 0 && kind < COLO_STEP_KINDS ? colo::g_step_launches[kind].load(std::memory_order_relaxed) : 0ULL;
 }
+
+int colo_set_step_overlap(int on) { return colo::g_step_overlap.exchange(on ? 1 : 0); }
+
+unsigned long long colo_step_overlap_launches(void) { return colo::g_overlap_launches.load(std::memory_order_relaxed); }
 
 int colo_emit_observations(const float* table, const int* state, const int* h, const unsigned char* step_type,
                            long long N, int H, int S, int D, float* out, void* stream) {

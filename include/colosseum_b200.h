@@ -71,6 +71,14 @@ unsigned long long colo_backup_tma_sweeps(void);
 #define COLO_STEP_KIND_BREAKS_GENERAL 8 /* env_step_dense_kary_kernel searching the breakpoint table (other f32 calls) */
 #define COLO_STEP_KINDS 9
 unsigned long long colo_step_kernel_launches(int kind);
+/* launch overlap of the lean step kernels (kinds 0 and 7): launched with programmatic dependent launch, a step's grid
+ * becomes resident and prefetches its batch's lines into L2 while the step ahead of it on the stream still runs.
+ * Results are the same either way.  Process-wide, on by default (the environment variable COLO_STEP_OVERLAP=0 turns it
+ * off at load); returns the previous setting.  The steppers (colo_env_stepper_*, colo_env_pipeline_run*) never
+ * use it: each of their launches follows a host synchronisation or a stream memory operation. */
+int colo_set_step_overlap(int on);
+/* lean step launches since load that were made with the overlap attribute (counted as colo_step_kernel_launches) */
+unsigned long long colo_step_overlap_launches(void);
 /* Bellman-solver launches since load that went to each solver path (`kind`: COLO_PATH_*; 0 for any other value): the
  * solvers of (B) pick their kernel from the tensor's shape and sparsity, and this tells a caller which one served a
  * call.  Counted on the host when the launch is enqueued, one count per launch (a solve of n sweeps on a per-sweep

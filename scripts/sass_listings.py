@@ -14,16 +14,16 @@ syms = subprocess.run(["cuobjdump", "-elf", so], capture_output=True, text=True)
 for tag, pat in (("backup_kernel_f32_max_vec_warp", r"_ZN4colo13backup_kernelIfLi0ELb1ELb0EEEv\w+?(?=_param|\s|$)"),
                  ("backup_tma_kernel_max_8", r"_ZN4colo17backup_tma_kernelILi0ELi8EEEv\w+?(?=_param|\s|$)"),
                  ("gs_solve_tma_kernel_f32", r"_ZN4colo19gs_solve_tma_kernelIfEEv\w+?(?=_param|\s|$)"),
-                 ("env_step_kary_lean_kernel_4", r"_ZN4colo25env_step_kary_lean_kernelILi4ELb0EEEv\w+?(?=_param|\s|$)"),
-                 ("env_step_kary_lean_kernel_4_compact", r"_ZN4colo25env_step_kary_lean_kernelILi4ELb1EEEv\w+?(?=_param|\s|$)"),
+                 ("env_step_kary_lean_kernel_4", r"_ZN4colo25env_step_kary_lean_kernelILi4ELb0ELb0EEEv\w+?(?=_param|\s|$)"),
+                 ("env_step_kary_lean_kernel_4_compact", r"_ZN4colo25env_step_kary_lean_kernelILi4ELb1ELb0EEEv\w+?(?=_param|\s|$)"),
                  ("hitting_umma_kernel_128", r"_ZN4colo19hitting_umma_kernelILi128ELb0EEEv\w+?(?=_param|\s|$)"),
                  ("hitting_umma_kernel_128_multicast", r"_ZN4colo19hitting_umma_kernelILi128ELb1EEEv\w+?(?=_param|\s|$)"),
-                 ("env_step_breaks_lean_kernel_2", r"_ZN4colo27env_step_breaks_lean_kernelILi2ELb0EEEv\w+?(?=_param|\s|$)"),
+                 ("env_step_breaks_lean_kernel_2", r"_ZN4colo27env_step_breaks_lean_kernelILi2ELb0ELb1EEEv\w+?(?=_param|\s|$)"),
                  ("env_step_dense_kary_kernel_breaks_2",
                   r"_ZN4colo26env_step_dense_kary_kernelIfLi1ELb0ELi2EEEv\w+?(?=_param|\s|$)")):
     if len(sys.argv) > 1 and sys.argv[1] not in tag:
         continue
-    rnd = "r3" if "breaks" in tag else "r2"
+    rnd = "r4" if tag == "env_step_breaks_lean_kernel_2" else "r3" if "breaks" in tag else "r2"
     m = re.search(pat, syms)
     if not m:
         print("symbol not found:", tag)
